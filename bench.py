@@ -21,6 +21,8 @@ roofline = algorithmic bytes (SURVEY.md 8d gather model, no cache credit) per ho
         measured live (csrc/microbench.cu) -- the HBM fraction of such a kernel is meaningless.
 --impl reference times the reference's CPU path (the oracle's restated PyG gather -> scale -> scatter_add_, this
 tier's definition) on the host cores, rank 0 only.  Prints ONE JSON line on rank 0.
+--dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (see dump_outputs), so that two builds
+run with the same arguments -- hence on the same seeded inputs -- can be compared output for output.
 """
 from __future__ import annotations
 
@@ -32,6 +34,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -41,6 +44,8 @@ if ROOT not in sys.path:
 K_HOPS, ALPHA, F_CLASSES = 10, 0.1, 47
 GRAPH_SEED = 20261018
 CPU_SAMPLE_FRACTION = 0.10          # share of the target rows used by the bounded CPU sample (products)
+DUMP_BYTES = 60 << 20               # --dump-outputs: payload of all .npy files of a run together, all ranks (< 64 MB)
+DUMP_SEED = 20261019
 METRIC = {"products": "appnp_propagate_gteps", "arxiv_sage": "sage_mean_aggregate_gteps",
           "reddit_gat": "gat_layer_forward_gteps", "papers100m": "gcn_propagate_bf16_gteps"}
 
@@ -106,6 +111,24 @@ def workload_name(wl: str, N: int, nnz: int) -> str:
     if wl == "reddit_gat":
         return f"GATConv 8 heads x 8 edge-softmax + aggregate forward, Reddit-shaped R-MAT graph (N={N}, nnz={nnz} with self loops)"
     return f"GCN propagation 2 hops, bf16 F=128, papers100M-shaped row-generated graph (N={N}, nnz={nnz} with self loops)"
+
+
+def dump_outputs(out_dir: str, arrays: dict, budget: int = DUMP_BYTES, seed: int = DUMP_SEED) -> None:
+    """Write every tensor of `arrays` (name -> tensor, rows first) as out_dir/<name>.npy: float64 stays float64, every
+    other dtype becomes float32.  When the arrays hold more than `budget` bytes together, each keeps the same share of
+    its rows: a sorted sample drawn from a generator seeded with `seed`, so the same shapes always give the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(v.numel() * (8 if v.dtype == torch.float64 else 4) for v in arrays.values())      # bytes as written
+    keep = budget / total if total > budget else 1.0
+    for name, v in arrays.items():
+        v = v.detach()
+        if keep < 1.0:                   # sample first: a bf16 output is never widened at full size
+            n = v.size(0)
+            rows = torch.randperm(n, generator=torch.Generator().manual_seed(seed))[: max(1, int(n * keep))].sort().values
+            v = v.index_select(0, rows.to(v.device))
+        if v.dtype != torch.float64:
+            v = v.float()
+        np.save(os.path.join(out_dir, name + ".npy"), v.cpu().numpy())
 
 
 def make_products(device):
@@ -229,9 +252,13 @@ def run_reference(args, rank):
     for _ in range(args.warmup):
         fn()
     t0 = time.perf_counter()
-    for _ in range(args.steps):
+    for _ in range(args.steps - 1):
         fn()
+    last = fn()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"out": last})
+    del last
     val = edges * args.steps / dt / 1e9
     sample = "per step: " + sample
     cpu = {"value": val, "unit": "GTEPS", "cores": cores, "kind": "port", "sample": sample}
@@ -331,6 +358,7 @@ class Case:
     l2_table = None              # (table bytes, row bytes): feature matrix is L2-resident -> also report the gather roofline
     gathered_bytes_per_step = 0
     check = None                 # () -> dict, run after the timed region
+    outputs = None               # (what step returned) -> {name: tensor} a caller receives; None: {"out": it}
     close = None
     scaling = "strong"
     keep = None
@@ -422,6 +450,7 @@ def case_products(args, dev, rank, world):
             return res
 
         c.check = check
+        c.outputs = lambda z: {"out": z[: blk.hi - blk.lo, :F_local]}      # this rank's rows (renamed ids) and slice
         c.close = prop.close
         c.keep = (blk, prop, z0l, z0h, outh, sg)
     c.edges_per_step, c.hops_per_step = nnz * K_HOPS, K_HOPS
@@ -452,12 +481,10 @@ def case_arxiv_sage(args, dev, rank, world):
         return SU.add_self_loops(e2, num_nodes=N)[0]
 
     def step():
-        out = None
-        for x in xs:
-            out = mp.propagate(edited(), x=x)
-        return out
+        return [mp.propagate(edited(), x=x) for x in xs]
 
     c.step = step
+    c.outputs = lambda outs: {f"aggr{i}": o for i, o in enumerate(outs)}
     g = P.get_graph(edited(), N, P.LOOP_NONE)
     nnz = g.nnz
     xh = [x.cpu().pin_memory() for x in xs]
@@ -551,6 +578,7 @@ def case_papers100m(args, dev, rank, world):
     z0l[: blk.hi - blk.lo, :Fl] = torch.randn(blk.hi - blk.lo, Fl, device=dev,
                                               generator=torch.Generator(device=dev).manual_seed(1 + rank)).to(dt)
     c.step = lambda: prop.run(z0l, hops, 0.0)
+    c.outputs = lambda z: {"out": z[: blk.hi - blk.lo, :Fl]}
     z0h = z0l.cpu().pin_memory()
     outh = torch.empty_like(z0h).pin_memory()
 
@@ -599,7 +627,12 @@ def main():
                     help="N>1: fused push of finished rows into every peer over NVLink (default) or NCCL all-gather")
     ap.add_argument("--scale", type=float, default=0.0, help="papers100m: shrink nodes and edges together (0 = full size)")
     ap.add_argument("--locality", type=float, default=0.0, help="papers100m: share of neighbours within +-N/64 of the row")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float32, a seeded "
+                         "sample of rows where the whole would exceed 60 MiB; with N GPUs, <name>_rank<r>.npy per rank)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -645,13 +678,20 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     e0.record()
-    for _ in range(args.steps):
+    for _ in range(args.steps - 1):
         c.step()
+    last = c.step()
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     sampler.stop_flag = True
     sampler.join()
+    if args.dump_outputs:
+        outs = c.outputs(last) if c.outputs is not None else {"out": last}
+        suffix = f"_rank{rank}" if world > 1 else ""
+        dump_outputs(args.dump_outputs, {k + suffix: v for k, v in outs.items()}, budget=DUMP_BYTES // world)
+        del outs
+    del last
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

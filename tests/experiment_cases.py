@@ -1,9 +1,9 @@
 """Shared definition of the end-to-end ``experiment()`` parity cases (SURVEY.md 8c K5).
 
-Used by ``tests/golden/make_experiment_golden.py`` (runs the UNMODIFIED reference driver on the CPU
-oracle shim in the build container and commits the accuracies as ``tests/golden/experiment_acc.json``)
-and by ``tests/test_z_gpu_experiment.py`` (runs the same calls on a B200 through the product shim,
-the reference coming from the git-ignored snapshot ``baseline/_ref``).
+Used by ``tests/golden/make_experiment_golden.py``, which runs the UNMODIFIED reference driver on the CPU
+oracle shim and records the accuracies as ``tests/golden/experiment_acc.json`` (it needs the original
+package, which this repository does not contain); ``tests/test_z_gpu_experiment.py`` takes its graphs
+from ``make_data``.
 
 The stochastic forwards of the reference (dropout inside DAGNN / FAGCN / GIN / SuperGAT, SuperGAT's
 edge sampling; SURVEY Appendix B5) draw from different RNG streams on CPU and CUDA, so those cases
@@ -17,17 +17,6 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN_JSON = os.path.join(ROOT, "tests", "golden", "experiment_acc.json")
-
-
-def reference_root():
-    """Directory to put on sys.path so that ``import rgb_experiment`` finds the unmodified reference:
-    the snapshot that travels to the GPU box, else the build container's read-only checkout."""
-    snap = os.path.join(ROOT, "baseline", "_ref")
-    if os.path.isdir(os.path.join(snap, "rgb_experiment")):
-        return snap
-    if os.path.isdir("/root/reference/rgb_experiment"):
-        return "/root/reference"
-    return None
 
 
 def make_data(shape: str):
