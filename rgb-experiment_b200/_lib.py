@@ -147,6 +147,13 @@ def require_cuda(t: torch.Tensor, name: str):
                            "this package has no CPU path")
 
 
+def require_f32(t: torch.Tensor, name: str):
+    """The attention / edge-score kernels read every operand as float32: refuse any other dtype before a launch
+    instead of reinterpreting its bytes."""
+    if t.dtype != torch.float32:
+        raise RuntimeError(f"rgb-experiment_b200: {name} takes float32 only (got {t.dtype})")
+
+
 def dtype_code(t: torch.Tensor) -> int:
     if t.dtype == torch.float32:
         return F32

@@ -394,6 +394,7 @@ class Graph:
         return out
 
     def to_edge_order(self, csr_vals: torch.Tensor, transpose: bool = False) -> torch.Tensor:
+        _lib.require_f32(csr_vals, "to_edge_order")
         csr = self.bwd if transpose else self.fwd
         cv = csr_vals.contiguous()
         H = 1 if cv.dim() == 1 else cv.size(1)

@@ -215,8 +215,8 @@ class _PropagateWeighted(torch.autograd.Function):
         dx = dw = None
         if ctx.needs_input_grad[0]:
             dx = spmm_raw(g.bwd, dy, g.to_csr_order(w, transpose=True))
-        if ctx.needs_input_grad[1]:
-            dw = g.to_edge_order(sddmm(g.fwd, dy, x, 1, dy.size(1))).view_as(w)
+        if ctx.needs_input_grad[1]:       # the SDDMM kernel is fp32-only: a bf16 dy / x widens exactly
+            dw = g.to_edge_order(sddmm(g.fwd, dy.float(), x.float(), 1, dy.size(1))).view_as(w).to(w.dtype)
         return dx, dw, None
 
 
@@ -350,7 +350,7 @@ def label_propagation(graph: Graph, out0: torch.Tensor, num_layers: int, alpha: 
     keep = [xb]
     if reset_mask is not None:
         m = reset_mask.to(torch.uint8).contiguous()
-        rv, ldr = as_rows(reset_val)
+        rv, ldr = as_rows(reset_val.float())      # the epilogue reads reset rows as float32 whatever the feature dtype
         kw = dict(reset_mask=m, reset_val=rv, ld_reset=ldr, reset_when=RESET_AFTER_CLAMP)
         keep += [m, rv]
         clamp = None
@@ -393,6 +393,8 @@ def pta_label_propagation(graph: Graph, labels: torch.Tensor, idx: torch.Tensor,
 # ------------------------------------------------------------------------------------------
 def sddmm(csr: CSR, A: torch.Tensor, B: torch.Tensor, H: int, Cc: int) -> torch.Tensor:
     """out[k,h] = <A[row_i,h,:], B[col[k],h,:]> in CSR order."""
+    _lib.require_f32(A, "sddmm A")
+    _lib.require_f32(B, "sddmm B")
     Ab, lda = as_rows(A)
     Bb, ldb = as_rows(B)
     out = torch.empty((csr.nnz, H), dtype=torch.float32, device=A.device)
@@ -407,6 +409,8 @@ def _edge_call(fn_name, csr: CSR, *args):
 
 
 def spmm_heads_raw(csr: CSR, w: torch.Tensor, X: torch.Tensor, H: int, Cc: int) -> torch.Tensor:
+    _lib.require_f32(w, "spmm_heads w")
+    _lib.require_f32(X, "spmm_heads X")
     Xb, ldx = as_rows(X)
     out, ldo = alloc_rows(csr.n_rows, H * Cc, torch.float32, X.device)
     _edge_call("rgbmp_spmm_heads", csr, ptr(w.contiguous()), ptr(Xb), ldx, H, Cc, ptr(out), ldo)
@@ -414,6 +418,7 @@ def spmm_heads_raw(csr: CSR, w: torch.Tensor, X: torch.Tensor, H: int, Cc: int) 
 
 
 def seg_sum_raw(csr: CSR, vals: torch.Tensor, H: int) -> torch.Tensor:
+    _lib.require_f32(vals, "seg_sum")
     out = torch.empty((csr.n_rows, H), dtype=torch.float32, device=vals.device)
     _edge_call("rgbmp_seg_sum", csr, ptr(vals.contiguous()), H, ptr(out))
     return out
@@ -443,6 +448,8 @@ class _UAddV(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, u, v, graph: Graph):
+        _lib.require_f32(u, "u_add_v u")
+        _lib.require_f32(v, "u_add_v v")
         ctx.graph = graph
         H = u.size(1)
         out = torch.empty((graph.nnz, H), dtype=torch.float32, device=u.device)
@@ -464,6 +471,7 @@ class _SegSoftmax(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, e, graph: Graph):
+        _lib.require_f32(e, "edge_softmax")
         ctx.graph = graph
         e = e.contiguous()
         out = torch.empty_like(e)
@@ -557,6 +565,8 @@ class _Att(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, a_nbr, a_own, graph: Graph, score: int, H: int, Cc: int, slope: float, drop_csr):
         _lib.require_cuda(x, "x")
+        for t, nm in ((x, "x"), (a_nbr, "a_nbr"), (a_own, "a_own")):
+            _lib.require_f32(t, f"fused attention {nm}")
         xb, ldx = _rows_zero_padded(x)
         a_n, a_o = a_nbr.contiguous().view(-1, H), a_own.contiguous().view(-1, H)
         N, dev = graph.N, x.device

@@ -2,7 +2,7 @@
 """The small-graph workout for memory-safety checking (SURVEY.md section 5 "race detection"; VERDICT r1 item 7):
 every kernel family of librgbmp.so on the edge-case graphs of tests/helpers.CASES -- graph build (all three radix
 variants), loop edits, coalesce, locality groups, SpMM (vector, scalar / unaligned, bf16, long rows, every epilogue),
-K-hop, fused attention forward + backward for GAT / SuperGAT-MX / FAConv (all head shape classes, long rows), the
+K-hop (fp32 and bf16), fused attention forward + backward for GAT / SuperGAT-MX / FAConv (all head shape classes, long rows), the
 generic edge-score kernels.  Every result and gradient is checked to be finite.
 
 Meant for   compute-sanitizer --tool memcheck|racecheck|initcheck python tools/sanitize_run.py   (one tool per call).
@@ -106,6 +106,21 @@ def main():
                         P._lib.lib().rgbmp_set_push_bulk(oldb)
             else:
                 fin(P.ops.spmm_raw(g.fwd, x, None))
+                # bf16 K-hop (always the K-launch driver), every epilogue form, reset rows (read as fp32)
+                d = g.dinv()
+                xb, ldx = P.ops.as_rows(x)
+                m = torch.zeros(n, dtype=torch.bool, device=dev)
+                m[::3] = True
+                m8, rv = m.to(torch.uint8), x.float()
+                fin(P.ops.spmm_raw(g.fwd, x, g.gcn_val(False), ep=P.ops.make_epilogue(
+                    row_scale=d, a=0.9, b=0.1, T=xb, ldt=ldx, clamp=(-1.0, 1.0), acc_in=xb, ld_acc=ldx,
+                    reset_mask=m8, reset_val=rv, ld_reset=F, reset_when=2), keep=(xb, d, m8, rv)))
+                for fold in (False, True):
+                    fin(P.ops.appnp(x, g, 3, 0.1, fold))
+                    fin(P.ops.gcn_power(x, g, 2, fold))
+                    fin(P.ops.label_propagation(gn, x, 3, 0.8, clamp=(-1.0, 1.0), fold=fold))
+                    fin(P.ops.label_propagation(gn, x, 3, 0.8, reset_mask=m, reset_val=x, fold=fold))
+                fin(P.ops.dagnn_hops(x, g, 3))
             n_calls += 8
         for H, C in ((8, 8), (1, 41), (3, 5), (5, 32), (2, 47)):
             xp = (torch.randn(n, H * C, device=dev, generator=gen) * 0.5).requires_grad_(True)
