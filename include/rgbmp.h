@@ -348,6 +348,40 @@ int rgbmp_att_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int scor
                        float* dX, int64_t lddx, float* dXf, int64_t lddxf, float* da_nbr, float* da_own,
                        void* ws, size_t ws_bytes, int device, void* stream);
 
+/* Attention dropout generated inside the kernels (csrc/philox.cuh): no mask tensor exists.  For edge e (its id in
+ * the edited edge list) and head h (FA: h = 0):
+ *   u = Philox4x32-10(counter = (e, h, 0, 0), key = (seed & 0xffffffff, seed >> 32)).word0
+ *   multiplier = (u < thresh) ? 0 : scale,   thresh = floor(p * 2^32),  scale = float32(1 / (1 - p))
+ * p == 1 is passed as thresh = 0xffffffff, scale = 0 (every multiplier 0).  The multiplier is applied where the
+ * explicit `drop` mask is, with the same operands: a fused call is bit-identical to the explicit-mask call fed the
+ * mask rgbmp_dropout_mask writes for the same seed.  `seed` is read on the device (no host synchronisation). */
+typedef struct rgbmp_dropout {
+  const int64_t* seed;    /* device pointer to one int64 */
+  const int32_t* eid;     /* [nnz] edge id of every forward-CSR entry */
+  const int32_t* eid_t;   /* [nnz] edge id of every transpose-CSR entry; backward only */
+  uint32_t thresh;
+  float    scale;
+} rgbmp_dropout_t;
+
+/* = rgbmp_att_forward with the dropout descriptor in place of `drop` (d->eid required). */
+int rgbmp_att_forward_dropout(const rgbmp_graph_t* g, int score, const float* X, int64_t ldx,
+                              const float* a_nbr, const float* a_own, const float* dinv, int H, int C, float slope,
+                              const rgbmp_dropout_t* d, float* out, int64_t ldo, float* rowmax, float* rowsum,
+                              float* out2, int64_t ldo2, float* rowq,
+                              void* ws, size_t ws_bytes, int device, void* stream);
+/* = rgbmp_att_backward with the dropout descriptor in place of `drop, tpos` (d->eid_t required; MX also d->eid).
+ * The transpose pass streams eid_t: no tpos, no random gather. */
+int rgbmp_att_backward_dropout(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int score, const float* X, int64_t ldx,
+                               const float* a_nbr, const float* a_own, const float* dinv, int H, int C, float slope,
+                               const rgbmp_dropout_t* d,
+                               const float* rowmax, const float* rowsum, const float* rowq,
+                               const float* out, int64_t ldo, const float* out2, int64_t ldo2,
+                               const float* dout, int64_t ldd,
+                               float* dX, int64_t lddx, float* dXf, int64_t lddxf, float* da_nbr, float* da_own,
+                               void* ws, size_t ws_bytes, int device, void* stream);
+/* out[e*H + h] = the multiplier of edge e, head h, in EDGE order [nnz, H] (the mask of the unfused paths). */
+int rgbmp_dropout_mask(const rgbmp_dropout_t* d, int64_t nnz, int H, float* out, int device, void* stream);
+
 /* S[i,h] = sum_c A[i,h*C+c]*B[i,h*C+c] */
 int rgbmp_rowdot(const float* A, int64_t lda, const float* B, int64_t ldb, int64_t n_rows,
                  int H, int C, float* S, int device, void* stream);

@@ -32,6 +32,11 @@ class Epilogue(C.Structure):
                 ("peer_out", c_vp * 8), ("n_peers", c_i32), ("peer_row0", c_i64), ("ld_peer", c_i64)]
 
 
+class DropoutStruct(C.Structure):
+    """rgbmp_dropout_t"""
+    _fields_ = [("seed", c_vp), ("eid", c_vp), ("eid_t", c_vp), ("thresh", C.c_uint32), ("scale", c_f32)]
+
+
 _lib = None
 
 
@@ -45,7 +50,7 @@ def lib():
             f"rgb-experiment_b200: {LIB_PATH} is missing -- build it with "
             "`python rgb-experiment_b200/build.py` (nvcc, sm_100a). There is no CPU fallback.")
     L = C.CDLL(LIB_PATH)
-    GP, EP = C.POINTER(GraphStruct), C.POINTER(Epilogue)
+    GP, EP, DP = C.POINTER(GraphStruct), C.POINTER(Epilogue), C.POINTER(DropoutStruct)
     sig = {
         "rgbmp_version": (C.c_int, []),
         "rgbmp_last_error": (C.c_char_p, []),
@@ -90,6 +95,12 @@ def lib():
         "rgbmp_att_backward": (C.c_int, [GP, GP, C.c_int, c_vp, c_i64, c_vp, c_vp, c_vp, C.c_int, C.c_int, c_f32, c_vp, c_vp,
                                          c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64,
                                          c_vp, c_vp, c_vp, c_sz, C.c_int, c_vp]),
+        "rgbmp_att_forward_dropout": (C.c_int, [GP, C.c_int, c_vp, c_i64, c_vp, c_vp, c_vp, C.c_int, C.c_int, c_f32, DP, c_vp,
+                                                c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_sz, C.c_int, c_vp]),
+        "rgbmp_att_backward_dropout": (C.c_int, [GP, GP, C.c_int, c_vp, c_i64, c_vp, c_vp, c_vp, C.c_int, C.c_int, c_f32, DP,
+                                                 c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp,
+                                                 c_i64, c_vp, c_vp, c_vp, c_sz, C.c_int, c_vp]),
+        "rgbmp_dropout_mask": (C.c_int, [DP, c_i64, C.c_int, c_vp, C.c_int, c_vp]),
         "rgbmp_coalesce_workspace_bytes": (c_sz, [c_i64, c_i64, C.c_int]),
         "rgbmp_coalesce": (C.c_int, [c_vp, c_vp, c_i64, c_i64, C.c_int, c_vp, c_vp, c_vp, c_vp, c_sz, C.c_int, c_vp]),
         "rgbmp_peer_alloc": (C.c_int, [c_sz, c_vp, c_vp, C.c_int]),

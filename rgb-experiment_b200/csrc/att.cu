@@ -29,6 +29,7 @@
 //         orientation anyway (forward CSR: dX_i += dlogit x_j, da_r; transpose CSR: dX_j += alpha dout_i + dlogit x_i, da_l).
 #include <stdlib.h>
 #include "common.cuh"
+#include "philox.cuh"
 
 namespace rgbmp {
 
@@ -97,6 +98,12 @@ struct AttParams {
   // attention dropout: keep-mask / (1-p) in forward-CSR order [nnz,H]; tpos maps transpose entries to it
   const float* drop;
   const int32_t* tpos;
+  // fused attention dropout (the DR instantiations): multiplier of entry k = dropout_mult(seed, eid[k], head),
+  // eid = edge id of every entry of THIS pass's CSR (forward CSR or transpose CSR), read as a stream
+  const int64_t* seed;
+  const int32_t* eid;
+  uint32_t thresh;
+  float dscale;
   // outputs
   float* out;  int64_t ldo;           // fwd: out ; bwd: dX of the own row
   float* out2; int64_t ldo2;          // fwd TRAIN: second aggregate (P / Q)
@@ -135,6 +142,16 @@ __device__ __forceinline__ Lane lane_of(const AttParams& p, int gl) {
   L.h = (p.H == 1) ? 0 : L.f / p.C;
   L.lead = L.nact > 0 && (p.H == 1 ? gl == 0 : (L.f % p.C) == 0);
   return L;
+}
+
+// the key is built once per thread from the device-resident seed; the hash runs per (entry, head)
+template <bool DR>
+__device__ __forceinline__ PhiloxKey drop_key(const AttParams& p) {
+  if constexpr (DR) return philox_key((uint64_t)__ldg(p.seed));
+  else return PhiloxKey{0u, 0u};
+}
+__device__ __forceinline__ float drop_mult(const AttParams& p, PhiloxKey key, int64_t k, int h) {
+  return dropout_mult(key, (uint32_t)__ldg(p.eid + k), (uint32_t)h, p.thresh, p.dscale);
 }
 
 // sum over the LPH lanes of a head (all lanes of the warp execute)
@@ -200,17 +217,18 @@ __device__ __forceinline__ void lds_ids(const int32_t* p, uint32_t (&c)[N]) {
   }
 }
 
-template <int SC, bool TRAIN, int UU>
+template <int SC, bool TRAIN, int UU, bool DR>
 __device__ __forceinline__ void fwd_consume(const AttParams& p, const float4 (&x)[UU][2], const float (&sn)[UU], const float (&dn)[UU],
                                             int nvalid, int64_t kbase, const Lane& L, float so, float d_own,
-                                            const float4 (&xi)[2], FwdState& st) {
+                                            const float4 (&xi)[2], PhiloxKey key, FwdState& st) {
   if constexpr (SC == SC_FA) {
 #pragma unroll
     for (int u = 0; u < UU; ++u) {
       if (u < nvalid) {
         const float t = tanhf(sn[u] + so);
         float wgt = dn[u] * d_own;
-        if (p.drop) wgt *= __ldg(p.drop + (kbase + u));
+        if constexpr (DR) wgt *= drop_mult(p, key, kbase + u, 0);
+        else if (p.drop) wgt *= __ldg(p.drop + (kbase + u));
         const float w = t * wgt;
         fma4(st.acc[0], w, x[u][0]);
         fma4(st.acc[1], w, x[u][1]);
@@ -251,7 +269,9 @@ __device__ __forceinline__ void fwd_consume(const AttParams& p, const float4 (&x
       if (u < nvalid) {
         const float pe = ex2(e[u] - st.m);
         st.s += pe;
-        const float mu = p.drop ? __ldg(p.drop + (kbase + u) * p.H + L.h) : 1.0f;
+        float mu;
+        if constexpr (DR) mu = drop_mult(p, key, kbase + u, L.h);
+        else mu = p.drop ? __ldg(p.drop + (kbase + u) * p.H + L.h) : 1.0f;
         const float w = pe * mu;
         fma4(st.acc[0], w, x[u][0]);
         fma4(st.acc[1], w, x[u][1]);
@@ -268,9 +288,9 @@ __device__ __forceinline__ void fwd_consume(const AttParams& p, const float4 (&x
 }
 
 // UU edges per step; PIPE: software-pipelined full batches (the gathers of step j+UU fly while step j is consumed)
-template <int SC, bool TRAIN, int G, int UU, bool PIPE>
+template <int SC, bool TRAIN, int G, int UU, bool PIPE, bool DR>
 __device__ __forceinline__ void fwd_range(const AttParams& p, int64_t k0, int64_t k1, int gl, const Lane& L, float so,
-                                          float d_own, const float4 (&xi)[2], int32_t* sm_ids, FwdState& st) {
+                                          float d_own, const float4 (&xi)[2], PhiloxKey key, int32_t* sm_ids, FwdState& st) {
   const int len = (k1 > k0) ? (int)(k1 - k0) : 0;
   const int maxlen = __reduce_max_sync(FULLMASK, len);
   if (maxlen == 0) return;
@@ -319,7 +339,7 @@ __device__ __forceinline__ void fwd_range(const AttParams& p, int64_t k0, int64_
           lds_ids<UU>(gids + jn, c);
 #pragma unroll
           for (int u = 0; u < UU; ++u) gather(c[u], xn[u], asn[u], dnn[u]);
-          fwd_consume<SC, TRAIN, UU>(p, x, as, dn, UU, k0 + off + j, L, so, d_own, xi, st);
+          fwd_consume<SC, TRAIN, UU, DR>(p, x, as, dn, UU, k0 + off + j, L, so, d_own, xi, key, st);
 #pragma unroll
           for (int u = 0; u < UU; ++u) {
             as[u] = asn[u];
@@ -337,7 +357,7 @@ __device__ __forceinline__ void fwd_range(const AttParams& p, int64_t k0, int64_
           lds_ids<UU>(gids + j, c);
 #pragma unroll
           for (int u = 0; u < UU; ++u) gather(c[u], x[u], as[u], dn[u]);
-          fwd_consume<SC, TRAIN, UU>(p, x, as, dn, UU, k0 + off + j, L, so, d_own, xi, st);
+          fwd_consume<SC, TRAIN, UU, DR>(p, x, as, dn, UU, k0 + off + j, L, so, d_own, xi, key, st);
         }
       }
     } else {
@@ -352,7 +372,7 @@ __device__ __forceinline__ void fwd_range(const AttParams& p, int64_t k0, int64_
         for (int u = 0; u < UU; ++u) gather(c[u], x[u], as[u], dn[u]);
         int nv = nb - j;
         nv = nv < 0 ? 0 : (nv > UU ? UU : nv);
-        fwd_consume<SC, TRAIN, UU>(p, x, as, dn, nv, k0 + off + j, L, so, d_own, xi, st);
+        fwd_consume<SC, TRAIN, UU, DR>(p, x, as, dn, nv, k0 + off + j, L, so, d_own, xi, key, st);
       }
     }
   }
@@ -374,7 +394,7 @@ __device__ __forceinline__ void fwd_init(FwdState& st) {
   st.acc[0] = st.acc[1] = st.acc2[0] = st.acc2[1] = zero4();
 }
 
-template <int SC, bool TRAIN, int G, int UU, bool PIPE>
+template <int SC, bool TRAIN, int G, int UU, bool PIPE, bool DR>
 __global__ void __launch_bounds__(ATT_THREADS, fwd_minb<SC, TRAIN>()) att_fwd_rows_kernel(const AttParams p) {
   __shared__ __align__(16) int32_t sm_ids[ATT_THREADS];
   const int gl = threadIdx.x % G;
@@ -390,7 +410,7 @@ __global__ void __launch_bounds__(ATT_THREADS, fwd_minb<SC, TRAIN>()) att_fwd_ro
   }
   FwdState st;
   fwd_init(st);
-  fwd_range<SC, TRAIN, G, UU, PIPE>(p, k0, k1, gl, L, so, d_own, xi, sm_ids, st);
+  fwd_range<SC, TRAIN, G, UU, PIPE, DR>(p, k0, k1, gl, L, so, d_own, xi, drop_key<DR>(p), sm_ids, st);
   if (!live || L.nact == 0) return;
   float inv = 1.0f;
   if constexpr (SC != SC_FA) inv = (k1 > k0) ? 1.0f / (st.s + 1e-16f) : 0.f;
@@ -416,7 +436,7 @@ __global__ void __launch_bounds__(ATT_THREADS, fwd_minb<SC, TRAIN>()) att_fwd_ro
 
 // long rows: one CTA per (work item, head tile); the CTA's Q groups take contiguous sub-ranges, their states
 // are merged through shared memory in group order
-template <int SC, bool TRAIN, int G, int UU, bool PIPE>
+template <int SC, bool TRAIN, int G, int UU, bool PIPE, bool DR>
 __global__ void __launch_bounds__(ATT_THREADS, fwd_minb<SC, TRAIN>()) att_fwd_long_kernel(const AttParams p) {
   constexpr int Q = ATT_THREADS / G;
   constexpr int W = G * 8;
@@ -435,7 +455,7 @@ __global__ void __launch_bounds__(ATT_THREADS, fwd_minb<SC, TRAIN>()) att_fwd_lo
   if constexpr (SC == SC_MX) load_own(p.Xo, p.ldo_, row, L, xi);
   FwdState st;
   fwd_init(st);
-  fwd_range<SC, TRAIN, G, UU, PIPE>(p, k0, k1, gl, L, so, d_own, xi, sm_ids, st);
+  fwd_range<SC, TRAIN, G, UU, PIPE, DR>(p, k0, k1, gl, L, so, d_own, xi, drop_key<DR>(p), sm_ids, st);
 #pragma unroll
   for (int v = 0; v < 2; ++v) {
     const bool act = v < L.nact;
@@ -546,6 +566,16 @@ __global__ void __launch_bounds__(256) att_fwd_combine_kernel(const AttParams p)
   }
 }
 
+// out[e*H + h] = dropout multiplier of edge e, head h (edge order): the mask of the unfused paths and of the tests
+__global__ void __launch_bounds__(256) att_dropout_mask_kernel(const int64_t* __restrict__ seed, int64_t n, int H,
+                                                              uint32_t thresh, float scale, float* __restrict__ out) {
+  const PhiloxKey key = philox_key((uint64_t)__ldg(seed));
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t e = t / H;
+    out[t] = dropout_mult(key, (uint32_t)e, (uint32_t)(t - e * H), thresh, scale);
+  }
+}
+
 // scaled copies of the score terms: out[i] = in[i] * log2(e)
 __global__ void __launch_bounds__(256) att_scale_kernel(const float* __restrict__ in, int64_t n, float* __restrict__ out) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -597,9 +627,10 @@ att_bwd_prep_kernel(const float* __restrict__ dout, int64_t ldd, const float* __
 }
 
 // ---- transpose pass: rows = sources j, neighbours = targets i -----------------------------------------------
-template <int SC, int G>
+template <int SC, int G, bool DR>
 __device__ __forceinline__ void bwdT_range(const AttParams& p, int64_t k0, int64_t k1, int gl, const Lane& L, float so2,
-                                           float d_own, const float4 (&xj)[2], int32_t* sm_ids, float4 (&acc)[2], float& das) {
+                                           float d_own, const float4 (&xj)[2], PhiloxKey key, int32_t* sm_ids, float4 (&acc)[2],
+                                           float& das) {
   constexpr int UB = (SC == SC_FA && G >= 8) ? 4 : 2;     // edges per step: 4 only where it measured faster (FAConv: 11.8 -> 11.05 ms fwd+bwd;
                                                           // GAT 6.6 -> 6.8, MX does not fit the registers)
   const int len = (k1 > k0) ? (int)(k1 - k0) : 0;
@@ -652,7 +683,8 @@ __device__ __forceinline__ void bwdT_range(const AttParams& p, int64_t k0, int64
         if constexpr (SC == SC_MX) sg = sigmoidf(head_sum(dot4(x2[u][0], xj[0]) + dot4(x2[u][1], xj[1]), p.LPH));
         if (j + u < nb) {
           float mu = 1.0f;
-          if (p.drop) mu = __ldg(p.drop + (int64_t)__ldg(p.tpos + k0 + off + j + u) * p.H + L.h);
+          if constexpr (DR) mu = drop_mult(p, key, k0 + off + j + u, L.h);
+          else if (p.drop) mu = __ldg(p.drop + (int64_t)__ldg(p.tpos + k0 + off + j + u) * p.H + L.h);
           if constexpr (SC == SC_FA) {
             const float t = tanhf(so2 + st[u].x);
             const float wgt = d_own * st[u].y * mu;
@@ -688,7 +720,7 @@ constexpr int bwdT_minb() {
   return RGBMP_ATT_OCC >= 1 ? (SC == SC_MX ? 3 : (SC == SC_GAT ? 4 : 3)) : (SC == SC_MX ? 2 : 3);
 }
 
-template <int SC, int G>
+template <int SC, int G, bool DR>
 __global__ void __launch_bounds__(ATT_THREADS, bwdT_minb<SC>()) att_bwdT_rows_kernel(const AttParams p) {
   __shared__ __align__(16) int32_t sm_ids[ATT_THREADS];
   const int gl = threadIdx.x % G;
@@ -703,7 +735,7 @@ __global__ void __launch_bounds__(ATT_THREADS, bwdT_minb<SC>()) att_bwdT_rows_ke
     load_own(p.Xo, p.ldo_, row, L, xj);
   }
   float das = 0.f;
-  bwdT_range<SC, G>(p, k0, k1, gl, L, so2, d_own, xj, sm_ids, acc, das);
+  bwdT_range<SC, G, DR>(p, k0, k1, gl, L, so2, d_own, xj, drop_key<DR>(p), sm_ids, acc, das);
   if (!live || L.nact == 0) return;
 #pragma unroll
   for (int v = 0; v < 2; ++v) {
@@ -749,7 +781,7 @@ __device__ __forceinline__ void bwd_long_merge(const AttParams& p, int gl, int q
   }
 }
 
-template <int SC, int G>
+template <int SC, int G, bool DR>
 __global__ void __launch_bounds__(ATT_THREADS, bwdT_minb<SC>()) att_bwdT_long_kernel(const AttParams p) {
   constexpr int Q = ATT_THREADS / G;
   __shared__ __align__(16) int32_t sm_ids[ATT_THREADS];
@@ -765,7 +797,7 @@ __global__ void __launch_bounds__(ATT_THREADS, bwdT_minb<SC>()) att_bwdT_long_ke
   float4 xj[2], acc[2] = {zero4(), zero4()};
   load_own(p.Xo, p.ldo_, row, L, xj);
   float das = 0.f;
-  bwdT_range<SC, G>(p, k0, k1, gl, L, so2, d_own, xj, sm_ids, acc, das);
+  bwdT_range<SC, G, DR>(p, k0, k1, gl, L, so2, d_own, xj, drop_key<DR>(p), sm_ids, acc, das);
   bwd_long_merge<G>(p, gl, q, L, acc, das, sm_acc, sm_s);
 }
 
@@ -789,10 +821,10 @@ __global__ void __launch_bounds__(256) att_bwd_combine_kernel(const AttParams p)
 
 // ---- MX forward-orientation pass: rows = targets i, neighbours = sources j ----------------------------------
 //   dXf_i = sum_j dlogit_ij x_j ;  da_r[i] = sum_j draw_ij * s_ij
-template <int G>
+template <int G, bool DR>
 __device__ __forceinline__ void bwdF_range(const AttParams& p, int64_t k0, int64_t k1, int gl, const Lane& L, const float4 st_own,
-                                           const float4 (&xi)[2], const float4 (&di)[2], int32_t* sm_ids, float4 (&acc)[2],
-                                           float& dar) {
+                                           const float4 (&xi)[2], const float4 (&di)[2], PhiloxKey key, int32_t* sm_ids,
+                                           float4 (&acc)[2], float& dar) {
   const int len = (k1 > k0) ? (int)(k1 - k0) : 0;
   const int maxlen = __reduce_max_sync(FULLMASK, len);
   if (maxlen == 0) return;
@@ -834,7 +866,9 @@ __device__ __forceinline__ void bwdF_range(const AttParams& p, int64_t k0, int64
         const float dot = head_sum(dot4(di[0], x[u][0]) + dot4(di[1], x[u][1]), p.LPH);              // <dout_i, x_j>
         const float sg = sigmoidf(head_sum(dot4(xi[0], x[u][0]) + dot4(xi[1], x[u][1]), p.LPH));     // sigmoid(<x_i, x_j>)
         if (j + u < nb) {
-          const float mu = p.drop ? __ldg(p.drop + (k0 + off + j + u) * p.H + L.h) : 1.0f;
+          float mu;
+          if constexpr (DR) mu = drop_mult(p, key, k0 + off + j + u, L.h);
+          else mu = p.drop ? __ldg(p.drop + (k0 + off + j + u) * p.H + L.h) : 1.0f;
           const float uu = as[u] + st_own.x;
           const float raw = uu * sg;
           const float alpha = ex2(leaky_relu(raw, p.slope) - st_own.y) * st_own.z;
@@ -849,7 +883,7 @@ __device__ __forceinline__ void bwdF_range(const AttParams& p, int64_t k0, int64
   }
 }
 
-template <int G>
+template <int G, bool DR>
 __global__ void __launch_bounds__(ATT_THREADS, RGBMP_ATT_OCC >= 1 ? 3 : 2) att_bwdF_rows_kernel(const AttParams p) {
   __shared__ __align__(16) int32_t sm_ids[ATT_THREADS];
   const int gl = threadIdx.x % G;
@@ -864,7 +898,7 @@ __global__ void __launch_bounds__(ATT_THREADS, RGBMP_ATT_OCC >= 1 ? 3 : 2) att_b
     st_own = __ldg(p.stats + row * p.H + L.h);
   }
   float dar = 0.f;
-  bwdF_range<G>(p, k0, k1, gl, L, st_own, xi, di, sm_ids, acc, dar);
+  bwdF_range<G, DR>(p, k0, k1, gl, L, st_own, xi, di, drop_key<DR>(p), sm_ids, acc, dar);
   if (!live || L.nact == 0) return;
 #pragma unroll
   for (int v = 0; v < 2; ++v)
@@ -872,7 +906,7 @@ __global__ void __launch_bounds__(ATT_THREADS, RGBMP_ATT_OCC >= 1 ? 3 : 2) att_b
   if (L.lead) p.ds[row * p.H + L.h] = dar;
 }
 
-template <int G>
+template <int G, bool DR>
 __global__ void __launch_bounds__(ATT_THREADS, RGBMP_ATT_OCC >= 1 ? 3 : 2) att_bwdF_long_kernel(const AttParams p) {
   constexpr int Q = ATT_THREADS / G;
   __shared__ __align__(16) int32_t sm_ids[ATT_THREADS];
@@ -887,7 +921,7 @@ __global__ void __launch_bounds__(ATT_THREADS, RGBMP_ATT_OCC >= 1 ? 3 : 2) att_b
   load_own(p.Do, p.lddo, row, L, di);
   const float4 st_own = __ldg(p.stats + row * p.H + L.h);
   float dar = 0.f;
-  bwdF_range<G>(p, k0, k1, gl, L, st_own, xi, di, sm_ids, acc, dar);
+  bwdF_range<G, DR>(p, k0, k1, gl, L, st_own, xi, di, drop_key<DR>(p), sm_ids, acc, dar);
   bwd_long_merge<G>(p, gl, q, L, acc, dar, sm_acc, sm_s);
 }
 
@@ -978,19 +1012,19 @@ static int att_fwd_variant() {
   return v;
 }
 
-template <int SC, bool TRAIN, int UU, bool PIPE>
+template <int SC, bool TRAIN, int UU, bool PIPE, bool DR>
 static int launch_fwd_v(const AttParams& p, const Shape& s, cudaStream_t st) {
   const int HC = p.H * p.C;
   dim3 grid_rows((unsigned)ceil_div(p.n_rows, ATT_THREADS / s.G), (unsigned)s.tiles);
-  ATT_G_SWITCH(s.G, (att_fwd_rows_kernel<SC, TRAIN, 4, UU, PIPE><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
-               (att_fwd_rows_kernel<SC, TRAIN, 8, UU, PIPE><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
-               (att_fwd_rows_kernel<SC, TRAIN, 16, UU, PIPE><<<grid_rows, ATT_THREADS, 0, st>>>(p)))
+  ATT_G_SWITCH(s.G, (att_fwd_rows_kernel<SC, TRAIN, 4, UU, PIPE, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
+               (att_fwd_rows_kernel<SC, TRAIN, 8, UU, PIPE, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
+               (att_fwd_rows_kernel<SC, TRAIN, 16, UU, PIPE, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)))
   RGBMP_LAUNCH_CHECK("att_fwd_rows_kernel");
   if (p.n_items > 0) {
     dim3 grid_items((unsigned)p.n_items, (unsigned)s.tiles);
-    ATT_G_SWITCH(s.G, (att_fwd_long_kernel<SC, TRAIN, 4, UU, PIPE><<<grid_items, ATT_THREADS, 0, st>>>(p)),
-                 (att_fwd_long_kernel<SC, TRAIN, 8, UU, PIPE><<<grid_items, ATT_THREADS, 0, st>>>(p)),
-                 (att_fwd_long_kernel<SC, TRAIN, 16, UU, PIPE><<<grid_items, ATT_THREADS, 0, st>>>(p)))
+    ATT_G_SWITCH(s.G, (att_fwd_long_kernel<SC, TRAIN, 4, UU, PIPE, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
+                 (att_fwd_long_kernel<SC, TRAIN, 8, UU, PIPE, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
+                 (att_fwd_long_kernel<SC, TRAIN, 16, UU, PIPE, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)))
     RGBMP_LAUNCH_CHECK("att_fwd_long_kernel");
     att_fwd_combine_kernel<SC, TRAIN><<<(unsigned)ceil_div(p.n_long * HC, 256), 256, 0, st>>>(p);
     RGBMP_LAUNCH_CHECK("att_fwd_combine_kernel");
@@ -998,28 +1032,30 @@ static int launch_fwd_v(const AttParams& p, const Shape& s, cudaStream_t st) {
   return 0;
 }
 
-template <int SC, bool TRAIN>
+// the fused-dropout forward exists in the default loop variant only
+template <int SC, bool TRAIN, bool DR>
 static int launch_fwd(const AttParams& p, const Shape& s, cudaStream_t st) {
+  if constexpr (DR) return launch_fwd_v<SC, TRAIN, 2, false, true>(p, s, st);
   switch (att_fwd_variant()) {
-    case 1: return launch_fwd_v<SC, TRAIN, 4, false>(p, s, st);
-    case 0: return launch_fwd_v<SC, TRAIN, 2, true>(p, s, st);
-    default: return launch_fwd_v<SC, TRAIN, 2, false>(p, s, st);
+    case 1: return launch_fwd_v<SC, TRAIN, 4, false, false>(p, s, st);
+    case 0: return launch_fwd_v<SC, TRAIN, 2, true, false>(p, s, st);
+    default: return launch_fwd_v<SC, TRAIN, 2, false, false>(p, s, st);
   }
 }
 
-template <int SC>
+template <int SC, bool DR>
 static int launch_bwdT(const AttParams& p, const Shape& s, cudaStream_t st) {
   const int HC = p.H * p.C;
   dim3 grid_rows((unsigned)ceil_div(p.n_rows, ATT_THREADS / s.G), (unsigned)s.tiles);
-  ATT_G_SWITCH(s.G, (att_bwdT_rows_kernel<SC, 4><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
-               (att_bwdT_rows_kernel<SC, 8><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
-               (att_bwdT_rows_kernel<SC, 16><<<grid_rows, ATT_THREADS, 0, st>>>(p)))
+  ATT_G_SWITCH(s.G, (att_bwdT_rows_kernel<SC, 4, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
+               (att_bwdT_rows_kernel<SC, 8, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
+               (att_bwdT_rows_kernel<SC, 16, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)))
   RGBMP_LAUNCH_CHECK("att_bwdT_rows_kernel");
   if (p.n_items > 0) {
     dim3 grid_items((unsigned)p.n_items, (unsigned)s.tiles);
-    ATT_G_SWITCH(s.G, (att_bwdT_long_kernel<SC, 4><<<grid_items, ATT_THREADS, 0, st>>>(p)),
-                 (att_bwdT_long_kernel<SC, 8><<<grid_items, ATT_THREADS, 0, st>>>(p)),
-                 (att_bwdT_long_kernel<SC, 16><<<grid_items, ATT_THREADS, 0, st>>>(p)))
+    ATT_G_SWITCH(s.G, (att_bwdT_long_kernel<SC, 4, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
+                 (att_bwdT_long_kernel<SC, 8, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
+                 (att_bwdT_long_kernel<SC, 16, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)))
     RGBMP_LAUNCH_CHECK("att_bwdT_long_kernel");
     att_bwd_combine_kernel<<<(unsigned)ceil_div(p.n_long * HC, 256), 256, 0, st>>>(p);
     RGBMP_LAUNCH_CHECK("att_bwd_combine_kernel");
@@ -1027,18 +1063,19 @@ static int launch_bwdT(const AttParams& p, const Shape& s, cudaStream_t st) {
   return 0;
 }
 
+template <bool DR>
 static int launch_bwdF(const AttParams& p, const Shape& s, cudaStream_t st) {
   const int HC = p.H * p.C;
   dim3 grid_rows((unsigned)ceil_div(p.n_rows, ATT_THREADS / s.G), (unsigned)s.tiles);
-  ATT_G_SWITCH(s.G, (att_bwdF_rows_kernel<4><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
-               (att_bwdF_rows_kernel<8><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
-               (att_bwdF_rows_kernel<16><<<grid_rows, ATT_THREADS, 0, st>>>(p)))
+  ATT_G_SWITCH(s.G, (att_bwdF_rows_kernel<4, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
+               (att_bwdF_rows_kernel<8, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
+               (att_bwdF_rows_kernel<16, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)))
   RGBMP_LAUNCH_CHECK("att_bwdF_rows_kernel");
   if (p.n_items > 0) {
     dim3 grid_items((unsigned)p.n_items, (unsigned)s.tiles);
-    ATT_G_SWITCH(s.G, (att_bwdF_long_kernel<4><<<grid_items, ATT_THREADS, 0, st>>>(p)),
-                 (att_bwdF_long_kernel<8><<<grid_items, ATT_THREADS, 0, st>>>(p)),
-                 (att_bwdF_long_kernel<16><<<grid_items, ATT_THREADS, 0, st>>>(p)))
+    ATT_G_SWITCH(s.G, (att_bwdF_long_kernel<4, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
+                 (att_bwdF_long_kernel<8, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
+                 (att_bwdF_long_kernel<16, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)))
     RGBMP_LAUNCH_CHECK("att_bwdF_long_kernel");
     att_bwd_combine_kernel<<<(unsigned)ceil_div(p.n_long * HC, 256), 256, 0, st>>>(p);
     RGBMP_LAUNCH_CHECK("att_bwd_combine_kernel");
@@ -1065,31 +1102,40 @@ size_t rgbmp_att_forward_workspace_bytes(const rgbmp_graph_t* g, int H, int C) {
          split_bytes(g->n_items, H, H * C);
 }
 
-int rgbmp_att_forward(const rgbmp_graph_t* g, int score, const float* X, int64_t ldx, const float* a_nbr,
-                      const float* a_own, const float* dinv, int H, int C, float slope, const float* drop, float* out,
-                      int64_t ldo, float* rowmax, float* rowsum, float* out2, int64_t ldo2, float* rowq, void* ws,
-                      size_t ws_bytes, int device, void* stream) {
-  int rc = check_g(g, "rgbmp_att_forward");
+static void set_dropout(AttParams& p, const rgbmp_dropout_t* d, const int32_t* eid) {
+  p.seed = d->seed;
+  p.eid = eid;
+  p.thresh = d->thresh;
+  p.dscale = d->scale;
+}
+
+// d == NULL: the explicit `drop` mask (or none); d != NULL: fused dropout
+static int att_forward(const char* fn, const rgbmp_graph_t* g, int score, const float* X, int64_t ldx, const float* a_nbr,
+                       const float* a_own, const float* dinv, int H, int C, float slope, const float* drop,
+                       const rgbmp_dropout_t* d, float* out, int64_t ldo, float* rowmax, float* rowsum, float* out2,
+                       int64_t ldo2, float* rowq, void* ws, size_t ws_bytes, int device, void* stream) {
+  int rc = check_g(g, fn);
   if (rc) return rc;
   Shape s;
   if (score < RGBMP_ATT_GAT || score > RGBMP_ATT_FA || (score == RGBMP_ATT_FA && H != 1) || !att_shape(H, C, &s))
-    return fail(RGBMP_ERANGE, "rgbmp_att_forward: unsupported score %d / H %d / C %d (H == 1 with C <= 128, or C in {8..128} a power of two)",
-                score, H, C);
-  if (!X || !a_nbr || !a_own || !out || !ws) return fail(RGBMP_EINVAL, "rgbmp_att_forward: null pointer");
+    return fail(RGBMP_ERANGE, "%s: unsupported score %d / H %d / C %d (H == 1 with C <= 128, or C in {8..128} a power of two)",
+                fn, score, H, C);
+  if (!X || !a_nbr || !a_own || !out || !ws) return fail(RGBMP_EINVAL, "%s: null pointer", fn);
+  if (d && (!d->seed || (g->nnz > 0 && !d->eid))) return fail(RGBMP_EINVAL, "%s: dropout needs seed and eid", fn);
   const bool softmax = score != RGBMP_ATT_FA;
-  if (softmax && (!rowmax || !rowsum)) return fail(RGBMP_EINVAL, "rgbmp_att_forward: rowmax / rowsum required");
-  if (!softmax && !dinv) return fail(RGBMP_EINVAL, "rgbmp_att_forward: FA needs dinv");
+  if (softmax && (!rowmax || !rowsum)) return fail(RGBMP_EINVAL, "%s: rowmax / rowsum required", fn);
+  if (!softmax && !dinv) return fail(RGBMP_EINVAL, "%s: FA needs dinv", fn);
   const bool train = out2 != nullptr;
-  if (train && score == RGBMP_ATT_MX) return fail(RGBMP_EINVAL, "rgbmp_att_forward: MX has no second aggregate");
-  if (train && score == RGBMP_ATT_GAT && !rowq) return fail(RGBMP_EINVAL, "rgbmp_att_forward: rowq required with out2");
+  if (train && score == RGBMP_ATT_MX) return fail(RGBMP_EINVAL, "%s: MX has no second aggregate", fn);
+  if (train && score == RGBMP_ATT_GAT && !rowq) return fail(RGBMP_EINVAL, "%s: rowq required with out2", fn);
   const int HC = H * C;
   const int64_t need_ld = (int64_t)align_up((size_t)HC, 4);
   if (!al16(X, ldx) || !al16(out, ldo) || ldx < need_ld || ldo < need_ld || (train && (!al16(out2, ldo2) || ldo2 < need_ld)))
-    return fail(RGBMP_EALIGN, "rgbmp_att_forward: X/out/out2 need 16-byte aligned rows with ld >= roundup(H*C,4)");
+    return fail(RGBMP_EALIGN, "%s: X/out/out2 need 16-byte aligned rows with ld >= roundup(H*C,4)", fn);
   if (ws_bytes < rgbmp_att_forward_workspace_bytes(g, H, C))
-    return fail(RGBMP_EWORKSPACE, "rgbmp_att_forward: workspace %zu < %zu", ws_bytes, rgbmp_att_forward_workspace_bytes(g, H, C));
+    return fail(RGBMP_EWORKSPACE, "%s: workspace %zu < %zu", fn, ws_bytes, rgbmp_att_forward_workspace_bytes(g, H, C));
   DeviceGuard dg(device);
-  if (!dg.ok) return fail(RGBMP_EINVAL, "rgbmp_att_forward: bad device");
+  if (!dg.ok) return fail(RGBMP_EINVAL, "%s: bad device", fn);
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t n = g->n_rows;
   if (n == 0) return 0;
@@ -1099,8 +1145,9 @@ int rgbmp_att_forward(const rgbmp_graph_t* g, int score, const float* X, int64_t
   Carver cv(ws, ws_bytes);
   float* an2 = cv.take<float>((size_t)g->n_cols * H);
   float* ao2 = cv.take<float>((size_t)n * H);
-  if (!carve_split(p, cv, HC, p.n_items) || !cv.ok()) return fail(RGBMP_EWORKSPACE, "rgbmp_att_forward: workspace carve");
+  if (!carve_split(p, cv, HC, p.n_items) || !cv.ok()) return fail(RGBMP_EWORKSPACE, "%s: workspace carve", fn);
   p.Xn = X; p.ldn = ldx; p.Xo = X; p.ldo_ = ldx; p.dinv = dinv; p.drop = drop;
+  if (d) set_dropout(p, d, d->eid);
   p.out = out; p.ldo = ldo; p.out2 = out2; p.ldo2 = ldo2; p.rowmax = rowmax; p.rowsum = rowsum; p.rowq = rowq;
   if (softmax) {                                           // log2-domain copies of the score terms
     att_scale_kernel<<<(unsigned)ceil_div(g->n_cols * H, 256), 256, 0, st>>>(a_nbr, g->n_cols * H, an2);
@@ -1110,9 +1157,31 @@ int rgbmp_att_forward(const rgbmp_graph_t* g, int score, const float* X, int64_t
   } else {
     p.sn = a_nbr; p.so = a_own;
   }
-  if (score == RGBMP_ATT_GAT) return train ? launch_fwd<SC_GAT, true>(p, s, st) : launch_fwd<SC_GAT, false>(p, s, st);
-  if (score == RGBMP_ATT_MX) return launch_fwd<SC_MX, false>(p, s, st);
-  return train ? launch_fwd<SC_FA, true>(p, s, st) : launch_fwd<SC_FA, false>(p, s, st);
+  if (d) {
+    if (score == RGBMP_ATT_GAT) return train ? launch_fwd<SC_GAT, true, true>(p, s, st) : launch_fwd<SC_GAT, false, true>(p, s, st);
+    if (score == RGBMP_ATT_MX) return launch_fwd<SC_MX, false, true>(p, s, st);
+    return train ? launch_fwd<SC_FA, true, true>(p, s, st) : launch_fwd<SC_FA, false, true>(p, s, st);
+  }
+  if (score == RGBMP_ATT_GAT) return train ? launch_fwd<SC_GAT, true, false>(p, s, st) : launch_fwd<SC_GAT, false, false>(p, s, st);
+  if (score == RGBMP_ATT_MX) return launch_fwd<SC_MX, false, false>(p, s, st);
+  return train ? launch_fwd<SC_FA, true, false>(p, s, st) : launch_fwd<SC_FA, false, false>(p, s, st);
+}
+
+int rgbmp_att_forward(const rgbmp_graph_t* g, int score, const float* X, int64_t ldx, const float* a_nbr,
+                      const float* a_own, const float* dinv, int H, int C, float slope, const float* drop, float* out,
+                      int64_t ldo, float* rowmax, float* rowsum, float* out2, int64_t ldo2, float* rowq, void* ws,
+                      size_t ws_bytes, int device, void* stream) {
+  return att_forward("rgbmp_att_forward", g, score, X, ldx, a_nbr, a_own, dinv, H, C, slope, drop, nullptr, out, ldo,
+                     rowmax, rowsum, out2, ldo2, rowq, ws, ws_bytes, device, stream);
+}
+
+int rgbmp_att_forward_dropout(const rgbmp_graph_t* g, int score, const float* X, int64_t ldx, const float* a_nbr,
+                              const float* a_own, const float* dinv, int H, int C, float slope, const rgbmp_dropout_t* d,
+                              float* out, int64_t ldo, float* rowmax, float* rowsum, float* out2, int64_t ldo2,
+                              float* rowq, void* ws, size_t ws_bytes, int device, void* stream) {
+  if (!d) return fail(RGBMP_EINVAL, "rgbmp_att_forward_dropout: null dropout descriptor");
+  return att_forward("rgbmp_att_forward_dropout", g, score, X, ldx, a_nbr, a_own, dinv, H, C, slope, nullptr, d, out,
+                     ldo, rowmax, rowsum, out2, ldo2, rowq, ws, ws_bytes, device, stream);
 }
 
 size_t rgbmp_att_backward_workspace_bytes(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int H, int C) {
@@ -1122,33 +1191,35 @@ size_t rgbmp_att_backward_workspace_bytes(const rgbmp_graph_t* g, const rgbmp_gr
          split_bytes(items, H, H * C);
 }
 
-int rgbmp_att_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int score, const float* X, int64_t ldx,
-                       const float* a_nbr, const float* a_own, const float* dinv, int H, int C, float slope,
-                       const float* drop, const int32_t* tpos, const float* rowmax, const float* rowsum,
-                       const float* rowq, const float* out, int64_t ldo, const float* out2, int64_t ldo2,
-                       const float* dout, int64_t ldd, float* dX, int64_t lddx, float* dXf, int64_t lddxf,
-                       float* da_nbr, float* da_own, void* ws, size_t ws_bytes, int device, void* stream) {
-  int rc = check_g(g, "rgbmp_att_backward");
+static int att_backward(const char* fn, const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int score, const float* X,
+                        int64_t ldx, const float* a_nbr, const float* a_own, const float* dinv, int H, int C, float slope,
+                        const float* drop, const int32_t* tpos, const rgbmp_dropout_t* d, const float* rowmax,
+                        const float* rowsum, const float* rowq, const float* out, int64_t ldo, const float* out2,
+                        int64_t ldo2, const float* dout, int64_t ldd, float* dX, int64_t lddx, float* dXf, int64_t lddxf,
+                        float* da_nbr, float* da_own, void* ws, size_t ws_bytes, int device, void* stream) {
+  int rc = check_g(g, fn);
   if (rc) return rc;
-  rc = check_g(gT, "rgbmp_att_backward");
+  rc = check_g(gT, fn);
   if (rc) return rc;
   Shape s;
   if (score < RGBMP_ATT_GAT || score > RGBMP_ATT_FA || (score == RGBMP_ATT_FA && H != 1) || !att_shape(H, C, &s))
-    return fail(RGBMP_ERANGE, "rgbmp_att_backward: unsupported score %d / H %d / C %d", score, H, C);
+    return fail(RGBMP_ERANGE, "%s: unsupported score %d / H %d / C %d", fn, score, H, C);
   if (!X || !a_nbr || !a_own || !dout || !dX || !da_nbr || !da_own || !ws || (drop && !tpos))
-    return fail(RGBMP_EINVAL, "rgbmp_att_backward: null pointer");
+    return fail(RGBMP_EINVAL, "%s: null pointer", fn);
+  if (d && (!d->seed || (gT->nnz > 0 && !d->eid_t) || (score == RGBMP_ATT_MX && g->nnz > 0 && !d->eid)))
+    return fail(RGBMP_EINVAL, "%s: dropout needs seed, eid_t (and eid for MX)", fn);
   const bool softmax = score != RGBMP_ATT_FA;
-  if (softmax && (!rowmax || !rowsum || !out)) return fail(RGBMP_EINVAL, "rgbmp_att_backward: forward statistics required");
-  if (score != RGBMP_ATT_MX && !out2) return fail(RGBMP_EINVAL, "rgbmp_att_backward: the training-mode forward's second aggregate is required");
-  if (score == RGBMP_ATT_GAT && !rowq) return fail(RGBMP_EINVAL, "rgbmp_att_backward: rowq required");
-  if (score == RGBMP_ATT_MX && !dXf) return fail(RGBMP_EINVAL, "rgbmp_att_backward: MX needs the dXf scratch [n, ld]");
-  if (!softmax && !dinv) return fail(RGBMP_EINVAL, "rgbmp_att_backward: FA needs dinv");
+  if (softmax && (!rowmax || !rowsum || !out)) return fail(RGBMP_EINVAL, "%s: forward statistics required", fn);
+  if (score != RGBMP_ATT_MX && !out2) return fail(RGBMP_EINVAL, "%s: the training-mode forward's second aggregate is required", fn);
+  if (score == RGBMP_ATT_GAT && !rowq) return fail(RGBMP_EINVAL, "%s: rowq required", fn);
+  if (score == RGBMP_ATT_MX && !dXf) return fail(RGBMP_EINVAL, "%s: MX needs the dXf scratch [n, ld]", fn);
+  if (!softmax && !dinv) return fail(RGBMP_EINVAL, "%s: FA needs dinv", fn);
   if (!al16(X, ldx) || !al16(dout, ldd) || !al16(dX, lddx) || (dXf && !al16(dXf, lddxf)))
-    return fail(RGBMP_EALIGN, "rgbmp_att_backward: X/dout/dX need 16-byte aligned rows");
+    return fail(RGBMP_EALIGN, "%s: X/dout/dX need 16-byte aligned rows", fn);
   if (ws_bytes < rgbmp_att_backward_workspace_bytes(g, gT, H, C))
-    return fail(RGBMP_EWORKSPACE, "rgbmp_att_backward: workspace %zu < %zu", ws_bytes, rgbmp_att_backward_workspace_bytes(g, gT, H, C));
+    return fail(RGBMP_EWORKSPACE, "%s: workspace %zu < %zu", fn, ws_bytes, rgbmp_att_backward_workspace_bytes(g, gT, H, C));
   DeviceGuard dg(device);
-  if (!dg.ok) return fail(RGBMP_EINVAL, "rgbmp_att_backward: bad device");
+  if (!dg.ok) return fail(RGBMP_EINVAL, "%s: bad device", fn);
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t n_dst = g->n_rows, n_src = gT->n_rows;
   if (n_dst == 0 || n_src == 0) return 0;
@@ -1160,7 +1231,7 @@ int rgbmp_att_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int scor
   fill_graph(pt, gT);
   pt.H = H; pt.HT = s.HT; pt.C = C; pt.LPH = s.LPH; pt.slope = slope;
   if (!carve_split(pt, cv, HC, g->n_items > gT->n_items ? g->n_items : gT->n_items) || !cv.ok())
-    return fail(RGBMP_EWORKSPACE, "rgbmp_att_backward: workspace carve");
+    return fail(RGBMP_EWORKSPACE, "%s: workspace carve", fn);
   const unsigned prep_grid = (unsigned)ceil_div(n_dst * H, 256);
   if (score == RGBMP_ATT_GAT)
     att_bwd_prep_kernel<SC_GAT><<<prep_grid, 256, 0, st>>>(dout, ldd, out, ldo, out2, ldo2, a_own, rowmax, rowsum, rowq, dinv, n_dst, H, C, stats, da_own);
@@ -1177,7 +1248,8 @@ int rgbmp_att_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int scor
     fill_graph(pf, g);
     pf.Xn = X; pf.ldn = ldx; pf.sn = an2; pf.stats = stats; pf.Xo = X; pf.ldo_ = ldx; pf.Do = dout; pf.lddo = ldd;
     pf.drop = drop; pf.out = dXf; pf.ldo = lddxf; pf.ds = da_own;
-    rc = launch_bwdF(pf, s, st);
+    if (d) set_dropout(pf, d, d->eid);
+    rc = d ? launch_bwdF<true>(pf, s, st) : launch_bwdF<false>(pf, s, st);
     if (rc) return rc;
     pt.acc_in = dXf; pt.ld_acc = lddxf;
     pt.Xn2 = X; pt.ldn2 = ldx;
@@ -1185,9 +1257,53 @@ int rgbmp_att_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int scor
   // pass T on the transpose CSR: dX_j, da_src[j]
   pt.Xn = dout; pt.ldn = ldd; pt.stats = stats; pt.dinv = dinv; pt.Xo = X; pt.ldo_ = ldx; pt.so = a_nbr;
   pt.drop = drop; pt.tpos = tpos; pt.out = dX; pt.ldo = lddx; pt.ds = da_nbr;
-  if (score == RGBMP_ATT_GAT) return launch_bwdT<SC_GAT>(pt, s, st);
-  if (score == RGBMP_ATT_MX) return launch_bwdT<SC_MX>(pt, s, st);
-  return launch_bwdT<SC_FA>(pt, s, st);
+  if (d) {
+    set_dropout(pt, d, d->eid_t);
+    if (score == RGBMP_ATT_GAT) return launch_bwdT<SC_GAT, true>(pt, s, st);
+    if (score == RGBMP_ATT_MX) return launch_bwdT<SC_MX, true>(pt, s, st);
+    return launch_bwdT<SC_FA, true>(pt, s, st);
+  }
+  if (score == RGBMP_ATT_GAT) return launch_bwdT<SC_GAT, false>(pt, s, st);
+  if (score == RGBMP_ATT_MX) return launch_bwdT<SC_MX, false>(pt, s, st);
+  return launch_bwdT<SC_FA, false>(pt, s, st);
+}
+
+int rgbmp_att_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int score, const float* X, int64_t ldx,
+                       const float* a_nbr, const float* a_own, const float* dinv, int H, int C, float slope,
+                       const float* drop, const int32_t* tpos, const float* rowmax, const float* rowsum,
+                       const float* rowq, const float* out, int64_t ldo, const float* out2, int64_t ldo2,
+                       const float* dout, int64_t ldd, float* dX, int64_t lddx, float* dXf, int64_t lddxf,
+                       float* da_nbr, float* da_own, void* ws, size_t ws_bytes, int device, void* stream) {
+  return att_backward("rgbmp_att_backward", g, gT, score, X, ldx, a_nbr, a_own, dinv, H, C, slope, drop, tpos, nullptr,
+                      rowmax, rowsum, rowq, out, ldo, out2, ldo2, dout, ldd, dX, lddx, dXf, lddxf, da_nbr, da_own, ws,
+                      ws_bytes, device, stream);
+}
+
+int rgbmp_att_backward_dropout(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int score, const float* X, int64_t ldx,
+                               const float* a_nbr, const float* a_own, const float* dinv, int H, int C, float slope,
+                               const rgbmp_dropout_t* d, const float* rowmax, const float* rowsum, const float* rowq,
+                               const float* out, int64_t ldo, const float* out2, int64_t ldo2, const float* dout,
+                               int64_t ldd, float* dX, int64_t lddx, float* dXf, int64_t lddxf, float* da_nbr,
+                               float* da_own, void* ws, size_t ws_bytes, int device, void* stream) {
+  if (!d) return fail(RGBMP_EINVAL, "rgbmp_att_backward_dropout: null dropout descriptor");
+  return att_backward("rgbmp_att_backward_dropout", g, gT, score, X, ldx, a_nbr, a_own, dinv, H, C, slope, nullptr,
+                      nullptr, d, rowmax, rowsum, rowq, out, ldo, out2, ldo2, dout, ldd, dX, lddx, dXf, lddxf, da_nbr,
+                      da_own, ws, ws_bytes, device, stream);
+}
+
+int rgbmp_dropout_mask(const rgbmp_dropout_t* d, int64_t nnz, int H, float* out, int device, void* stream) {
+  if (!d || !d->seed || nnz < 0 || H <= 0 || (nnz > 0 && !out))
+    return fail(RGBMP_EINVAL, "rgbmp_dropout_mask: bad arguments");
+  if (nnz > INT32_MAX) return fail(RGBMP_ERANGE, "rgbmp_dropout_mask: edge ids are 32-bit");
+  DeviceGuard dg(device);
+  if (!dg.ok) return fail(RGBMP_EINVAL, "rgbmp_dropout_mask: bad device");
+  const int64_t n = nnz * H;
+  if (n == 0) return 0;
+  const int64_t blocks = ceil_div(n, 256);
+  att_dropout_mask_kernel<<<(unsigned)(blocks < 148 * 64 ? blocks : 148 * 64), 256, 0, (cudaStream_t)stream>>>(
+      d->seed, n, H, d->thresh, d->scale, out);
+  RGBMP_LAUNCH_CHECK("att_dropout_mask_kernel");
+  return 0;
 }
 
 }  // extern "C"

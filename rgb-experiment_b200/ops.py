@@ -7,6 +7,7 @@ provides the tensors (device memory), the stream and the autograd graph.
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import Optional, Tuple
 
 import torch
@@ -230,6 +231,9 @@ def propagate_weighted(x, w, graph: Graph):
 # ------------------------------------------------------------------------------------------
 FOLD_KHOP = True     # K-hop families apply D^-1/2 (A+I) D^-1/2 as row scalings around an unweighted sum (no per-edge
                      # weight stream, 4 B/edge less and adds instead of FMAs); False: per-edge gcn_norm weights as PyG multiplies them
+FUSED_DROPOUT = False  # GATConv / SuperGATConv / FAConv in training mode: True = attention dropout generated inside the
+                       # attention kernels (counter-based, keyed by edge id, nothing edge-sized allocated); False = a torch
+                       # F.dropout mask per call, so the same torch.manual_seed draws the same masks as it always has
 
 
 def _khop_gcn(csr: CSR, graph: Graph, x0b: torch.Tensor, K: int, transpose: bool, fold: bool, **epkw):
@@ -560,10 +564,12 @@ class _Att(torch.autograd.Function):
     """Fused edge-score attention + aggregate (csrc/att.cu): GATConv (A10/A11; gat.py:18-21), SuperGATConv-MX
     (A12; supergat.py:15-21) and FAConv (A13; fagcn.py:15,31).  Nothing edge-sized is allocated: the forward saves
     per-node statistics (max, sum and -- in training mode -- the second aggregate that yields the gradient of the
-    target-side score term), the backward recomputes the edge weights.  Deterministic (no atomics)."""
+    target-side score term), the backward recomputes the edge weights.  Deterministic (no atomics).
+    Attention dropout: either an explicit mask in forward-CSR order (drop_csr) or a device seed tensor (seed, rate p)
+    from which forward and backward regenerate the same multipliers inside the kernels -- still nothing edge-sized."""
 
     @staticmethod
-    def forward(ctx, x, a_nbr, a_own, graph: Graph, score: int, H: int, Cc: int, slope: float, drop_csr):
+    def forward(ctx, x, a_nbr, a_own, graph: Graph, score: int, H: int, Cc: int, slope: float, drop_csr, seed, p):
         _lib.require_cuda(x, "x")
         for t, nm in ((x, "x"), (a_nbr, "a_nbr"), (a_own, "a_own")):
             _lib.require_f32(t, f"fused attention {nm}")
@@ -586,16 +592,22 @@ class _Att(torch.autograd.Function):
         L = lib()
         wsb = L.rgbmp_att_forward_workspace_bytes(graph.fwd.ref, H, Cc)
         ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
-        check(L.rgbmp_att_forward(graph.fwd.ref, score, ptr(xb), ldx, ptr(a_n), ptr(a_o), ptr(dinv), H, Cc, slope,
-                                  ptr(drop_csr), ptr(out), ldo, ptr(rmax), ptr(rsum), ptr(out2), ldo2, ptr(rowq),
-                                  ptr(ws), wsb, dev.index, stream_of(dev)), "att_forward")
-        ctx.graph, ctx.score, ctx.H, ctx.Cc, ctx.slope = graph, score, H, Cc, slope
-        ctx.save_for_backward(xb, a_n, a_o, rmax, rsum, rowq, out, out2, drop_csr)
+        if seed is None:
+            check(L.rgbmp_att_forward(graph.fwd.ref, score, ptr(xb), ldx, ptr(a_n), ptr(a_o), ptr(dinv), H, Cc, slope,
+                                      ptr(drop_csr), ptr(out), ldo, ptr(rmax), ptr(rsum), ptr(out2), ldo2, ptr(rowq),
+                                      ptr(ws), wsb, dev.index, stream_of(dev)), "att_forward")
+        else:
+            d = _dropout_struct(p, seed, graph)
+            check(L.rgbmp_att_forward_dropout(graph.fwd.ref, score, ptr(xb), ldx, ptr(a_n), ptr(a_o), ptr(dinv), H, Cc,
+                                              slope, C.byref(d), ptr(out), ldo, ptr(rmax), ptr(rsum), ptr(out2), ldo2,
+                                              ptr(rowq), ptr(ws), wsb, dev.index, stream_of(dev)), "att_forward_dropout")
+        ctx.graph, ctx.score, ctx.H, ctx.Cc, ctx.slope, ctx.p = graph, score, H, Cc, slope, p
+        ctx.save_for_backward(xb, a_n, a_o, rmax, rsum, rowq, out, out2, drop_csr, seed)
         return out
 
     @staticmethod
     def backward(ctx, dout):
-        xb, a_n, a_o, rmax, rsum, rowq, out, out2, drop = ctx.saved_tensors
+        xb, a_n, a_o, rmax, rsum, rowq, out, out2, drop, seed = ctx.saved_tensors
         g, score, H, Cc = ctx.graph, ctx.score, ctx.H, ctx.Cc
         dev, N = dout.device, g.N
         db, ldd = _rows_zero_padded(dout)
@@ -608,33 +620,92 @@ class _Att(torch.autograd.Function):
         L = lib()
         wsb = L.rgbmp_att_backward_workspace_bytes(g.fwd.ref, g.bwd.ref, H, Cc)
         ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
-        check(L.rgbmp_att_backward(g.fwd.ref, g.bwd.ref, score, ptr(xb), xb.stride(0), ptr(a_n), ptr(a_o), ptr(dinv), H, Cc,
-                                   ctx.slope, ptr(drop), ptr(tpos), ptr(rmax), ptr(rsum), ptr(rowq), ptr(out),
-                                   out.stride(0), ptr(out2), 0 if out2 is None else out2.stride(0), ptr(db), ldd,
-                                   ptr(dx), lddx, ptr(dxf), lddxf, ptr(da_n), ptr(da_o), ptr(ws), wsb, dev.index,
-                                   stream_of(dev)), "att_backward")
-        return dx, da_n, da_o, None, None, None, None, None, None
+        ld2 = 0 if out2 is None else out2.stride(0)
+        if seed is None:
+            check(L.rgbmp_att_backward(g.fwd.ref, g.bwd.ref, score, ptr(xb), xb.stride(0), ptr(a_n), ptr(a_o), ptr(dinv), H,
+                                       Cc, ctx.slope, ptr(drop), ptr(tpos), ptr(rmax), ptr(rsum), ptr(rowq), ptr(out),
+                                       out.stride(0), ptr(out2), ld2, ptr(db), ldd, ptr(dx), lddx, ptr(dxf), lddxf,
+                                       ptr(da_n), ptr(da_o), ptr(ws), wsb, dev.index, stream_of(dev)), "att_backward")
+        else:
+            d = _dropout_struct(ctx.p, seed, g, backward=True)
+            check(L.rgbmp_att_backward_dropout(g.fwd.ref, g.bwd.ref, score, ptr(xb), xb.stride(0), ptr(a_n), ptr(a_o),
+                                               ptr(dinv), H, Cc, ctx.slope, C.byref(d), ptr(rmax), ptr(rsum), ptr(rowq),
+                                               ptr(out), out.stride(0), ptr(out2), ld2, ptr(db), ldd, ptr(dx), lddx,
+                                               ptr(dxf), lddxf, ptr(da_n), ptr(da_o), ptr(ws), wsb, dev.index,
+                                               stream_of(dev)), "att_backward_dropout")
+        return dx, da_n, da_o, None, None, None, None, None, None, None, None
 
 
-def _att(score: int, name: str, x, a_nbr, a_own, graph: Graph, H: int, Cc: int, slope: float, drop_edge):
+def _att(score: int, name: str, x, a_nbr, a_own, graph: Graph, H: int, Cc: int, slope: float, drop_edge,
+         dropout_p: float = 0.0, seed: Optional[torch.Tensor] = None):
     """Pads heads to the kernel's channel count (torch ops on node-sized tensors, autograd-transparent), memoises
-    the no-grad call, applies the fused op."""
+    the no-grad call, applies the fused op.  seed: fused dropout at rate dropout_p (see dropout_mask)."""
     Cp = _head_pad(H, Cc)
     N = x.size(0)
     xk = x if Cp == Cc else torch.nn.functional.pad(x.view(N, H, Cc), (0, Cp - Cc)).reshape(N, H * Cp)
     drop_csr = None if drop_edge is None else graph.to_csr_order(drop_edge)
-    if drop_csr is None:
+    if drop_csr is None and seed is None:
         out = memo.cached(graph, (name, H, Cc, float(slope)), (xk, a_nbr, a_own), _work(graph, xk),
-                          lambda: _Att.apply(xk, a_nbr, a_own, graph, score, H, Cp, float(slope), None))
+                          lambda: _Att.apply(xk, a_nbr, a_own, graph, score, H, Cp, float(slope), None, None, 0.0))
     else:
-        out = _Att.apply(xk, a_nbr, a_own, graph, score, H, Cp, float(slope), drop_csr)
+        out = _Att.apply(xk, a_nbr, a_own, graph, score, H, Cp, float(slope), drop_csr, seed, float(dropout_p))
     return out if Cp == Cc else out.view(N, H, Cp)[:, :, :Cc].reshape(N, H * Cc)
 
 
-def gat(xp, a_src, a_dst, graph: Graph, H: int, Cc: int, slope: float = 0.2, drop_edge: Optional[torch.Tensor] = None):
-    """xp [N,H*C], a_src/a_dst [N,H] -> [N,H*C].  drop_edge: optional [nnz,H] keep-mask/(1-p) in EDGE order."""
+# ------------------------------------------------------------------------------------------
+# attention dropout generated from a seed (csrc/philox.cuh): multiplier of edge e, head h =
+#   Philox4x32-10(counter (e, h, 0, 0), key (seed lo, seed hi)).word0 < floor(p 2^32) ? 0 : float32(1/(1-p))
+# ------------------------------------------------------------------------------------------
+def dropout_seed(device, generator: Optional[torch.Generator] = None) -> torch.Tensor:
+    """One int64 drawn on the device from its CUDA generator (or `generator`): no host synchronisation,
+    governed by torch.manual_seed / fork_rng, safe under graph capture."""
+    return torch.empty(1, dtype=torch.int64, device=device).random_(generator=generator)
+
+
+def _dropout_struct(p: float, seed: torch.Tensor, graph: Optional[Graph] = None, backward: bool = False):
+    """rgbmp_dropout_t for rate p (thresh = floor(p 2^32) exactly; p == 1 -> every multiplier 0)."""
+    if p >= 1.0:
+        thresh, scale = 0xFFFFFFFF, 0.0
+    else:
+        thresh, scale = int(math.floor(p * 4294967296.0)), 1.0 / (1.0 - p)    # c_float rounds scale to float32
+    eid = eid_t = None
+    if graph is not None:
+        if graph.fwd.eid is None:
+            raise RuntimeError("fused attention dropout needs the edge ids of the graph")
+        eid = graph.fwd.eid
+        eid_t = graph.bwd.eid if backward else None
+    return _lib.DropoutStruct(ptr(seed), ptr(eid), ptr(eid_t), thresh, scale)
+
+
+def dropout_mask(graph: Graph, H: int, p: float, seed: torch.Tensor) -> torch.Tensor:
+    """[nnz, H] float32 multipliers in EDGE order: the mask the fused kernels apply for `seed` (unfused paths, tests)."""
+    out = torch.empty((graph.nnz, H), dtype=torch.float32, device=graph.device)
+    d = _dropout_struct(float(p), seed)
+    check(lib().rgbmp_dropout_mask(C.byref(d), graph.nnz, H, ptr(out), graph.device.index, stream_of(graph.device)),
+          "dropout_mask")
+    return out
+
+
+def _draw_dropout(graph: Graph, drop_edge, dropout_p: float, generator) -> Optional[torch.Tensor]:
+    """Validate the dropout arguments; the seed tensor when dropout_p > 0, else None."""
+    p = float(dropout_p)
+    if not 0.0 <= p <= 1.0:
+        raise ValueError(f"dropout_p must lie in [0, 1] (got {dropout_p})")
+    if p > 0.0 and drop_edge is not None:
+        raise ValueError("drop_edge and dropout_p are mutually exclusive")
+    return dropout_seed(graph.device, generator) if p > 0.0 else None
+
+
+def gat(xp, a_src, a_dst, graph: Graph, H: int, Cc: int, slope: float = 0.2, drop_edge: Optional[torch.Tensor] = None,
+        dropout_p: float = 0.0, generator: Optional[torch.Generator] = None):
+    """xp [N,H*C], a_src/a_dst [N,H] -> [N,H*C].  drop_edge: optional [nnz,H] keep-mask/(1-p) in EDGE order.
+    dropout_p: attention dropout drawn from a seed (`generator` or the device's default CUDA generator) and
+    generated inside the kernels; exclusive with drop_edge."""
+    seed = _draw_dropout(graph, drop_edge, dropout_p, generator)
     if att_fusable(ATT_GAT, H, Cc):
-        return _att(ATT_GAT, "gat", xp, a_src, a_dst, graph, H, Cc, slope, drop_edge)
+        return _att(ATT_GAT, "gat", xp, a_src, a_dst, graph, H, Cc, slope, drop_edge, dropout_p, seed)
+    if seed is not None:
+        drop_edge = dropout_mask(graph, H, dropout_p, seed)
     e = torch.nn.functional.leaky_relu(edge_u_add_v(a_src, a_dst, graph), slope)
     alpha = edge_softmax(e, graph)
     if drop_edge is not None:
@@ -643,10 +714,15 @@ def gat(xp, a_src, a_dst, graph: Graph, H: int, Cc: int, slope: float = 0.2, dro
 
 
 def supergat_mx(xp, a_l, a_r, graph: Graph, H: int, Cc: int, slope: float = 0.2,
-                drop_edge: Optional[torch.Tensor] = None):
-    """SuperGATConv MX attention + aggregate (A12): alpha = softmax(leaky_relu((a_l[j] + a_r[i]) * sigmoid(<x_i, x_j>)))."""
+                drop_edge: Optional[torch.Tensor] = None, dropout_p: float = 0.0,
+                generator: Optional[torch.Generator] = None):
+    """SuperGATConv MX attention + aggregate (A12): alpha = softmax(leaky_relu((a_l[j] + a_r[i]) * sigmoid(<x_i, x_j>))).
+    drop_edge / dropout_p / generator as in gat."""
+    seed = _draw_dropout(graph, drop_edge, dropout_p, generator)
     if att_fusable(ATT_MX, H, Cc):
-        return _att(ATT_MX, "supergat_mx", xp, a_l, a_r, graph, H, Cc, slope, drop_edge)
+        return _att(ATT_MX, "supergat_mx", xp, a_l, a_r, graph, H, Cc, slope, drop_edge, dropout_p, seed)
+    if seed is not None:
+        drop_edge = dropout_mask(graph, H, dropout_p, seed)
     logits = edge_sddmm(xp, xp, graph, H, Cc)
     alpha = torch.nn.functional.leaky_relu(edge_u_add_v(a_l, a_r, graph) * logits.sigmoid(), slope)
     alpha = edge_softmax(alpha, graph)
@@ -655,11 +731,17 @@ def supergat_mx(xp, a_l, a_r, graph: Graph, H: int, Cc: int, slope: float = 0.2,
     return spmm_heads(alpha, xp, graph, H, Cc)
 
 
-def faconv(x, a_l, a_r, graph: Graph, drop_edge: Optional[torch.Tensor] = None):
-    """FAConv aggregate (A13): out[i] = sum_j tanh(a_l[j] + a_r[i]) * gcn_norm_ij * mask_ij * x[j]; a_l, a_r [N,1]."""
+def faconv(x, a_l, a_r, graph: Graph, drop_edge: Optional[torch.Tensor] = None, dropout_p: float = 0.0,
+           generator: Optional[torch.Generator] = None):
+    """FAConv aggregate (A13): out[i] = sum_j tanh(a_l[j] + a_r[i]) * gcn_norm_ij * mask_ij * x[j]; a_l, a_r [N,1].
+    drop_edge / dropout_p / generator as in gat (head 0)."""
     Cc = x.size(1)
+    seed = _draw_dropout(graph, drop_edge, dropout_p, generator)
     if att_fusable(ATT_FA, 1, Cc):
-        return _att(ATT_FA, "faconv", x, a_l, a_r, graph, 1, Cc, 0.0, None if drop_edge is None else drop_edge.view(-1, 1))
+        return _att(ATT_FA, "faconv", x, a_l, a_r, graph, 1, Cc, 0.0, None if drop_edge is None else drop_edge.view(-1, 1),
+                    dropout_p, seed)
+    if seed is not None:
+        drop_edge = dropout_mask(graph, 1, dropout_p, seed)
     c = edge_u_add_v(a_l.view(-1, 1), a_r.view(-1, 1), graph).tanh()
     if drop_edge is not None:
         c = c * graph.to_csr_order(drop_edge).view(-1, 1)

@@ -210,10 +210,13 @@ class GATConv(MessagePassing):
         a_d = (x3 * self.att_dst).sum(-1)
         N = xp.size(0)
         g = get_graph(edge_index, N, LOOP_REMOVE_THEN_ADD if self.add_self_loops else LOOP_NONE)
-        drop = None
+        drop, p = None, 0.0
         if self.training and self.dropout > 0:
-            drop = F.dropout(torch.ones((g.nnz, H), device=x.device), p=self.dropout, training=True)
-        out = ops.gat(xp, a_s, a_d, g, H, C, self.negative_slope, drop)
+            if ops.FUSED_DROPOUT:                                     # generated inside the kernels from a seed
+                p = self.dropout
+            else:
+                drop = F.dropout(torch.ones((g.nnz, H), device=x.device), p=self.dropout, training=True)
+        out = ops.gat(xp, a_s, a_d, g, H, C, self.negative_slope, drop, dropout_p=p)
         out = out if self.concat else out.view(-1, H, C).mean(dim=1)
         if self.bias is not None:
             out = out + self.bias
@@ -277,14 +280,19 @@ class SuperGATConv(MessagePassing):
         g = get_graph(edge_index, N, LOOP_REMOVE_THEN_ADD if self.add_self_loops else LOOP_NONE)
         xp = self.lin(x)
         x3 = xp.view(-1, H, C)
-        keep = None
-        if self.training and self.dropout > 0:                        # PyTorch RNG mask, edge order (like GATConv)
-            keep = F.dropout(torch.ones((g.nnz, H), device=x.device), p=self.dropout, training=True)
+        keep, p = None, 0.0
+        if self.training and self.dropout > 0:
+            if ops.FUSED_DROPOUT:                                     # generated from a seed (like GATConv)
+                p = self.dropout
+            else:                                                     # PyTorch RNG mask, edge order (like GATConv)
+                keep = F.dropout(torch.ones((g.nnz, H), device=x.device), p=self.dropout, training=True)
         if self.attention_type == "MX":
             a_l = (x3 * self.att_l).sum(-1)
             a_r = (x3 * self.att_r).sum(-1)
-            out = ops.supergat_mx(xp, a_l, a_r, g, H, C, self.negative_slope, keep)      # one fused pass
+            out = ops.supergat_mx(xp, a_l, a_r, g, H, C, self.negative_slope, keep, dropout_p=p)      # one fused pass
         else:                                                         # SD attention: not used by the reference
+            if p > 0:                                                 # the mask the seed stands for, edge order
+                keep = ops.dropout_mask(g, H, p, ops.dropout_seed(x.device))
             alpha = F.leaky_relu(ops.edge_sddmm(xp, xp, g, H, C) / math.sqrt(C), self.negative_slope)
             alpha = ops.edge_softmax(alpha, g)
             if keep is not None:
@@ -379,10 +387,13 @@ class FAConv(MessagePassing):
             raise NotImplementedError("FAConv(normalize=False) is not used by the reference")
         N = x.size(0)
         g = get_graph(edge_index, N, LOOP_ADD_REMAINING if self.add_self_loops else LOOP_NONE)
-        keep = None
+        keep, p = None, 0.0
         if self.training and self.dropout > 0:
-            keep = F.dropout(torch.ones(g.nnz, device=x.device), p=self.dropout, training=True)
-        out = ops.faconv(x, self.att_l(x), self.att_r(x), g, keep)            # tanh score * gcn weight, fused
+            if ops.FUSED_DROPOUT:                                     # generated inside the kernel from a seed
+                p = self.dropout
+            else:
+                keep = F.dropout(torch.ones(g.nnz, device=x.device), p=self.dropout, training=True)
+        out = ops.faconv(x, self.att_l(x), self.att_r(x), g, keep, dropout_p=p)   # tanh score * gcn weight, fused
         if self.eps != 0.0:
             out = out + self.eps * x_0
         return out
