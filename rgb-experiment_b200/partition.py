@@ -128,11 +128,25 @@ def all_gather_rows(local: torch.Tensor, full: torch.Tensor, group=None):
     return full
 
 
-class PartitionedPropagator:
-    """Device-agnostic K-hop driver: z <- a * A_hat z + b * z0 on a row partition.
+def check_post_step(R: int, clamp=None, reset=None) -> None:
+    """Shapes of label propagation's post-step on a row block of R rows: clamp = (lo, hi); reset = (mask [R],
+    values [R, >= F]) -- rows of THIS block, in its naming."""
+    if clamp is not None and len(clamp) != 2:
+        raise RuntimeError("clamp takes (lo, hi)")
+    if reset is not None:
+        mask, vals = reset
+        if mask.dim() != 1 or mask.size(0) != R or vals.dim() != 2 or vals.size(0) != R:
+            raise RuntimeError(f"reset takes (mask [{R}], values [{R}, F]) rows of this block; got "
+                               f"{tuple(mask.shape)} / {tuple(vals.shape)}")
 
-    spmm(x_full [P*R, ld], z0_local, a, b) -> next local iterate [R, ld] is injected: the CUDA
-    kernel in production, the CPU oracle in the gloo tests."""
+
+class PartitionedPropagator:
+    """Device-agnostic K-hop driver: z <- post(a * A_hat z + b * z0) on a row partition.
+
+    spmm(x_full [P*R, ld], z0_local, a, b[, clamp=, reset=]) -> next local iterate [R, ld] is injected: the CUDA
+    kernel in production, the CPU oracle in the gloo tests.  The label-propagation post-step (clamp, then the reset
+    rows) belongs to the same hop, so it goes to `spmm` with it; `spmm` is called without those keywords when the run
+    has no post-step (APPNP / SGC)."""
 
     def __init__(self, N: int, rank: int, world: int, spmm: Callable, group=None):
         self.N, self.rank, self.world, self.group = N, rank, world, group
@@ -141,9 +155,11 @@ class PartitionedPropagator:
         self.spmm = spmm
 
     def run(self, z0_local: torch.Tensor, K: int, a: float, b: float,
-            full: Optional[torch.Tensor] = None) -> torch.Tensor:
+            full: Optional[torch.Tensor] = None, clamp=None, reset=None) -> torch.Tensor:
         R, ld = z0_local.shape
         assert R == self.R, "every rank passes ceil(N/P) rows (pad the last block)"
+        check_post_step(R, clamp, reset)
+        post = {k: v for k, v in (("clamp", clamp), ("reset", reset)) if v is not None}
         if full is None:
             full = torch.empty((R * self.world, ld), dtype=z0_local.dtype, device=z0_local.device)
         cur = z0_local
@@ -153,7 +169,7 @@ class PartitionedPropagator:
                 src = full
             else:
                 src = cur
-            cur = self.spmm(src, z0_local, a, b)
+            cur = self.spmm(src, z0_local, a, b, **post)
         return cur
 
 
@@ -331,6 +347,25 @@ def _wrap(ptr: int, nbytes: int, device) -> torch.Tensor:
     return torch.as_tensor(_RawCuda(ptr, nbytes), device=device)
 
 
+def _reset_rows(reset, F: int):
+    """(mask [R], values [R, >= F]) -> (uint8 mask, float32 values with 16-byte aligned rows), once per run: the
+    epilogue reads a byte per row and the values as float32 whatever the feature dtype (as ops.label_propagation)."""
+    from . import _lib, ops
+    mask, vals = reset
+    _lib.require_cuda(mask, "reset mask")
+    rv, _ = ops.as_rows(vals[:, :F].float())
+    return mask.to(torch.uint8).contiguous(), rv
+
+
+def _post_epilogue(clamp, reset) -> dict:
+    """make_epilogue keywords of label propagation's post-step (`reset` as _reset_rows returns it)."""
+    from . import ops
+    kw = {} if clamp is None else dict(clamp=clamp)
+    if reset is not None:
+        kw.update(reset_mask=reset[0], reset_val=reset[1], ld_reset=reset[1].stride(0), reset_when=ops.RESET_AFTER_CLAMP)
+    return kw
+
+
 class PartitionedAPPNP:
     """APPNP / LP-style K-hop propagation over a LocalBlock.
 
@@ -343,7 +378,8 @@ class PartitionedAPPNP:
 
     def __init__(self, block: LocalBlock, F: int, group=None, mode: str = "push", dtype=torch.float32,
                  ld: Optional[int] = None):
-        from . import ops
+        from . import _lib, ops
+        _lib.dtype_code(torch.empty(0, dtype=dtype))        # float32 / bfloat16 only: anything else raises here
         self.block, self.F, self.group, self.dtype = block, F, group, dtype
         self.ld = ops.padded_width(F, dtype) if ld is None else int(ld)
         if self.ld < ops.padded_width(F, dtype) or self.ld % ops.padded_width(1, dtype) != 0:
@@ -364,44 +400,60 @@ class PartitionedAPPNP:
         self.pong = torch.zeros((R, self.ld), dtype=dtype, device=dev)
         self._flip = False
 
-        def spmm(x_full, z0_local, a, b):
+        def spmm(x_full, z0_local, a, b, clamp=None, reset=None):
             out = self.pong if self._flip else self.ping
             self._flip = not self._flip
-            ep = (ops.make_epilogue(a=a, b=b, T=z0_local, ldt=z0_local.stride(0)) if b != 0.0
-                  else ops.make_epilogue(a=a))
-            ops.spmm_raw(block.csr, x_full[:, :F], block.val, ep=ep, keep=(z0_local,), out=out[:, :F])
+            tele = dict(b=b, T=z0_local, ldt=z0_local.stride(0)) if b != 0.0 else {}
+            ep = ops.make_epilogue(a=a, **tele, **_post_epilogue(clamp, reset))
+            ops.spmm_raw(block.csr, x_full[:, :F], block.val, ep=ep, keep=(z0_local, reset), out=out[:, :F])
             return out
 
         self.driver = PartitionedPropagator(block.N, block.rank, block.world, spmm, group)
         self.launches_per_hop = 1 + (2 if block.csr.n_items > 0 else 0)
 
-    def run(self, z0_local: torch.Tensor, K: int, alpha: float) -> torch.Tensor:
+    def run(self, z0_local: torch.Tensor, K: int, alpha: float = 0.0, *, teleport=None, clamp=None,
+            reset=None) -> torch.Tensor:
         """z0_local: [R, ld] (padded rows beyond N are zero).  Returns this rank's rows of z_K.
-        alpha = 0 is the plain K-hop GCN propagation A_hat^K z0 (no teleport read)."""
+        alpha = 0 is the plain K-hop GCN propagation A_hat^K z0 (no teleport read).
+
+        Label propagation (ops.label_propagation on a LOOP_NONE block) through the same hops:
+          teleport=(a, b): z <- a * A_hat z + b * z0 in place of (1 - alpha, alpha); LP's is (alpha, 1 - alpha);
+          clamp=(lo, hi): every new iterate is clamped after the teleport;
+          reset=(mask [R], values [R, >= F]): then the masked rows of every new iterate take their `values` (read as
+          float32, RESET_AFTER_CLAMP).  Rows are this block's."""
+        from . import _lib
+        if z0_local.dtype != self.dtype:
+            _lib.dtype_code(z0_local)
+            raise RuntimeError(f"z0_local is {z0_local.dtype}; this propagation was built for {self.dtype}")
+        a, b = (1.0 - alpha, alpha) if teleport is None else (float(teleport[0]), float(teleport[1]))
+        check_post_step(self.block.R, clamp, reset)
+        if reset is not None:
+            reset = _reset_rows(reset, self.F)
         if self.mode != "push":
-            return self.driver.run(z0_local, K, 1.0 - alpha, alpha, self.full)
+            return self.driver.run(z0_local, K, a, b, self.full, clamp=clamp, reset=reset)
         from . import ops
         blk, F, R = self.block, self.F, self.block.R
         full = self.peers.local
         d = blk.dinv_local
         # folded normalisation: the peer buffers hold u_k = D^-1/2 z_k (what the hop gathers, no per-edge
-        # weight stream); the epilogue rebuilds z_{k+1} = a * d_i * sum_j u_k[j] + b * z0_i and pushes d_i * z_{k+1}
+        # weight stream); the epilogue rebuilds z_{k+1} = post(a * d_i * sum_j u_k[j] + b * z0_i) and pushes d_i * z_{k+1}
         u0 = ops.row_scale(z0_local, d)
         dist.all_gather_into_tensor(full[0], u0, group=self.group)                # iterate 0 everywhere
         # timing-only switches for attributing the hop time (results are WRONG with either of them set)
         dbg_self_only = os.environ.get("RGBMP_DEBUG_PUSH") == "self"
         dbg_no_tick = os.environ.get("RGBMP_DEBUG_TICK") == "0"
+        tele = dict(b=b, T=z0_local, ldt=z0_local.stride(0)) if b != 0.0 else {}
+        post = _post_epilogue(clamp, reset)
         for k in range(K):
             src, nxt, last = full[k & 1], (k + 1) & 1, k == K - 1
-            tele = dict(b=alpha, T=z0_local, ldt=z0_local.stride(0)) if alpha != 0.0 else {}
             if last:                       # the result stays local and unscaled: no push, no tick
-                ep = ops.make_epilogue(row_scale=d, a=1.0 - alpha, **tele)
-                ops.spmm_raw(blk.csr, src[:, :F], None, ep=ep, keep=(z0_local, d), out=self.out[:, :F])
+                ep = ops.make_epilogue(row_scale=d, a=a, **tele, **post)
+                ops.spmm_raw(blk.csr, src[:, :F], None, ep=ep, keep=(z0_local, d, reset), out=self.out[:, :F])
                 break
             peers = [self.peers.ptrs[nxt][blk.rank]] if dbg_self_only else self.peers.ptrs[nxt]
-            ep = ops.make_epilogue(row_scale=d, a=1.0 - alpha, out2_scale=d, peers=peers, peer_row0=blk.rank * R,
-                                   ld_peer=self.ld, **tele)
-            ops.spmm_raw(blk.csr, src[:, :F], None, ep=ep, keep=(z0_local, d), store_local=False)
+            ep = ops.make_epilogue(row_scale=d, a=a, out2_scale=d, peers=peers, peer_row0=blk.rank * R,
+                                   ld_peer=self.ld, **tele, **post)
+            ops.spmm_raw(blk.csr, src[:, :F], None, ep=ep, keep=(z0_local, d, reset), store_local=False)
             if not dbg_no_tick:
                 dist.all_reduce(self.tick, group=self.group)     # orders the hops: every push has landed
         return self.out
@@ -500,3 +552,106 @@ class DistAPPNP(torch.nn.Module):
         z = _DistKHop.apply(z0, lambda t: self.fwd_runner(t, self.K, self.alpha),
                             lambda t: self.bwd_runner(t, self.K, self.alpha))
         return _GatherSlices.apply(z, self.grid, self.F, self.col_group)
+
+
+class DistCorrectAndSmooth:
+    """Correct & Smooth (shim.nn.CorrectAndSmooth, SURVEY A15) over a process grid: `correct` / `smooth` take this rank's
+    [R, F] rows in the block's naming (R = ceil(N / Pr); rows >= N of the last block are padding) and return [R, F] rows.
+
+    Both label propagations run through `runner(z0 [R, ld], K, *, teleport=(a, b), clamp=, reset=) -> [R, ld]` on this
+    rank's feature slice `grid.feature_slice(F)` -- PartitionedAPPNP.run on a LOOP_NONE block built with
+    ld = DistCorrectAndSmooth.slice_ld(grid, F, dtype) in production, a CPU stand-in in the gloo tests.  What the
+    reference computes over the whole graph is reduced over the grid:
+      * sigma = sum |error[mask]| / numel and the mean row sum of y_soft (checked to be 1, as the reference does):
+        float64 partial sums of the real rows, taken once per row (by the ranks of feature group 0, which hold the
+        same full-width rows as the rest of their row block) and all-reduced over every rank, then rounded once --
+        so sigma does not depend on the grid;
+      * the per-row L1 norm of the smoothed error: taken over the full row after the feature slices are assembled
+        (one all-gather among the Pf ranks of a row block, which the [R, F] result needs anyway);
+      * fixed-scale correction resets this rank's rows of the training mask to its rows of the error.
+    Padded rows count nowhere and keep scale 1, so they never turn into NaN.  float32 / bfloat16 only."""
+
+    def __init__(self, num_correction_layers, correction_alpha, num_smoothing_layers, smoothing_alpha,
+                 autoscale=True, scale=1.0, *, grid: "Grid", N: int, runner, col_group=None):
+        self.num_correction_layers, self.correction_alpha = int(num_correction_layers), float(correction_alpha)
+        self.num_smoothing_layers, self.smoothing_alpha = int(num_smoothing_layers), float(smoothing_alpha)
+        self.autoscale, self.scale = autoscale, scale
+        self.grid, self.N, self.runner = grid, N, runner
+        self.col_group = grid.col_group if col_group is None else col_group
+        self.R = rows_per_rank(N, grid.Pr)
+        lo, hi = row_range(N, grid.rp, grid.Pr)
+        self.n_real = hi - lo                     # rows of this block that are nodes; the rest is padding
+
+    @staticmethod
+    def slice_ld(grid: "Grid", F: int, dtype=torch.float32) -> int:
+        """Leading dimension of the [R, ld] slice buffers the runners take: the widest slice, 16-byte vectors."""
+        v = 8 if dtype == torch.bfloat16 else 4
+        return (DistAPPNP.slice_ld(grid, F) + v - 1) // v * v
+
+    def _check(self, y_soft: torch.Tensor):
+        if y_soft.dtype not in (torch.float32, torch.bfloat16):
+            raise RuntimeError(f"DistCorrectAndSmooth takes float32 / bfloat16 rows (got {y_soft.dtype})")
+        if y_soft.dim() != 2 or y_soft.size(0) != self.R:
+            raise RuntimeError(f"y_soft must be this block's [{self.R}, F] rows (got {tuple(y_soft.shape)})")
+
+    def _one_hot(self, y_true: torch.Tensor, y_soft: torch.Tensor) -> torch.Tensor:
+        if y_true.dtype == torch.long:
+            return torch.nn.functional.one_hot(y_true.view(-1), y_soft.size(-1)).to(y_soft.dtype)
+        return y_true
+
+    def _propagate(self, y: torch.Tensor, K: int, alpha: float, clamp=None, reset_mask=None) -> torch.Tensor:
+        """Label propagation of the [R, F] rows `y` (res = (1 - alpha) * y; K x {y = alpha * A_hat y + res; post}),
+        reset rows taking their values from `y`; returns the assembled [R, F] rows."""
+        if K == 0:
+            return y
+        F = y.size(1)
+        a, b = self.grid.feature_slice(F)
+        z0 = torch.zeros((y.size(0), self.slice_ld(self.grid, F, y.dtype)), dtype=y.dtype, device=y.device)
+        z0[:, : b - a] = y[:, a:b]
+        reset = None if reset_mask is None else (reset_mask, z0)
+        z = self.runner(z0, K, teleport=(alpha, 1.0 - alpha), clamp=clamp, reset=reset)
+        # the runner's result lives in its own buffers, which its next run overwrites
+        return _GatherSlices.apply(z, self.grid, F, self.col_group).clone()
+
+    @torch.no_grad()
+    def correct(self, y_soft: torch.Tensor, y_true: torch.Tensor, mask: torch.Tensor) -> torch.Tensor:
+        self._check(y_soft)
+        R, n = self.R, self.n_real
+        y_true = self._one_hot(y_true, y_soft)
+        error = torch.zeros_like(y_soft)
+        error[mask] = y_true - y_soft[mask]
+        if mask.dtype == torch.bool:
+            numel, bad = mask.sum(), mask[n:].sum()
+        else:
+            numel, bad = mask.numel(), (mask >= n).sum()
+        stats = torch.zeros(5, dtype=torch.float64, device=y_soft.device)
+        if self.grid.fp == 0:                      # every rank of a row block holds the same rows: count them once
+            stats[0] = y_soft[:n].sum(dtype=torch.float64)
+            stats[1] = n
+            stats[2] = error[mask].abs().sum(dtype=torch.float64)
+            stats[3] = numel
+            stats[4] = bad
+        if self.grid.world > 1:
+            dist.all_reduce(stats)
+        ysum, nodes, abs_err, numel, bad = stats.tolist()
+        if bad:
+            raise RuntimeError(f"the training mask selects {int(bad)} padded rows (>= N in the last block)")
+        assert abs(ysum / nodes - 1.0) < 1e-2
+        if self.autoscale:
+            smoothed = self._propagate(error, self.num_correction_layers, self.correction_alpha, clamp=(-1.0, 1.0))
+            sigma = torch.tensor(abs_err / numel if numel else float("nan"), dtype=y_soft.dtype, device=y_soft.device)
+            scale = sigma / smoothed.abs().sum(dim=1, keepdim=True)
+            scale[scale.isinf() | (scale > 1000)] = 1.0
+            scale[n:] = 1.0
+            return y_soft + scale * smoothed
+        rmask = mask if mask.dtype == torch.bool else torch.zeros(
+            R, dtype=torch.bool, device=y_soft.device).index_fill_(0, mask, True)
+        smoothed = self._propagate(error, self.num_correction_layers, self.correction_alpha, reset_mask=rmask)
+        return y_soft + self.scale * smoothed
+
+    @torch.no_grad()
+    def smooth(self, y_soft: torch.Tensor, y_true: torch.Tensor, mask: torch.Tensor) -> torch.Tensor:
+        self._check(y_soft)
+        y_soft = y_soft.clone()
+        y_soft[mask] = self._one_hot(y_true, y_soft)
+        return self._propagate(y_soft, self.num_smoothing_layers, self.smoothing_alpha, clamp=(0.0, 1.0))
