@@ -382,6 +382,49 @@ int rgbmp_att_backward_dropout(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, 
 /* out[e*H + h] = the multiplier of edge e, head h, in EDGE order [nnz, H] (the mask of the unfused paths). */
 int rgbmp_dropout_mask(const rgbmp_dropout_t* d, int64_t nnz, int H, float* out, int device, void* stream);
 
+/* SuperGAT's self-supervised attention loss (SuperGATConv.get_attention_loss, supergat.py:26,29; csrc/supergat_loss.cu).
+ * Seeded sampling, keyed like attention dropout but on counter word 2 = 1 (positives) or 2 (negatives):
+ *   positive edge e (its id in the edited edge list) is kept iff keep_thresh == 0 or
+ *     Philox4x32-10(counter = (e, 0, 1, 0), key = (seed lo, seed hi)).word0 >= keep_thresh,
+ *     keep_thresh = floor((1 - edge_sample_ratio) * 2^32) (64-bit: 2^32 drops every edge);
+ *   negative candidate k of round r (r = 0, 1, 2): (w0..w3) = Philox4x32-10((k, r, 2, 0), key),
+ *     (row, col) = (umulhi64(w1:w0, N), umulhi64(w3:w2, N))  (bias <= N / 2^64 per id).
+ * `seed` is read on the device. */
+typedef struct rgbmp_sgat_sample {
+  const int64_t* seed;     /* device pointer to one int64 */
+  const int32_t* eid;      /* [nnz] edge id of every forward-CSR entry (needed when keep_thresh != 0) */
+  const int32_t* eid_t;    /* [nnz] edge id of every transpose-CSR entry; backward only */
+  uint64_t keep_thresh;
+} rgbmp_sgat_sample_t;
+
+/* Negative sampling (torch_geometric.utils.negative_sampling as SuperGATConv calls it): candidates of round r are
+ * rejected iff (row, col) is a pair of U, given as a CSR over rows with sorted columns (u_rowptr [N+1], u_col);
+ * survivors are compacted stably in (round, k) order into neg_src / neg_dst (capacity num_neg) and cut to num_neg;
+ * rounds after the one that reaches num_neg do nothing (decided on the device).  *count_dev = pairs written.
+ * num_neg and sample_size come from the host (the oracle's float formulas); sample_size >= 2^31 is RGBMP_ERANGE. */
+size_t rgbmp_sgat_negative_sampling_workspace_bytes(int64_t sample_size);
+int rgbmp_sgat_negative_sampling(const int64_t* u_rowptr, const int32_t* u_col, int64_t N, const rgbmp_sgat_sample_t* s,
+                                 int64_t num_neg, int64_t sample_size, int32_t* neg_src, int32_t* neg_dst,
+                                 int64_t* count_dev, void* ws, size_t ws_bytes, int device, void* stream);
+/* out[e] = 1 if positive edge e is kept, else 0, in EDGE order (uint8 [nnz]; unfused paths, tests). */
+int rgbmp_sgat_keep_mask(const rgbmp_sgat_sample_t* s, int64_t nnz, uint8_t* out, int device, void* stream);
+
+/* Pair-logit BCE over the kept positives (forward CSR g, rows = targets i, through s->eid) and the negatives
+ * (CSR gneg over the same N rows; the columns are the other endpoints):
+ *   s_ij = scale * <X[i,:], X[j,:]>,  loss = (sum_pos softplus(-s) + sum_neg softplus(s)) / P,  P = pairs
+ * F <= 512, fp32, rows 16-byte aligned (ld % 4 == 0, zero padding up to roundup(F, 4)).  Per-row fp32 partials,
+ * then a fixed-order fp64 reduction: *loss (float, device) and *npairs (int64, device) -- deterministic. */
+size_t rgbmp_sgat_loss_workspace_bytes(int64_t n_rows);
+int rgbmp_sgat_loss_forward(const rgbmp_graph_t* g, const rgbmp_graph_t* gneg, const rgbmp_sgat_sample_t* s,
+                            const float* X, int64_t ldx, int F, float scale, float* loss, int64_t* npairs,
+                            void* ws, size_t ws_bytes, int device, void* stream);
+/* dX = d loss / dX * (*dloss): one pass over target rows (g, gneg) writes every row of dX, one over source rows
+ * (gT with s->eid_t, gnegT) adds into its own rows.  No atomics: bit-reproducible. */
+int rgbmp_sgat_loss_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, const rgbmp_graph_t* gneg,
+                             const rgbmp_graph_t* gnegT, const rgbmp_sgat_sample_t* s, const float* X, int64_t ldx, int F,
+                             float scale, const int64_t* npairs, const float* dloss, float* dX, int64_t lddx,
+                             int device, void* stream);
+
 /* S[i,h] = sum_c A[i,h*C+c]*B[i,h*C+c] */
 int rgbmp_rowdot(const float* A, int64_t lda, const float* B, int64_t ldb, int64_t n_rows,
                  int H, int C, float* S, int device, void* stream);

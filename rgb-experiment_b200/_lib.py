@@ -37,6 +37,11 @@ class DropoutStruct(C.Structure):
     _fields_ = [("seed", c_vp), ("eid", c_vp), ("eid_t", c_vp), ("thresh", C.c_uint32), ("scale", c_f32)]
 
 
+class SgatSampleStruct(C.Structure):
+    """rgbmp_sgat_sample_t"""
+    _fields_ = [("seed", c_vp), ("eid", c_vp), ("eid_t", c_vp), ("keep_thresh", C.c_uint64)]
+
+
 _lib = None
 
 
@@ -51,6 +56,7 @@ def lib():
             "`python rgb-experiment_b200/build.py` (nvcc, sm_100a). There is no CPU fallback.")
     L = C.CDLL(LIB_PATH)
     GP, EP, DP = C.POINTER(GraphStruct), C.POINTER(Epilogue), C.POINTER(DropoutStruct)
+    SP = C.POINTER(SgatSampleStruct)
     sig = {
         "rgbmp_version": (C.c_int, []),
         "rgbmp_last_error": (C.c_char_p, []),
@@ -101,6 +107,14 @@ def lib():
                                                  c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp,
                                                  c_i64, c_vp, c_vp, c_vp, c_sz, C.c_int, c_vp]),
         "rgbmp_dropout_mask": (C.c_int, [DP, c_i64, C.c_int, c_vp, C.c_int, c_vp]),
+        "rgbmp_sgat_negative_sampling_workspace_bytes": (c_sz, [c_i64]),
+        "rgbmp_sgat_negative_sampling": (C.c_int, [c_vp, c_vp, c_i64, SP, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_sz, C.c_int,
+                                                   c_vp]),
+        "rgbmp_sgat_keep_mask": (C.c_int, [SP, c_i64, c_vp, C.c_int, c_vp]),
+        "rgbmp_sgat_loss_workspace_bytes": (c_sz, [c_i64]),
+        "rgbmp_sgat_loss_forward": (C.c_int, [GP, GP, SP, c_vp, c_i64, C.c_int, c_f32, c_vp, c_vp, c_vp, c_sz, C.c_int, c_vp]),
+        "rgbmp_sgat_loss_backward": (C.c_int, [GP, GP, GP, GP, SP, c_vp, c_i64, C.c_int, c_f32, c_vp, c_vp, c_vp, c_i64,
+                                               C.c_int, c_vp]),
         "rgbmp_coalesce_workspace_bytes": (c_sz, [c_i64, c_i64, C.c_int]),
         "rgbmp_coalesce": (C.c_int, [c_vp, c_vp, c_i64, c_i64, C.c_int, c_vp, c_vp, c_vp, c_vp, c_sz, C.c_int, c_vp]),
         "rgbmp_peer_alloc": (C.c_int, [c_sz, c_vp, c_vp, C.c_int]),

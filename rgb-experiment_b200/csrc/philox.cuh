@@ -1,6 +1,6 @@
 // Counter-based attention dropout: the keep rule shared by the fused attention kernels (csrc/att.cu), the mask
 // kernel of the unfused paths (rgbmp_dropout_mask) and, compiled as host code, the test that checks it against the
-// numpy restatement (oracle/philox.py).
+// numpy restatement (oracle/philox.py).  Also the draws of SuperGAT's edge and negative sampling (below).
 //
 // For edge e (its id in the edited edge list) and head h:
 //   u    = Philox4x32-10(counter = (e, h, 0, 0), key = (seed & 0xffffffff, seed >> 32)).word0
@@ -75,6 +75,41 @@ RGBMP_HD uint32_t dropout_bits(PhiloxKey key, uint32_t e, uint32_t h) {
 // the multiplier of edge e, head h: 0 (dropped) or scale (kept)
 RGBMP_HD float dropout_mult(PhiloxKey key, uint32_t e, uint32_t h, uint32_t thresh, float scale) {
   return dropout_bits(key, e, h) < thresh ? 0.0f : scale;
+}
+
+// SuperGAT's self-supervised sampling (csrc/supergat_loss.cu).  Counter word 2 tells the streams apart: 0 attention
+// dropout, 1 the positive keep rule, 2 the negative candidates.
+//   positive edge e is dropped iff Philox(counter (e, 0, 1, 0)).word0 < thresh,  thresh = floor((1 - ratio) * 2^32)
+//   negative candidate k of round r: (w0, w1, w2, w3) = Philox(counter (k, r, 2, 0)),
+//     row = umulhi64(w1:w0, N), col = umulhi64(w3:w2, N)
+// The 64-bit multiply-high maps a uniform 64-bit word onto [0, N) with a bias of at most N / 2^64 per value
+// (< 2^-33 for N < 2^31): every id is hit by floor(2^64 / N) or that plus one of the 2^64 words.
+RGBMP_HD uint32_t edge_sample_bits(PhiloxKey key, uint32_t e) {
+  const uint32_t ctr[4] = {e, 0u, 1u, 0u};
+  uint32_t out[4];
+  philox4x32_10(ctr, key, out);
+  return out[0];
+}
+
+// thresh is 64-bit so that ratio 0 (thresh = 2^32) drops every edge
+RGBMP_HD bool edge_sample_keep(PhiloxKey key, uint32_t e, uint64_t thresh) {
+  return thresh == 0 || (uint64_t)edge_sample_bits(key, e) >= thresh;
+}
+
+RGBMP_HD uint64_t umulhi64(uint64_t a, uint64_t b) {
+#if defined(__CUDA_ARCH__)
+  return __umul64hi(a, b);
+#else
+  return (uint64_t)(((unsigned __int128)a * (unsigned __int128)b) >> 64);
+#endif
+}
+
+RGBMP_HD void neg_candidate(PhiloxKey key, uint32_t k, uint32_t round, uint64_t n, uint32_t& row, uint32_t& col) {
+  const uint32_t ctr[4] = {k, round, 2u, 0u};
+  uint32_t w[4];
+  philox4x32_10(ctr, key, w);
+  row = (uint32_t)umulhi64(((uint64_t)w[1] << 32) | w[0], n);
+  col = (uint32_t)umulhi64(((uint64_t)w[3] << 32) | w[2], n);
 }
 
 }  // namespace rgbmp

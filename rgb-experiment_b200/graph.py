@@ -365,6 +365,22 @@ class Graph:
         """[nnz(,H)] values in forward-CSR order -> transpose-CSR order."""
         return csr_vals[self.tpos().long()].contiguous()
 
+    def undirected_csr(self, symmetrize: bool = True):
+        """(rowptr int64 [N+1], col int32 [n_u]): the unique (src, dst) pairs of the edited edge list -- with
+        `symmetrize` every reversed pair as well (to_undirected) -- as a CSR over src with each row's columns sorted,
+        the set SuperGAT's negative sampler rejects candidates against.  Built once (rgbmp_coalesce, then a lower_bound
+        row pointer) and held like the transpose CSR, instead of a 2 nnz coalesce on every training forward."""
+        key = ("undirected", bool(symmetrize))
+        v = self._vals.get(key)
+        if v is None:
+            from .shim.utils import _coalesce_cuda
+            pairs = _coalesce_cuda(torch.stack([self.e_src, self.e_dst]).to(torch.int64), self.N, bool(symmetrize))
+            nodes = torch.arange(self.N + 1, dtype=torch.int64, device=self.device)
+            rowptr = torch.searchsorted(pairs[0].contiguous(), nodes)
+            v = (rowptr, pairs[1].to(torch.int32))
+            self._vals[key] = v
+        return v
+
     def edge_index(self) -> torch.Tensor:
         """The edited edge list as an int64 [2, nnz] tensor (what PyG's loop utilities return)."""
         v = self._vals.get("edge_index")

@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 import math
-from typing import Optional, Tuple
+from typing import NamedTuple, Optional, Tuple
 
 import torch
 
@@ -234,6 +234,9 @@ FOLD_KHOP = True     # K-hop families apply D^-1/2 (A+I) D^-1/2 as row scalings 
 FUSED_DROPOUT = False  # GATConv / SuperGATConv / FAConv in training mode: True = attention dropout generated inside the
                        # attention kernels (counter-based, keyed by edge id, nothing edge-sized allocated); False = a torch
                        # F.dropout mask per call, so the same torch.manual_seed draws the same masks as it always has
+FUSED_SUPERGAT_LOSS = False  # SuperGATConv in training mode: True = its attention loss on the device (seeded edge and
+                             # negative sampling, fused pair-logit BCE, nothing edge-sized); False = torch sampling and
+                             # [pairs, H, C] gathers, so the same torch.manual_seed draws the same samples as it always has
 
 
 def _khop_gcn(csr: CSR, graph: Graph, x0b: torch.Tensor, K: int, transpose: bool, fold: bool, **epkw):
@@ -746,6 +749,165 @@ def faconv(x, a_l, a_r, graph: Graph, drop_edge: Optional[torch.Tensor] = None, 
     if drop_edge is not None:
         c = c * graph.to_csr_order(drop_edge).view(-1, 1)
     return spmm_heads(c * graph.gcn_val(False).view(-1, 1), x, graph, 1, Cc)
+
+
+# ------------------------------------------------------------------------------------------
+# SuperGAT's self-supervised attention loss (supergat.py:26,29) on the device (csrc/supergat_loss.cu):
+#   positive edge e kept iff Philox(counter (e, 0, 1, 0)).word0 >= floor((1 - edge_sample_ratio) 2^32)
+#   negative candidate k of round r: Philox(counter (k, r, 2, 0)) -> (umulhi64(w1:w0, N), umulhi64(w3:w2, N)),
+#   rejected when it is a pair of U (Graph.undirected_csr), survivors compacted stably and cut to num_neg
+#   loss = BCE-with-logits(att_x.mean(-1), y) = (sum_pos softplus(-s) + sum_neg softplus(s)) / P, s = scale <x'_i, x'_j>
+# ------------------------------------------------------------------------------------------
+class SupergatSamples(NamedTuple):
+    seed: torch.Tensor                     # int64 [1] on the device
+    keep_thresh: int                       # positive edge e dropped iff its draw < keep_thresh (0: all kept)
+    keep_mask: Optional[torch.Tensor]      # bool [nnz] in edge order, when asked for
+    neg_edge_index: torch.Tensor           # int64 [2, n]: (src, dst) of the negatives
+
+
+def supergat_keep_thresh(edge_sample_ratio: float) -> int:
+    """floor(p 2^32) for the dropout_adj rate p = 1 - edge_sample_ratio (2^32 at ratio 0: every edge dropped)."""
+    p = 1.0 - float(edge_sample_ratio)
+    if not 0.0 <= p <= 1.0:
+        raise ValueError(f"edge_sample_ratio must lie in [0, 1] (got {edge_sample_ratio})")
+    return int(math.floor(p * 4294967296.0))
+
+
+def supergat_neg_counts(N: int, E_u: int, num_neg_samples: int) -> Tuple[int, int]:
+    """(num_neg, sample_size) with negative_sampling's own formulas; E_u = the size of the edge set it is given."""
+    size = N * N
+    num_neg = min(int(num_neg_samples), size - E_u)
+    if num_neg <= 0:
+        return num_neg, 0
+    alpha = abs(1 / (1 - 1.1 * (E_u / size)))
+    return num_neg, int(alpha * num_neg)
+
+
+def _sgat_struct(seed: torch.Tensor, keep_thresh: int, graph: Optional[Graph] = None, backward: bool = False):
+    eid = eid_t = None
+    if graph is not None and keep_thresh != 0:
+        eid = graph.fwd.eid
+        eid_t = graph.bwd.eid if backward else None
+    return _lib.SgatSampleStruct(ptr(seed), ptr(eid), ptr(eid_t), keep_thresh)
+
+
+def _sgat_negatives(graph: Graph, seed: torch.Tensor, num_neg_samples: int, is_undirected: bool):
+    """(src, dst) int32 of the device negative sampler; sizing the result is the call's one host synchronisation."""
+    dev = graph.device
+    rowptr, col = graph.undirected_csr(symmetrize=not is_undirected)
+    E_u = graph.nnz if is_undirected else col.numel()        # the torch path counts duplicates when is_undirected
+    num_neg, S = supergat_neg_counts(graph.N, E_u, num_neg_samples)
+    if num_neg <= 0:
+        empty = torch.empty(0, dtype=torch.int32, device=dev)
+        return empty, empty
+    if S >= 1 << 31:
+        raise RuntimeError(f"negative sampling: sample_size {S} >= 2^31 candidates per round")
+    L = lib()
+    src = torch.empty(num_neg, dtype=torch.int32, device=dev)
+    dst = torch.empty(num_neg, dtype=torch.int32, device=dev)
+    count = torch.empty(1, dtype=torch.int64, device=dev)
+    wsb = L.rgbmp_sgat_negative_sampling_workspace_bytes(S)
+    ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
+    s = _sgat_struct(seed, 0)
+    check(L.rgbmp_sgat_negative_sampling(ptr(rowptr), ptr(col), graph.N, C.byref(s), num_neg, S, ptr(src), ptr(dst),
+                                         ptr(count), ptr(ws), wsb, dev.index, stream_of(dev)), "sgat_negative_sampling")
+    n = int(count.item())
+    return src[:n], dst[:n]
+
+
+def supergat_samples(graph: Graph, edge_sample_ratio: float = 1.0, neg_sample_ratio: float = 0.5,
+                     is_undirected: bool = False, seed: Optional[torch.Tensor] = None, mask: bool = False,
+                     generator: Optional[torch.Generator] = None) -> SupergatSamples:
+    """The samples supergat_att_loss draws for `seed` (default: one drawn like dropout_seed): the positive keep rule
+    (and, with mask=True, its bool [nnz] mask in edge order) and the negatives as int64 [2, n]."""
+    seed = dropout_seed(graph.device, generator) if seed is None else seed
+    thresh = supergat_keep_thresh(edge_sample_ratio)
+    keep = None
+    if mask:
+        out = torch.empty(graph.nnz, dtype=torch.uint8, device=graph.device)
+        s = _sgat_struct(seed, thresh)
+        check(lib().rgbmp_sgat_keep_mask(C.byref(s), graph.nnz, ptr(out), graph.device.index, stream_of(graph.device)),
+              "sgat_keep_mask")
+        keep = out.bool()
+    num = int(neg_sample_ratio * edge_sample_ratio * graph.nnz)
+    src, dst = _sgat_negatives(graph, seed, num, is_undirected)
+    return SupergatSamples(seed, thresh, keep, torch.stack([src, dst]).to(torch.int64))
+
+
+def _pair_csrs(graph: Graph, src: torch.Tensor, dst: torch.Tensor):
+    """The negatives as two CSRs over the N nodes: keyed by dst (columns src) and its transpose."""
+    from ._lib import GraphStruct
+    out = []
+    for key, other in ((dst, src), (src, dst)):
+        csr = CSR(key, other, graph.N, graph.N, finish=False)
+        st = GraphStruct(graph.N, graph.N, csr.nnz, ptr(csr.rowptr), ptr(csr.col), 0, 0, 0, 0, None, None, None, None,
+                         None, 0)
+        out.append((csr, st))
+    return out
+
+
+class _SupergatLoss(torch.autograd.Function):
+    """Pair-logit BCE over the kept positives and the negatives; saves only node-sized rows, the seed, the pair count
+    and the negatives' CSRs.  The backward recomputes every logit."""
+
+    @staticmethod
+    def forward(ctx, xp, graph: Graph, scale: float, seed, keep_thresh: int, neg):
+        xb, ldx = _rows_zero_padded(xp)
+        dev, F = xp.device, xp.size(1)
+        L = lib()
+        loss = torch.empty((), dtype=torch.float32, device=dev)
+        npairs = torch.empty(1, dtype=torch.int64, device=dev)
+        wsb = L.rgbmp_sgat_loss_workspace_bytes(graph.N)
+        ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
+        s = _sgat_struct(seed, keep_thresh, graph)
+        check(L.rgbmp_sgat_loss_forward(graph.fwd.ref, C.byref(neg[0][1]), C.byref(s), ptr(xb), ldx, F, scale, ptr(loss),
+                                        ptr(npairs), ptr(ws), wsb, dev.index, stream_of(dev)), "sgat_loss_forward")
+        ctx.graph, ctx.scale, ctx.keep_thresh, ctx.neg = graph, scale, keep_thresh, neg
+        ctx.save_for_backward(xb, seed, npairs)
+        return loss
+
+    @staticmethod
+    def backward(ctx, dloss):
+        xb, seed, npairs = ctx.saved_tensors
+        g, neg = ctx.graph, ctx.neg
+        dev, N, F = xb.device, g.N, xb.size(1)
+        dl = dloss.detach().to(torch.float32).reshape(1).contiguous()
+        dx, lddx = alloc_rows(N, F, torch.float32, dev)
+        s = _sgat_struct(seed, ctx.keep_thresh, g, backward=True)
+        check(lib().rgbmp_sgat_loss_backward(g.fwd.ref, g.bwd.ref, C.byref(neg[0][1]), C.byref(neg[1][1]), C.byref(s),
+                                             ptr(xb), xb.stride(0), F, ctx.scale, ptr(npairs), ptr(dl), ptr(dx), lddx,
+                                             dev.index, stream_of(dev)), "sgat_loss_backward")
+        return dx, None, None, None, None, None
+
+
+def supergat_att_loss(xp: torch.Tensor, graph: Graph, H: int, Cc: int, scale: float, edge_sample_ratio: float = 1.0,
+                      neg_sample_ratio: float = 0.5, is_undirected: bool = False,
+                      neg_edge_index: Optional[torch.Tensor] = None,
+                      generator: Optional[torch.Generator] = None) -> torch.Tensor:
+    """SuperGATConv's get_attention_loss() as one fused op: BCE-with-logits of s = scale * <x'_i, x'_j> (MX: 1/H,
+    SD: 1/(H sqrt(C)) -- att_x.mean(-1) of the per-head dots) over the kept positive edges of `graph` (y = 1) and the
+    negatives (y = 0).  The negatives are `neg_edge_index` (int64 [2, n], ids in [0, N)) or drawn on the device; the
+    seed of the positive sampling and of the sampler is drawn like dropout_seed (`generator` or the device's CUDA
+    generator).  One host synchronisation: the negative count (or, for a given neg_edge_index, its range check)."""
+    _lib.require_cuda(xp, "xp")
+    _lib.require_f32(xp, "supergat_att_loss xp")
+    if xp.dim() != 2 or xp.size(1) != H * Cc or xp.size(0) != graph.N:
+        raise RuntimeError(f"supergat_att_loss: xp must be [N, H*C] = [{graph.N}, {H * Cc}] (got {tuple(xp.shape)})")
+    if graph.fwd.eid is None:
+        raise RuntimeError("supergat_att_loss needs the edge ids of the graph")
+    seed = dropout_seed(graph.device, generator)
+    thresh = supergat_keep_thresh(edge_sample_ratio)
+    if neg_edge_index is None:
+        num = int(neg_sample_ratio * edge_sample_ratio * graph.nnz)
+        src, dst = _sgat_negatives(graph, seed, num, is_undirected)
+    else:
+        _lib.require_cuda(neg_edge_index, "neg_edge_index")
+        if neg_edge_index.dim() != 2 or neg_edge_index.size(0) != 2:
+            raise RuntimeError("neg_edge_index must have shape [2, n]")
+        if neg_edge_index.numel() and bool(((neg_edge_index < 0) | (neg_edge_index >= graph.N)).any()):
+            raise RuntimeError(f"neg_edge_index contains node ids outside [0, {graph.N})")
+        src, dst = (neg_edge_index[i].to(torch.int32).contiguous() for i in (0, 1))
+    return _SupergatLoss.apply(xp, graph, float(scale), seed, thresh, _pair_csrs(graph, src, dst))
 
 
 class _EidView:

@@ -226,7 +226,8 @@ class GATConv(MessagePassing):
 class SuperGATConv(MessagePassing):
     """A12, MX attention (models/supergat.py:15-21,26,29): scores, edge softmax and aggregate in ONE fused
     kernel pass (ops.supergat_mx, csrc/att.cu; backward = one pass per orientation, nothing edge-sized is
-    allocated).  Edge sampling and the BCE loss on the sampled pairs stay PyTorch (node-pair sized)."""
+    allocated).  Edge sampling and the BCE loss on the sampled pairs stay PyTorch (node-pair sized) unless
+    ops.FUSED_SUPERGAT_LOSS: then both run on the device (ops.supergat_att_loss) and nothing edge-sized is allocated."""
 
     def __init__(self, in_channels, out_channels, heads=1, concat=True, negative_slope=0.2, dropout=0.0,
                  add_self_loops=True, bias=True, attention_type="MX", neg_sample_ratio=0.5,
@@ -247,6 +248,7 @@ class SuperGATConv(MessagePassing):
             self.register_parameter("att_l", None)
             self.register_parameter("att_r", None)
         self.att_x = self.att_y = None
+        self._att_loss = None
         if bias:
             self.bias = nn.Parameter(torch.empty(heads * out_channels if concat else out_channels))
         else:
@@ -298,7 +300,12 @@ class SuperGATConv(MessagePassing):
             if keep is not None:
                 alpha = alpha * g.to_csr_order(keep)
             out = ops.spmm_heads(alpha, xp, g, H, C)
-        if self.training:
+        if self.training and ops.FUSED_SUPERGAT_LOSS:                # sampling and BCE on the device
+            scale = 1.0 / H if self.attention_type == "MX" else 1.0 / (H * math.sqrt(C))     # att_x.mean(-1)
+            self._att_loss = ops.supergat_att_loss(xp, g, H, C, scale, self.edge_sample_ratio, self.neg_sample_ratio,
+                                                   self.is_undirected, neg_edge_index)
+            self.att_x = self.att_y = None
+        elif self.training:
             ei = g.edge_index()
             pos_ei, _ = U.dropout_adj(ei, p=1.0 - self.edge_sample_ratio, training=True)
             ei_for_neg = U.to_undirected(ei, N) if not self.is_undirected else ei
@@ -318,6 +325,8 @@ class SuperGATConv(MessagePassing):
     def get_attention_loss(self):
         if not self.training:
             return torch.tensor([0], device=self.lin.weight.device)
+        if self.att_x is None and self._att_loss is not None:
+            return self._att_loss
         return F.binary_cross_entropy_with_logits(self.att_x.mean(dim=-1), self.att_y)
 
 
