@@ -305,7 +305,7 @@ int rgbmp_peer_close(void* ptr, int device);
  * (c) attention kernels
  * ------------------------------------------------------------------------------------------ */
 
-/* Fused edge-score attention + weighted aggregate, one kernel family for the three layers of the reference whose
+/* Fused edge-score attention + weighted aggregate, one kernel family for the layers of the reference whose
  * per-edge weight is a function of the two endpoints (csrc/att.cu).  For target row i over its in-edges j -> i:
  *   RGBMP_ATT_GAT  GATConv (gat.py:18-21,28-30; SURVEY.md A10/A11):
  *                  e = leaky_relu(a_nbr[j] + a_own[i]);  alpha = exp(e - max)/(sum + 1e-16);  out[i] = sum alpha*mask*X[j]
@@ -313,6 +313,8 @@ int rgbmp_peer_close(void* ptr, int device);
  *                  e = leaky_relu((a_nbr[j] + a_own[i]) * sigmoid(<X[i,h,:], X[j,h,:]>)), then as GAT
  *   RGBMP_ATT_FA   FAConv (fagcn.py:15,31; A13), H = 1:
  *                  out[i] = sum tanh(a_nbr[j] + a_own[i]) * dinv[j]*dinv[i] * mask * X[j]        (no softmax)
+ *   RGBMP_ATT_SD   SuperGATConv, SD attention (A12), through rgbmp_att_sd_forward / _backward only:
+ *                  e = leaky_relu(logit_scale * <X[i,h,:], X[j,h,:]>), then as GAT
  * X [n_cols, H*C] (ldx), a_nbr [n_cols,H] (a_src / att_l side), a_own [n_rows,H] (a_dst / att_r side).
  * Shapes: H == 1 with any C <= 128 (padding columns of X up to roundup(C,4) must be ZERO), or C a power of two in
  * 8..128 with any H (heads are tiled over the grid) -- rgbmp_att_supported() says which; the host layer pads heads.
@@ -325,6 +327,7 @@ int rgbmp_peer_close(void* ptr, int device);
 #define RGBMP_ATT_GAT 0
 #define RGBMP_ATT_MX  1
 #define RGBMP_ATT_FA  2
+#define RGBMP_ATT_SD  3
 int rgbmp_att_supported(int score, int H, int C);
 size_t rgbmp_att_forward_workspace_bytes(const rgbmp_graph_t* g, int H, int C);
 int rgbmp_att_forward(const rgbmp_graph_t* g, int score, const float* X, int64_t ldx,
@@ -379,6 +382,23 @@ int rgbmp_att_backward_dropout(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, 
                                const float* dout, int64_t ldd,
                                float* dX, int64_t lddx, float* dXf, int64_t lddxf, float* da_nbr, float* da_own,
                                void* ws, size_t ws_bytes, int device, void* stream);
+/* SuperGATConv's SD attention: the RGBMP_ATT_SD score with no score scalars.  g must be square (X holds both
+ * endpoints), gT its transpose.  logit_scale is 1/sqrt(C) of the UNPADDED head width when the caller pads heads to a
+ * supported C.  At most one of `drop` (explicit mask, forward-CSR order; the backward also needs tpos) and `d`
+ * (dropout generated in the kernels; d->eid, and d->eid_t in the backward) may be non-NULL.  Workspaces: the
+ * rgbmp_att_forward / backward_workspace_bytes queries.  The forward saves rowmax, rowsum [n,H]; the backward runs
+ * one pass per orientation like MX (dXf = scratch [n, lddxf]) and writes dX.  Unsupported H / C, NULL pointers,
+ * both dropout forms or a non-square graph: RGBMP_EINVAL.  rgbmp_att_forward / backward(_dropout) do not take
+ * score 3. */
+int rgbmp_att_sd_forward(const rgbmp_graph_t* g, const float* X, int64_t ldx, int H, int C, float logit_scale,
+                         float slope, const float* drop, const rgbmp_dropout_t* d, float* out, int64_t ldo,
+                         float* rowmax, float* rowsum, void* ws, size_t ws_bytes, int device, void* stream);
+int rgbmp_att_sd_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, const float* X, int64_t ldx, int H, int C,
+                          float logit_scale, float slope, const float* drop, const int32_t* tpos,
+                          const rgbmp_dropout_t* d, const float* rowmax, const float* rowsum,
+                          const float* out, int64_t ldo, const float* dout, int64_t ldd,
+                          float* dX, int64_t lddx, float* dXf, int64_t lddxf,
+                          void* ws, size_t ws_bytes, int device, void* stream);
 /* out[e*H + h] = the multiplier of edge e, head h, in EDGE order [nnz, H] (the mask of the unfused paths). */
 int rgbmp_dropout_mask(const rgbmp_dropout_t* d, int64_t nnz, int H, float* out, int device, void* stream);
 

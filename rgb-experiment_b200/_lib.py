@@ -107,6 +107,10 @@ def lib():
                                                  c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp,
                                                  c_i64, c_vp, c_vp, c_vp, c_sz, C.c_int, c_vp]),
         "rgbmp_dropout_mask": (C.c_int, [DP, c_i64, C.c_int, c_vp, C.c_int, c_vp]),
+        "rgbmp_att_sd_forward": (C.c_int, [GP, c_vp, c_i64, C.c_int, C.c_int, c_f32, c_f32, c_vp, DP, c_vp, c_i64, c_vp, c_vp,
+                                           c_vp, c_sz, C.c_int, c_vp]),
+        "rgbmp_att_sd_backward": (C.c_int, [GP, GP, c_vp, c_i64, C.c_int, C.c_int, c_f32, c_f32, c_vp, c_vp, DP, c_vp, c_vp,
+                                            c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_sz, C.c_int, c_vp]),
         "rgbmp_sgat_negative_sampling_workspace_bytes": (c_sz, [c_i64]),
         "rgbmp_sgat_negative_sampling": (C.c_int, [c_vp, c_vp, c_i64, SP, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_sz, C.c_int,
                                                    c_vp]),

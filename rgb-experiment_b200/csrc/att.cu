@@ -1,9 +1,10 @@
 // Fused edge-score attention + aggregate over CSR, forward and backward (sm_100a).
 //
-// ONE kernel family for the three layers of the reference whose per-edge weight is a function of the two
-// endpoints (SURVEY.md 8a rows a4, a5, a9), selected by the template parameter SC:
+// ONE kernel family for the layers of the reference whose per-edge weight is a function of the two endpoints
+// (SURVEY.md 8a rows a4, a5, a9), selected by the template parameter SC:
 //   SC_GAT  GATConv (gat.py:18-21, A10):       e = leaky_relu(a_src[j] + a_dst[i]);                 softmax over i's in-edges
 //   SC_MX   SuperGATConv MX (supergat.py:15-21, A12): e = leaky_relu((a_l[j] + a_r[i]) * sigmoid(<x_i, x_j>)); softmax
+//   SC_SD   SuperGATConv SD (A12):             e = leaky_relu(logit_scale * <x_i, x_j>), logit_scale = 1/sqrt(C); softmax
 //   SC_FA   FAConv (fagcn.py:15,31, A13):      w = tanh(a_l[j] + a_r[i]) * dinv[j] * dinv[i];        no softmax, H = 1
 // out[i] = sum_j weight_ij * mask_ij * X[j].  No edge-sized tensor is ever written: the forward is one pass with
 // an online softmax, the backward recomputes the weights from per-node statistics (A10 identities).
@@ -27,6 +28,8 @@
 //   FA:   da_r[i] = <dout_i, Q_i>,  Q_i = sum_j (1 - tanh^2) dinv_j dinv_i mask_ij x_j, likewise;
 //   MX:   the logit <x_i, x_j> sends gradient to BOTH endpoints' features, so its backward runs one pass per
 //         orientation anyway (forward CSR: dX_i += dlogit x_j, da_r; transpose CSR: dX_j += alpha dout_i + dlogit x_i, da_l).
+//   SD:   MX without the score scalars and the sigmoid gate: the same two passes, no da_l / da_r.
+#include <math.h>
 #include <stdlib.h>
 #include "common.cuh"
 #include "philox.cuh"
@@ -38,7 +41,7 @@ constexpr int ATT_THREADS = 256;
 constexpr float LOG2E = 1.4426950408889634f;
 constexpr float LN2 = 0.6931471805599453f;
 constexpr int U = 2;       // edges per step
-enum { SC_GAT = RGBMP_ATT_GAT, SC_MX = RGBMP_ATT_MX, SC_FA = RGBMP_ATT_FA };
+enum { SC_GAT = RGBMP_ATT_GAT, SC_MX = RGBMP_ATT_MX, SC_FA = RGBMP_ATT_FA, SC_SD = RGBMP_ATT_SD };
 
 __device__ __forceinline__ float leaky_relu(float x, float slope) { return x > 0.f ? x : x * slope; }
 __device__ __forceinline__ float ex2(float x) {
@@ -113,6 +116,9 @@ struct AttParams {
   // long-row scratch
   float* part_m; float* part_s; float* part_q; float* part_acc; float* part_acc2;
   int64_t ldp;
+  // SD: natural-domain scale of the logit <x_i, x_j> (1/sqrt(C) of the UNPADDED head width); last, so that the
+  // parameter offsets of the other variants do not move
+  float logit_scale;
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -159,6 +165,9 @@ __device__ __forceinline__ float head_sum(float v, int LPH) {
   for (int o = LPH >> 1; o > 0; o >>= 1) v += __shfl_xor_sync(FULLMASK, v, o);
   return v;
 }
+
+// SD's raw score in the log2 domain; forward and both backward passes round it the same way
+__device__ __forceinline__ float sd_raw(const AttParams& p, float logit) { return logit * (p.logit_scale * LOG2E); }
 
 __device__ __forceinline__ void load_own(const float* X, int64_t ld, int64_t row, const Lane& L, float4 (&x)[2]) {
   x[0] = L.nact > 0 ? __ldg(reinterpret_cast<const float4*>(X + row * ld + L.f)) : zero4();
@@ -244,10 +253,15 @@ __device__ __forceinline__ void fwd_consume(const AttParams& p, const float4 (&x
     float mb = -INFINITY;
 #pragma unroll
     for (int u = 0; u < UU; ++u) {
-      float raw = sn[u] + so;                               // log2 domain (both terms pre-scaled)
-      if constexpr (SC == SC_MX) {
-        const float dot = head_sum(dot4(xi[0], x[u][0]) + dot4(xi[1], x[u][1]), p.LPH);
-        raw *= sigmoidf(dot);
+      float raw;
+      if constexpr (SC == SC_SD) {
+        raw = sd_raw(p, head_sum(dot4(xi[0], x[u][0]) + dot4(xi[1], x[u][1]), p.LPH));
+      } else {
+        raw = sn[u] + so;                                   // log2 domain (both terms pre-scaled)
+        if constexpr (SC == SC_MX) {
+          const float dot = head_sum(dot4(xi[0], x[u][0]) + dot4(xi[1], x[u][1]), p.LPH);
+          raw *= sigmoidf(dot);
+        }
       }
       e[u] = leaky_relu(raw, p.slope);
       if (u < nvalid) mb = fmaxf(mb, e[u]);
@@ -304,7 +318,8 @@ __device__ __forceinline__ void fwd_range(const AttParams& p, int64_t k0, int64_
   auto gather = [&](uint32_t c, float4 (&xx)[2], float& aa, float& dd) {
     xx[0] = a0 ? __ldg(reinterpret_cast<const float4*>(xb0 + (size_t)c * row_bytes)) : zero4();
     xx[1] = a1 ? __ldg(reinterpret_cast<const float4*>(xb1 + (size_t)c * row_bytes)) : zero4();
-    aa = __ldg(reinterpret_cast<const float*>(snb + (size_t)c * sn_bytes));
+    if constexpr (SC == SC_SD) aa = 0.f;                    // SD has no per-neighbour scalar
+    else aa = __ldg(reinterpret_cast<const float*>(snb + (size_t)c * sn_bytes));
     if constexpr (SC == SC_FA) dd = __ldg(p.dinv + c);
     else dd = 0.f;
   };
@@ -404,9 +419,9 @@ __global__ void __launch_bounds__(ATT_THREADS, fwd_minb<SC, TRAIN>()) att_fwd_ro
   float so = 0.f, d_own = 0.f;
   float4 xi[2] = {zero4(), zero4()};
   if (live) {
-    so = __ldg(p.so + row * p.H + L.h);
+    if constexpr (SC != SC_SD) so = __ldg(p.so + row * p.H + L.h);
     if constexpr (SC == SC_FA) d_own = __ldg(p.dinv + row);
-    if constexpr (SC == SC_MX) load_own(p.Xo, p.ldo_, row, L, xi);
+    if constexpr (SC == SC_MX || SC == SC_SD) load_own(p.Xo, p.ldo_, row, L, xi);
   }
   FwdState st;
   fwd_init(st);
@@ -448,11 +463,11 @@ __global__ void __launch_bounds__(ATT_THREADS, fwd_minb<SC, TRAIN>()) att_fwd_lo
   int64_t row, k0, k1;
   item_range(p, G, row, k0, k1);
   const Lane L = lane_of(p, gl);
-  const float so = __ldg(p.so + row * p.H + L.h);
+  const float so = (SC == SC_SD) ? 0.f : __ldg(p.so + row * p.H + L.h);
   float d_own = 0.f;
   float4 xi[2] = {zero4(), zero4()};
   if constexpr (SC == SC_FA) d_own = __ldg(p.dinv + row);
-  if constexpr (SC == SC_MX) load_own(p.Xo, p.ldo_, row, L, xi);
+  if constexpr (SC == SC_MX || SC == SC_SD) load_own(p.Xo, p.ldo_, row, L, xi);
   FwdState st;
   fwd_init(st);
   fwd_range<SC, TRAIN, G, UU, PIPE, DR>(p, k0, k1, gl, L, so, d_own, xi, drop_key<DR>(p), sm_ids, st);
@@ -589,6 +604,7 @@ __global__ void __launch_bounds__(256) att_scale_kernel(const float* __restrict_
 //   GAT: raw = a_src[j] + a_dst[i]:               da_src[j] += draw ; da_dst[i] = <dout_i, P_i> - S_i q_i
 //   MX:  raw = u * s, u = a_l[j] + a_r[i], s = sigmoid(<x_i, x_j>):
 //        da_l[j] += draw*s ; da_r[i] += draw*s ; dlogit = draw*u*s(1-s) ; dX_j += dlogit x_i ; dX_i += dlogit x_j
+//   SD:  raw = logit_scale * <x_i, x_j>:           dlogit = draw*logit_scale ; dX_j += dlogit x_i ; dX_i += dlogit x_j
 //   all: dX_j += alpha_ij mask_ij dout_i
 //   FA:  w = tanh(u) dinv_j dinv_i: dX_j += w mask dout_i ; da_l[j] += <dout_i, x_j> dinv_j dinv_i mask (1 - tanh^2) ;
 //        da_r[i] = <dout_i, Q_i>
@@ -616,7 +632,8 @@ att_bwd_prep_kernel(const float* __restrict__ dout, int64_t ldd, const float* __
     const float* b = out + i * ldo + h * C;
     float s = 0.f;
     for (int c = 0; c < C; ++c) s = fmaf(a[c], b[c], s);
-    stats[t] = make_float4(a_own[t] * LOG2E, rowmax[t] * LOG2E, 1.0f / (rowsum[t] + 1e-16f), s);
+    const float so = (SC == SC_SD) ? 0.f : a_own[t] * LOG2E;     // SD has no target-side scalar
+    stats[t] = make_float4(so, rowmax[t] * LOG2E, 1.0f / (rowsum[t] + 1e-16f), s);
     if constexpr (SC == SC_GAT) {
       const float* b2 = out2 + i * ldo2 + h * C;
       float s2 = 0.f;
@@ -640,8 +657,9 @@ __device__ __forceinline__ void bwdT_range(const AttParams& p, int64_t k0, int64
   const char* db0 = reinterpret_cast<const char*>(p.Xn + L.f);
   const char* db1 = reinterpret_cast<const char*>(p.Xn + L.f + 4);
   const uint32_t d_bytes = (uint32_t)(p.ldn * 4);
-  const char* xb0 = (SC == SC_MX) ? reinterpret_cast<const char*>(p.Xn2 + L.f) : nullptr;
-  const char* xb1 = (SC == SC_MX) ? reinterpret_cast<const char*>(p.Xn2 + L.f + 4) : nullptr;
+  constexpr bool LOGIT = SC == SC_MX || SC == SC_SD;       // the score reads <x_i, x_j>: x_i is gathered too
+  const char* xb0 = LOGIT ? reinterpret_cast<const char*>(p.Xn2 + L.f) : nullptr;
+  const char* xb1 = LOGIT ? reinterpret_cast<const char*>(p.Xn2 + L.f + 4) : nullptr;
   const uint32_t x_bytes = (uint32_t)(p.ldn2 * 4);
   const char* stb = reinterpret_cast<const char*>(p.stats + L.h);
   const uint32_t st_bytes = (uint32_t)(p.H * 16);
@@ -669,7 +687,7 @@ __device__ __forceinline__ void bwdT_range(const AttParams& p, int64_t k0, int64
         const uint32_t ci = cc[u];
         d[u][0] = a0 ? __ldg(reinterpret_cast<const float4*>(db0 + (size_t)ci * d_bytes)) : zero4();
         d[u][1] = a1 ? __ldg(reinterpret_cast<const float4*>(db1 + (size_t)ci * d_bytes)) : zero4();
-        if constexpr (SC == SC_MX) {
+        if constexpr (LOGIT) {
           x2[u][0] = a0 ? __ldg(reinterpret_cast<const float4*>(xb0 + (size_t)ci * x_bytes)) : zero4();
           x2[u][1] = a1 ? __ldg(reinterpret_cast<const float4*>(xb1 + (size_t)ci * x_bytes)) : zero4();
         }
@@ -679,8 +697,9 @@ __device__ __forceinline__ void bwdT_range(const AttParams& p, int64_t k0, int64
       for (int u = 0; u < UB; ++u) {
         // per-head dot products: lane-local, then reduced over the LPH lanes of the head (whole warp executes)
         const float dot = head_sum(dot4(d[u][0], xj[0]) + dot4(d[u][1], xj[1]), p.LPH);     // <dout_i, x_j>
-        float sg = 1.0f;
+        float sg = 1.0f, lg = 0.f;
         if constexpr (SC == SC_MX) sg = sigmoidf(head_sum(dot4(x2[u][0], xj[0]) + dot4(x2[u][1], xj[1]), p.LPH));
+        if constexpr (SC == SC_SD) lg = head_sum(dot4(x2[u][0], xj[0]) + dot4(x2[u][1], xj[1]), p.LPH);  // <x_i, x_j>
         if (j + u < nb) {
           float mu = 1.0f;
           if constexpr (DR) mu = drop_mult(p, key, k0 + off + j + u, L.h);
@@ -694,7 +713,7 @@ __device__ __forceinline__ void bwdT_range(const AttParams& p, int64_t k0, int64
             das = fmaf(dot * wgt, 1.0f - t * t, das);
           } else {
             const float uu = so2 + st[u].x;                  // log2 domain
-            const float raw = uu * sg;
+            const float raw = (SC == SC_SD) ? sd_raw(p, lg) : uu * sg;
             const float alpha = ex2(leaky_relu(raw, p.slope) - st[u].y) * st[u].z;
             const float w = alpha * mu;
             fma4(acc[0], w, d[u][0]);
@@ -705,6 +724,10 @@ __device__ __forceinline__ void bwdT_range(const AttParams& p, int64_t k0, int64
               fma4(acc[0], dlog, x2[u][0]);
               fma4(acc[1], dlog, x2[u][1]);
               das = fmaf(draw, sg, das);
+            } else if constexpr (SC == SC_SD) {
+              const float dlog = draw * p.logit_scale;
+              fma4(acc[0], dlog, x2[u][0]);
+              fma4(acc[1], dlog, x2[u][1]);
             } else {
               das += draw;
             }
@@ -730,7 +753,7 @@ __global__ void __launch_bounds__(ATT_THREADS, bwdT_minb<SC>()) att_bwdT_rows_ke
   float so2 = 0.f, d_own = 0.f;
   float4 xj[2] = {zero4(), zero4()}, acc[2] = {zero4(), zero4()};
   if (live) {
-    so2 = __ldg(p.so + row * p.H + L.h) * (SC == SC_FA ? 1.0f : LOG2E);
+    if constexpr (SC != SC_SD) so2 = __ldg(p.so + row * p.H + L.h) * (SC == SC_FA ? 1.0f : LOG2E);
     if constexpr (SC == SC_FA) d_own = __ldg(p.dinv + row);
     load_own(p.Xo, p.ldo_, row, L, xj);
   }
@@ -791,7 +814,7 @@ __global__ void __launch_bounds__(ATT_THREADS, bwdT_minb<SC>()) att_bwdT_long_ke
   int64_t row, k0, k1;
   item_range(p, G, row, k0, k1);
   const Lane L = lane_of(p, gl);
-  const float so2 = __ldg(p.so + row * p.H + L.h) * (SC == SC_FA ? 1.0f : LOG2E);
+  const float so2 = (SC == SC_SD) ? 0.f : __ldg(p.so + row * p.H + L.h) * (SC == SC_FA ? 1.0f : LOG2E);
   float d_own = 0.f;
   if constexpr (SC == SC_FA) d_own = __ldg(p.dinv + row);
   float4 xj[2], acc[2] = {zero4(), zero4()};
@@ -819,9 +842,9 @@ __global__ void __launch_bounds__(256) att_bwd_combine_kernel(const AttParams p)
   if (p.H == 1 ? (f == 0) : (f % p.C == 0)) p.ds[row * p.H + h] = s;
 }
 
-// ---- MX forward-orientation pass: rows = targets i, neighbours = sources j ----------------------------------
-//   dXf_i = sum_j dlogit_ij x_j ;  da_r[i] = sum_j draw_ij * s_ij
-template <int G, bool DR>
+// ---- MX / SD forward-orientation pass: rows = targets i, neighbours = sources j ----------------------------
+//   dXf_i = sum_j dlogit_ij x_j ;  MX: da_r[i] = sum_j draw_ij * s_ij
+template <int SC, int G, bool DR>
 __device__ __forceinline__ void bwdF_range(const AttParams& p, int64_t k0, int64_t k1, int gl, const Lane& L, const float4 st_own,
                                            const float4 (&xi)[2], const float4 (&di)[2], PhiloxKey key, int32_t* sm_ids,
                                            float4 (&acc)[2], float& dar) {
@@ -859,31 +882,41 @@ __device__ __forceinline__ void bwdF_range(const AttParams& p, int64_t k0, int64
         const uint32_t cj = cc[u];
         x[u][0] = a0 ? __ldg(reinterpret_cast<const float4*>(xb0 + (size_t)cj * row_bytes)) : zero4();
         x[u][1] = a1 ? __ldg(reinterpret_cast<const float4*>(xb1 + (size_t)cj * row_bytes)) : zero4();
-        as[u] = __ldg(reinterpret_cast<const float*>(snb + (size_t)cj * sn_bytes));
+        if constexpr (SC == SC_MX) as[u] = __ldg(reinterpret_cast<const float*>(snb + (size_t)cj * sn_bytes));
       }
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         const float dot = head_sum(dot4(di[0], x[u][0]) + dot4(di[1], x[u][1]), p.LPH);              // <dout_i, x_j>
-        const float sg = sigmoidf(head_sum(dot4(xi[0], x[u][0]) + dot4(xi[1], x[u][1]), p.LPH));     // sigmoid(<x_i, x_j>)
+        const float lg = head_sum(dot4(xi[0], x[u][0]) + dot4(xi[1], x[u][1]), p.LPH);              // <x_i, x_j>
+        const float sg = (SC == SC_MX) ? sigmoidf(lg) : 0.f;
         if (j + u < nb) {
           float mu;
           if constexpr (DR) mu = drop_mult(p, key, k0 + off + j + u, L.h);
           else mu = p.drop ? __ldg(p.drop + (k0 + off + j + u) * p.H + L.h) : 1.0f;
-          const float uu = as[u] + st_own.x;
-          const float raw = uu * sg;
-          const float alpha = ex2(leaky_relu(raw, p.slope) - st_own.y) * st_own.z;
-          const float draw = alpha * (mu * dot - st_own.w) * (raw > 0.f ? 1.0f : p.slope);
-          const float dlog = draw * (uu * LN2) * sg * (1.0f - sg);
-          fma4(acc[0], dlog, x[u][0]);
-          fma4(acc[1], dlog, x[u][1]);
-          dar = fmaf(draw, sg, dar);
+          if constexpr (SC == SC_SD) {
+            const float raw = sd_raw(p, lg);
+            const float alpha = ex2(leaky_relu(raw, p.slope) - st_own.y) * st_own.z;
+            const float draw = alpha * (mu * dot - st_own.w) * (raw > 0.f ? 1.0f : p.slope);
+            const float dlog = draw * p.logit_scale;
+            fma4(acc[0], dlog, x[u][0]);
+            fma4(acc[1], dlog, x[u][1]);
+          } else {
+            const float uu = as[u] + st_own.x;
+            const float raw = uu * sg;
+            const float alpha = ex2(leaky_relu(raw, p.slope) - st_own.y) * st_own.z;
+            const float draw = alpha * (mu * dot - st_own.w) * (raw > 0.f ? 1.0f : p.slope);
+            const float dlog = draw * (uu * LN2) * sg * (1.0f - sg);
+            fma4(acc[0], dlog, x[u][0]);
+            fma4(acc[1], dlog, x[u][1]);
+            dar = fmaf(draw, sg, dar);
+          }
         }
       }
     }
   }
 }
 
-template <int G, bool DR>
+template <int SC, int G, bool DR>
 __global__ void __launch_bounds__(ATT_THREADS, RGBMP_ATT_OCC >= 1 ? 3 : 2) att_bwdF_rows_kernel(const AttParams p) {
   __shared__ __align__(16) int32_t sm_ids[ATT_THREADS];
   const int gl = threadIdx.x % G;
@@ -898,7 +931,7 @@ __global__ void __launch_bounds__(ATT_THREADS, RGBMP_ATT_OCC >= 1 ? 3 : 2) att_b
     st_own = __ldg(p.stats + row * p.H + L.h);
   }
   float dar = 0.f;
-  bwdF_range<G, DR>(p, k0, k1, gl, L, st_own, xi, di, drop_key<DR>(p), sm_ids, acc, dar);
+  bwdF_range<SC, G, DR>(p, k0, k1, gl, L, st_own, xi, di, drop_key<DR>(p), sm_ids, acc, dar);
   if (!live || L.nact == 0) return;
 #pragma unroll
   for (int v = 0; v < 2; ++v)
@@ -906,7 +939,7 @@ __global__ void __launch_bounds__(ATT_THREADS, RGBMP_ATT_OCC >= 1 ? 3 : 2) att_b
   if (L.lead) p.ds[row * p.H + L.h] = dar;
 }
 
-template <int G, bool DR>
+template <int SC, int G, bool DR>
 __global__ void __launch_bounds__(ATT_THREADS, RGBMP_ATT_OCC >= 1 ? 3 : 2) att_bwdF_long_kernel(const AttParams p) {
   constexpr int Q = ATT_THREADS / G;
   __shared__ __align__(16) int32_t sm_ids[ATT_THREADS];
@@ -921,7 +954,7 @@ __global__ void __launch_bounds__(ATT_THREADS, RGBMP_ATT_OCC >= 1 ? 3 : 2) att_b
   load_own(p.Do, p.lddo, row, L, di);
   const float4 st_own = __ldg(p.stats + row * p.H + L.h);
   float dar = 0.f;
-  bwdF_range<G, DR>(p, k0, k1, gl, L, st_own, xi, di, drop_key<DR>(p), sm_ids, acc, dar);
+  bwdF_range<SC, G, DR>(p, k0, k1, gl, L, st_own, xi, di, drop_key<DR>(p), sm_ids, acc, dar);
   bwd_long_merge<G>(p, gl, q, L, acc, dar, sm_acc, sm_s);
 }
 
@@ -1032,14 +1065,17 @@ static int launch_fwd_v(const AttParams& p, const Shape& s, cudaStream_t st) {
   return 0;
 }
 
-// the fused-dropout forward exists in the default loop variant only
+// the fused-dropout and the SD forwards exist in the default loop variant only (SD spills in the other two)
 template <int SC, bool TRAIN, bool DR>
 static int launch_fwd(const AttParams& p, const Shape& s, cudaStream_t st) {
-  if constexpr (DR) return launch_fwd_v<SC, TRAIN, 2, false, true>(p, s, st);
-  switch (att_fwd_variant()) {
-    case 1: return launch_fwd_v<SC, TRAIN, 4, false, false>(p, s, st);
-    case 0: return launch_fwd_v<SC, TRAIN, 2, true, false>(p, s, st);
-    default: return launch_fwd_v<SC, TRAIN, 2, false, false>(p, s, st);
+  if constexpr (DR || SC == SC_SD) {
+    return launch_fwd_v<SC, TRAIN, 2, false, DR>(p, s, st);
+  } else {
+    switch (att_fwd_variant()) {
+      case 1: return launch_fwd_v<SC, TRAIN, 4, false, false>(p, s, st);
+      case 0: return launch_fwd_v<SC, TRAIN, 2, true, false>(p, s, st);
+      default: return launch_fwd_v<SC, TRAIN, 2, false, false>(p, s, st);
+    }
   }
 }
 
@@ -1063,19 +1099,19 @@ static int launch_bwdT(const AttParams& p, const Shape& s, cudaStream_t st) {
   return 0;
 }
 
-template <bool DR>
+template <int SC, bool DR>
 static int launch_bwdF(const AttParams& p, const Shape& s, cudaStream_t st) {
   const int HC = p.H * p.C;
   dim3 grid_rows((unsigned)ceil_div(p.n_rows, ATT_THREADS / s.G), (unsigned)s.tiles);
-  ATT_G_SWITCH(s.G, (att_bwdF_rows_kernel<4, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
-               (att_bwdF_rows_kernel<8, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
-               (att_bwdF_rows_kernel<16, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)))
+  ATT_G_SWITCH(s.G, (att_bwdF_rows_kernel<SC, 4, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
+               (att_bwdF_rows_kernel<SC, 8, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
+               (att_bwdF_rows_kernel<SC, 16, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)))
   RGBMP_LAUNCH_CHECK("att_bwdF_rows_kernel");
   if (p.n_items > 0) {
     dim3 grid_items((unsigned)p.n_items, (unsigned)s.tiles);
-    ATT_G_SWITCH(s.G, (att_bwdF_long_kernel<4, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
-                 (att_bwdF_long_kernel<8, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
-                 (att_bwdF_long_kernel<16, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)))
+    ATT_G_SWITCH(s.G, (att_bwdF_long_kernel<SC, 4, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
+                 (att_bwdF_long_kernel<SC, 8, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
+                 (att_bwdF_long_kernel<SC, 16, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)))
     RGBMP_LAUNCH_CHECK("att_bwdF_long_kernel");
     att_bwd_combine_kernel<<<(unsigned)ceil_div(p.n_long * HC, 256), 256, 0, st>>>(p);
     RGBMP_LAUNCH_CHECK("att_bwd_combine_kernel");
@@ -1091,7 +1127,7 @@ extern "C" {
 
 int rgbmp_att_supported(int score, int H, int C) {
   Shape s;
-  if (score < RGBMP_ATT_GAT || score > RGBMP_ATT_FA) return 0;
+  if (score < RGBMP_ATT_GAT || score > RGBMP_ATT_SD) return 0;
   if (score == RGBMP_ATT_FA && H != 1) return 0;
   return att_shape(H, C, &s) ? 1 : 0;
 }
@@ -1109,24 +1145,48 @@ static void set_dropout(AttParams& p, const rgbmp_dropout_t* d, const int32_t* e
   p.dscale = d->scale;
 }
 
+// The generic entry points take GAT / MX / FA (sd == false: score 3 stays unsupported there); SD comes through
+// rgbmp_att_sd_* only (sd == true, score == RGBMP_ATT_SD), which check its arguments first.  SD reads no score
+// scalars (a_nbr / a_own NULL) and scales the logit by logit_scale.
+static bool score_ok(int score, bool sd) { return sd ? score == RGBMP_ATT_SD : score >= RGBMP_ATT_GAT && score <= RGBMP_ATT_FA; }
+
+// What the SD entry points check before att_forward / att_backward (which check pointers and the dropout descriptor):
+// the shape (EINVAL here), a square graph -- X holds the features of both endpoints -- and gT its transpose, a finite
+// scale, and at most one dropout form.
+static int check_sd(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int H, int C, float logit_scale, const float* drop,
+                    const rgbmp_dropout_t* d, const char* fn) {
+  int rc = check_g(g, fn);
+  if (rc) return rc;
+  if (gT && (rc = check_g(gT, fn))) return rc;
+  Shape s;
+  if (!att_shape(H, C, &s))
+    return fail(RGBMP_EINVAL, "%s: unsupported H %d / C %d (H == 1 with C <= 128, or C in {8..128} a power of two)", fn, H, C);
+  if (g->n_rows != g->n_cols || (gT && (gT->n_rows != g->n_cols || gT->n_cols != g->n_rows || gT->nnz != g->nnz)))
+    return fail(RGBMP_EINVAL, "%s: SD needs a square graph (and its transpose)", fn);
+  if (!isfinite(logit_scale)) return fail(RGBMP_EINVAL, "%s: logit_scale must be finite", fn);
+  if (drop && d) return fail(RGBMP_EINVAL, "%s: at most one of drop / d", fn);
+  return 0;
+}
+
 // d == NULL: the explicit `drop` mask (or none); d != NULL: fused dropout
 static int att_forward(const char* fn, const rgbmp_graph_t* g, int score, const float* X, int64_t ldx, const float* a_nbr,
                        const float* a_own, const float* dinv, int H, int C, float slope, const float* drop,
                        const rgbmp_dropout_t* d, float* out, int64_t ldo, float* rowmax, float* rowsum, float* out2,
-                       int64_t ldo2, float* rowq, void* ws, size_t ws_bytes, int device, void* stream) {
+                       int64_t ldo2, float* rowq, void* ws, size_t ws_bytes, int device, void* stream,
+                       bool sd = false, float logit_scale = 0.f) {
   int rc = check_g(g, fn);
   if (rc) return rc;
   Shape s;
-  if (score < RGBMP_ATT_GAT || score > RGBMP_ATT_FA || (score == RGBMP_ATT_FA && H != 1) || !att_shape(H, C, &s))
+  if (!score_ok(score, sd) || (score == RGBMP_ATT_FA && H != 1) || !att_shape(H, C, &s))
     return fail(RGBMP_ERANGE, "%s: unsupported score %d / H %d / C %d (H == 1 with C <= 128, or C in {8..128} a power of two)",
                 fn, score, H, C);
-  if (!X || !a_nbr || !a_own || !out || !ws) return fail(RGBMP_EINVAL, "%s: null pointer", fn);
+  if (!X || (!sd && (!a_nbr || !a_own)) || !out || !ws) return fail(RGBMP_EINVAL, "%s: null pointer", fn);
   if (d && (!d->seed || (g->nnz > 0 && !d->eid))) return fail(RGBMP_EINVAL, "%s: dropout needs seed and eid", fn);
   const bool softmax = score != RGBMP_ATT_FA;
   if (softmax && (!rowmax || !rowsum)) return fail(RGBMP_EINVAL, "%s: rowmax / rowsum required", fn);
   if (!softmax && !dinv) return fail(RGBMP_EINVAL, "%s: FA needs dinv", fn);
   const bool train = out2 != nullptr;
-  if (train && score == RGBMP_ATT_MX) return fail(RGBMP_EINVAL, "%s: MX has no second aggregate", fn);
+  if (train && (score == RGBMP_ATT_MX || sd)) return fail(RGBMP_EINVAL, "%s: MX / SD have no second aggregate", fn);
   if (train && score == RGBMP_ATT_GAT && !rowq) return fail(RGBMP_EINVAL, "%s: rowq required with out2", fn);
   const int HC = H * C;
   const int64_t need_ld = (int64_t)align_up((size_t)HC, 4);
@@ -1141,7 +1201,7 @@ static int att_forward(const char* fn, const rgbmp_graph_t* g, int score, const 
   if (n == 0) return 0;
   AttParams p = {};
   fill_graph(p, g);
-  p.H = H; p.HT = s.HT; p.C = C; p.LPH = s.LPH; p.slope = slope;
+  p.H = H; p.HT = s.HT; p.C = C; p.LPH = s.LPH; p.slope = slope; p.logit_scale = logit_scale;
   Carver cv(ws, ws_bytes);
   float* an2 = cv.take<float>((size_t)g->n_cols * H);
   float* ao2 = cv.take<float>((size_t)n * H);
@@ -1149,6 +1209,7 @@ static int att_forward(const char* fn, const rgbmp_graph_t* g, int score, const 
   p.Xn = X; p.ldn = ldx; p.Xo = X; p.ldo_ = ldx; p.dinv = dinv; p.drop = drop;
   if (d) set_dropout(p, d, d->eid);
   p.out = out; p.ldo = ldo; p.out2 = out2; p.ldo2 = ldo2; p.rowmax = rowmax; p.rowsum = rowsum; p.rowq = rowq;
+  if (sd) return d ? launch_fwd<SC_SD, false, true>(p, s, st) : launch_fwd<SC_SD, false, false>(p, s, st);
   if (softmax) {                                           // log2-domain copies of the score terms
     att_scale_kernel<<<(unsigned)ceil_div(g->n_cols * H, 256), 256, 0, st>>>(a_nbr, g->n_cols * H, an2);
     att_scale_kernel<<<(unsigned)ceil_div(n * H, 256), 256, 0, st>>>(a_own, n * H, ao2);
@@ -1196,23 +1257,25 @@ static int att_backward(const char* fn, const rgbmp_graph_t* g, const rgbmp_grap
                         const float* drop, const int32_t* tpos, const rgbmp_dropout_t* d, const float* rowmax,
                         const float* rowsum, const float* rowq, const float* out, int64_t ldo, const float* out2,
                         int64_t ldo2, const float* dout, int64_t ldd, float* dX, int64_t lddx, float* dXf, int64_t lddxf,
-                        float* da_nbr, float* da_own, void* ws, size_t ws_bytes, int device, void* stream) {
+                        float* da_nbr, float* da_own, void* ws, size_t ws_bytes, int device, void* stream,
+                        bool sd = false, float logit_scale = 0.f) {
   int rc = check_g(g, fn);
   if (rc) return rc;
   rc = check_g(gT, fn);
   if (rc) return rc;
   Shape s;
-  if (score < RGBMP_ATT_GAT || score > RGBMP_ATT_FA || (score == RGBMP_ATT_FA && H != 1) || !att_shape(H, C, &s))
+  if (!score_ok(score, sd) || (score == RGBMP_ATT_FA && H != 1) || !att_shape(H, C, &s))
     return fail(RGBMP_ERANGE, "%s: unsupported score %d / H %d / C %d", fn, score, H, C);
-  if (!X || !a_nbr || !a_own || !dout || !dX || !da_nbr || !da_own || !ws || (drop && !tpos))
+  if (!X || !dout || !dX || (!sd && (!a_nbr || !a_own || !da_nbr || !da_own)) || !ws || (drop && !tpos))
     return fail(RGBMP_EINVAL, "%s: null pointer", fn);
-  if (d && (!d->seed || (gT->nnz > 0 && !d->eid_t) || (score == RGBMP_ATT_MX && g->nnz > 0 && !d->eid)))
-    return fail(RGBMP_EINVAL, "%s: dropout needs seed, eid_t (and eid for MX)", fn);
+  const bool logit = score == RGBMP_ATT_MX || sd;             // one pass per orientation
+  if (d && (!d->seed || (gT->nnz > 0 && !d->eid_t) || (logit && g->nnz > 0 && !d->eid)))
+    return fail(RGBMP_EINVAL, "%s: dropout needs seed, eid_t (and eid for MX / SD)", fn);
   const bool softmax = score != RGBMP_ATT_FA;
   if (softmax && (!rowmax || !rowsum || !out)) return fail(RGBMP_EINVAL, "%s: forward statistics required", fn);
-  if (score != RGBMP_ATT_MX && !out2) return fail(RGBMP_EINVAL, "%s: the training-mode forward's second aggregate is required", fn);
+  if (!logit && !out2) return fail(RGBMP_EINVAL, "%s: the training-mode forward's second aggregate is required", fn);
   if (score == RGBMP_ATT_GAT && !rowq) return fail(RGBMP_EINVAL, "%s: rowq required", fn);
-  if (score == RGBMP_ATT_MX && !dXf) return fail(RGBMP_EINVAL, "%s: MX needs the dXf scratch [n, ld]", fn);
+  if (logit && !dXf) return fail(RGBMP_EINVAL, "%s: MX / SD need the dXf scratch [n, ld]", fn);
   if (!softmax && !dinv) return fail(RGBMP_EINVAL, "%s: FA needs dinv", fn);
   if (!al16(X, ldx) || !al16(dout, ldd) || !al16(dX, lddx) || (dXf && !al16(dXf, lddxf)))
     return fail(RGBMP_EALIGN, "%s: X/dout/dX need 16-byte aligned rows", fn);
@@ -1229,7 +1292,7 @@ static int att_backward(const char* fn, const rgbmp_graph_t* g, const rgbmp_grap
   float* an2 = cv.take<float>((size_t)g->n_cols * H);
   AttParams pt = {};
   fill_graph(pt, gT);
-  pt.H = H; pt.HT = s.HT; pt.C = C; pt.LPH = s.LPH; pt.slope = slope;
+  pt.H = H; pt.HT = s.HT; pt.C = C; pt.LPH = s.LPH; pt.slope = slope; pt.logit_scale = logit_scale;
   if (!carve_split(pt, cv, HC, g->n_items > gT->n_items ? g->n_items : gT->n_items) || !cv.ok())
     return fail(RGBMP_EWORKSPACE, "%s: workspace carve", fn);
   const unsigned prep_grid = (unsigned)ceil_div(n_dst * H, 256);
@@ -1237,6 +1300,8 @@ static int att_backward(const char* fn, const rgbmp_graph_t* g, const rgbmp_grap
     att_bwd_prep_kernel<SC_GAT><<<prep_grid, 256, 0, st>>>(dout, ldd, out, ldo, out2, ldo2, a_own, rowmax, rowsum, rowq, dinv, n_dst, H, C, stats, da_own);
   else if (score == RGBMP_ATT_MX)
     att_bwd_prep_kernel<SC_MX><<<prep_grid, 256, 0, st>>>(dout, ldd, out, ldo, out2, ldo2, a_own, rowmax, rowsum, rowq, dinv, n_dst, H, C, stats, da_own);
+  else if (sd)
+    att_bwd_prep_kernel<SC_SD><<<prep_grid, 256, 0, st>>>(dout, ldd, out, ldo, out2, ldo2, nullptr, rowmax, rowsum, rowq, dinv, n_dst, H, C, stats, nullptr);
   else
     att_bwd_prep_kernel<SC_FA><<<prep_grid, 256, 0, st>>>(dout, ldd, out, ldo, out2, ldo2, a_own, rowmax, rowsum, rowq, dinv, n_dst, H, C, stats, da_own);
   RGBMP_LAUNCH_CHECK("att_bwd_prep_kernel");
@@ -1249,10 +1314,26 @@ static int att_backward(const char* fn, const rgbmp_graph_t* g, const rgbmp_grap
     pf.Xn = X; pf.ldn = ldx; pf.sn = an2; pf.stats = stats; pf.Xo = X; pf.ldo_ = ldx; pf.Do = dout; pf.lddo = ldd;
     pf.drop = drop; pf.out = dXf; pf.ldo = lddxf; pf.ds = da_own;
     if (d) set_dropout(pf, d, d->eid);
-    rc = d ? launch_bwdF<true>(pf, s, st) : launch_bwdF<false>(pf, s, st);
+    rc = d ? launch_bwdF<SC_MX, true>(pf, s, st) : launch_bwdF<SC_MX, false>(pf, s, st);
     if (rc) return rc;
     pt.acc_in = dXf; pt.ld_acc = lddxf;
     pt.Xn2 = X; pt.ldn2 = ldx;
+  }
+  if (sd) {
+    // SD has no score scalars, but the passes (att_bwd_combine_kernel among them) write a per-row ds: the zeros land
+    // in the slot of the scaled a_nbr copy, n_cols * H floats, which covers the rows of both orientations because
+    // check_sd admits square graphs only
+    AttParams pf = pt;
+    fill_graph(pf, g);
+    pf.Xn = X; pf.ldn = ldx; pf.stats = stats; pf.Xo = X; pf.ldo_ = ldx; pf.Do = dout; pf.lddo = ldd;
+    pf.drop = drop; pf.out = dXf; pf.ldo = lddxf; pf.ds = an2;
+    if (d) set_dropout(pf, d, d->eid);
+    rc = d ? launch_bwdF<SC_SD, true>(pf, s, st) : launch_bwdF<SC_SD, false>(pf, s, st);
+    if (rc) return rc;
+    pt.Xn = dout; pt.ldn = ldd; pt.stats = stats; pt.Xo = X; pt.ldo_ = ldx; pt.Xn2 = X; pt.ldn2 = ldx;
+    pt.drop = drop; pt.tpos = tpos; pt.out = dX; pt.ldo = lddx; pt.ds = an2; pt.acc_in = dXf; pt.ld_acc = lddxf;
+    if (d) set_dropout(pt, d, d->eid_t);
+    return d ? launch_bwdT<SC_SD, true>(pt, s, st) : launch_bwdT<SC_SD, false>(pt, s, st);
   }
   // pass T on the transpose CSR: dX_j, da_src[j]
   pt.Xn = dout; pt.ldn = ldd; pt.stats = stats; pt.dinv = dinv; pt.Xo = X; pt.ldo_ = ldx; pt.so = a_nbr;
@@ -1289,6 +1370,31 @@ int rgbmp_att_backward_dropout(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, 
   return att_backward("rgbmp_att_backward_dropout", g, gT, score, X, ldx, a_nbr, a_own, dinv, H, C, slope, nullptr,
                       nullptr, d, rowmax, rowsum, rowq, out, ldo, out2, ldo2, dout, ldd, dX, lddx, dXf, lddxf, da_nbr,
                       da_own, ws, ws_bytes, device, stream);
+}
+
+int rgbmp_att_sd_forward(const rgbmp_graph_t* g, const float* X, int64_t ldx, int H, int C, float logit_scale,
+                         float slope, const float* drop, const rgbmp_dropout_t* d, float* out, int64_t ldo,
+                         float* rowmax, float* rowsum, void* ws, size_t ws_bytes, int device, void* stream) {
+  const char* fn = "rgbmp_att_sd_forward";
+  int rc = check_sd(g, nullptr, H, C, logit_scale, drop, d, fn);
+  if (rc) return rc;
+  return att_forward(fn, g, RGBMP_ATT_SD, X, ldx, nullptr, nullptr, nullptr, H, C, slope, drop, d, out, ldo, rowmax,
+                     rowsum, nullptr, 0, nullptr, ws, ws_bytes, device, stream, true, logit_scale);
+}
+
+int rgbmp_att_sd_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, const float* X, int64_t ldx, int H, int C,
+                          float logit_scale, float slope, const float* drop, const int32_t* tpos,
+                          const rgbmp_dropout_t* d, const float* rowmax, const float* rowsum,
+                          const float* out, int64_t ldo, const float* dout, int64_t ldd,
+                          float* dX, int64_t lddx, float* dXf, int64_t lddxf,
+                          void* ws, size_t ws_bytes, int device, void* stream) {
+  const char* fn = "rgbmp_att_sd_backward";
+  if (!gT) return fail(RGBMP_EINVAL, "%s: null pointer", fn);
+  int rc = check_sd(g, gT, H, C, logit_scale, drop, d, fn);
+  if (rc) return rc;
+  return att_backward(fn, g, gT, RGBMP_ATT_SD, X, ldx, nullptr, nullptr, nullptr, H, C, slope, drop, tpos, d, rowmax,
+                      rowsum, nullptr, out, ldo, nullptr, 0, dout, ldd, dX, lddx, dXf, lddxf, nullptr, nullptr, ws,
+                      ws_bytes, device, stream, true, logit_scale);
 }
 
 int rgbmp_dropout_mask(const rgbmp_dropout_t* d, int64_t nnz, int H, float* out, int device, void* stream) {

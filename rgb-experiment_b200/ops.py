@@ -529,7 +529,7 @@ def spmm_heads(w, X, graph, H, Cc):
     return _SpmmHeads.apply(w, X, graph, H, Cc)
 
 
-ATT_GAT, ATT_MX, ATT_FA = 0, 1, 2
+ATT_GAT, ATT_MX, ATT_FA, ATT_SD = 0, 1, 2, 3
 
 
 def _head_pad(H: int, Cc: int) -> int:
@@ -565,19 +565,24 @@ def _rows_zero_padded(x: torch.Tensor) -> Tuple[torch.Tensor, int]:
 
 class _Att(torch.autograd.Function):
     """Fused edge-score attention + aggregate (csrc/att.cu): GATConv (A10/A11; gat.py:18-21), SuperGATConv-MX
-    (A12; supergat.py:15-21) and FAConv (A13; fagcn.py:15,31).  Nothing edge-sized is allocated: the forward saves
+    (A12; supergat.py:15-21), SuperGATConv-SD (A12; no score scalars: a_nbr = a_own = None, the logit <x_i, x_j>
+    scaled by logit_scale) and FAConv (A13; fagcn.py:15,31).  Nothing edge-sized is allocated: the forward saves
     per-node statistics (max, sum and -- in training mode -- the second aggregate that yields the gradient of the
     target-side score term), the backward recomputes the edge weights.  Deterministic (no atomics).
     Attention dropout: either an explicit mask in forward-CSR order (drop_csr) or a device seed tensor (seed, rate p)
     from which forward and backward regenerate the same multipliers inside the kernels -- still nothing edge-sized."""
 
     @staticmethod
-    def forward(ctx, x, a_nbr, a_own, graph: Graph, score: int, H: int, Cc: int, slope: float, drop_csr, seed, p):
+    def forward(ctx, x, a_nbr, a_own, graph: Graph, score: int, H: int, Cc: int, slope: float, drop_csr, seed, p,
+                logit_scale: float):
         _lib.require_cuda(x, "x")
         for t, nm in ((x, "x"), (a_nbr, "a_nbr"), (a_own, "a_own")):
-            _lib.require_f32(t, f"fused attention {nm}")
+            if t is not None:
+                _lib.require_f32(t, f"fused attention {nm}")
         xb, ldx = _rows_zero_padded(x)
-        a_n, a_o = a_nbr.contiguous().view(-1, H), a_own.contiguous().view(-1, H)
+        a_n = a_o = None
+        if score != ATT_SD:
+            a_n, a_o = a_nbr.contiguous().view(-1, H), a_own.contiguous().view(-1, H)
         N, dev = graph.N, x.device
         train = any(ctx.needs_input_grad[:3])
         out, ldo = alloc_rows(N, H * Cc, torch.float32, dev)
@@ -588,14 +593,19 @@ class _Att(torch.autograd.Function):
             rsum = torch.empty((N, H), dtype=torch.float32, device=dev)
         else:
             dinv = graph.dinv()
-        if train and score != ATT_MX:
+        if train and score in (ATT_GAT, ATT_FA):
             out2, ldo2 = alloc_rows(N, H * Cc, torch.float32, dev)
             if score == ATT_GAT:
                 rowq = torch.empty((N, H), dtype=torch.float32, device=dev)
         L = lib()
         wsb = L.rgbmp_att_forward_workspace_bytes(graph.fwd.ref, H, Cc)
         ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
-        if seed is None:
+        if score == ATT_SD:
+            d = None if seed is None else C.byref(_dropout_struct(p, seed, graph))
+            check(L.rgbmp_att_sd_forward(graph.fwd.ref, ptr(xb), ldx, H, Cc, logit_scale, slope, ptr(drop_csr), d,
+                                         ptr(out), ldo, ptr(rmax), ptr(rsum), ptr(ws), wsb, dev.index, stream_of(dev)),
+                  "att_sd_forward")
+        elif seed is None:
             check(L.rgbmp_att_forward(graph.fwd.ref, score, ptr(xb), ldx, ptr(a_n), ptr(a_o), ptr(dinv), H, Cc, slope,
                                       ptr(drop_csr), ptr(out), ldo, ptr(rmax), ptr(rsum), ptr(out2), ldo2, ptr(rowq),
                                       ptr(ws), wsb, dev.index, stream_of(dev)), "att_forward")
@@ -604,7 +614,7 @@ class _Att(torch.autograd.Function):
             check(L.rgbmp_att_forward_dropout(graph.fwd.ref, score, ptr(xb), ldx, ptr(a_n), ptr(a_o), ptr(dinv), H, Cc,
                                               slope, C.byref(d), ptr(out), ldo, ptr(rmax), ptr(rsum), ptr(out2), ldo2,
                                               ptr(rowq), ptr(ws), wsb, dev.index, stream_of(dev)), "att_forward_dropout")
-        ctx.graph, ctx.score, ctx.H, ctx.Cc, ctx.slope, ctx.p = graph, score, H, Cc, slope, p
+        ctx.graph, ctx.score, ctx.H, ctx.Cc, ctx.slope, ctx.p, ctx.logit_scale = graph, score, H, Cc, slope, p, logit_scale
         ctx.save_for_backward(xb, a_n, a_o, rmax, rsum, rowq, out, out2, drop_csr, seed)
         return out
 
@@ -615,14 +625,21 @@ class _Att(torch.autograd.Function):
         dev, N = dout.device, g.N
         db, ldd = _rows_zero_padded(dout)
         dx, lddx = alloc_rows(N, H * Cc, torch.float32, dev)
-        dxf, lddxf = (alloc_rows(N, H * Cc, torch.float32, dev) if score == ATT_MX else (None, 0))
-        da_n = torch.empty((N, H), dtype=torch.float32, device=dev)
-        da_o = torch.empty((N, H), dtype=torch.float32, device=dev)
+        dxf, lddxf = (alloc_rows(N, H * Cc, torch.float32, dev) if score in (ATT_MX, ATT_SD) else (None, 0))
         tpos = g.tpos() if drop is not None else None
         dinv = g.dinv() if score == ATT_FA else None
         L = lib()
         wsb = L.rgbmp_att_backward_workspace_bytes(g.fwd.ref, g.bwd.ref, H, Cc)
         ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
+        if score == ATT_SD:
+            d = None if seed is None else C.byref(_dropout_struct(ctx.p, seed, g, backward=True))
+            check(L.rgbmp_att_sd_backward(g.fwd.ref, g.bwd.ref, ptr(xb), xb.stride(0), H, Cc, ctx.logit_scale, ctx.slope,
+                                          ptr(drop), ptr(tpos), d, ptr(rmax), ptr(rsum), ptr(out), out.stride(0), ptr(db),
+                                          ldd, ptr(dx), lddx, ptr(dxf), lddxf, ptr(ws), wsb, dev.index, stream_of(dev)),
+                  "att_sd_backward")
+            return dx, None, None, None, None, None, None, None, None, None, None, None
+        da_n = torch.empty((N, H), dtype=torch.float32, device=dev)
+        da_o = torch.empty((N, H), dtype=torch.float32, device=dev)
         ld2 = 0 if out2 is None else out2.stride(0)
         if seed is None:
             check(L.rgbmp_att_backward(g.fwd.ref, g.bwd.ref, score, ptr(xb), xb.stride(0), ptr(a_n), ptr(a_o), ptr(dinv), H,
@@ -636,22 +653,25 @@ class _Att(torch.autograd.Function):
                                                ptr(out), out.stride(0), ptr(out2), ld2, ptr(db), ldd, ptr(dx), lddx,
                                                ptr(dxf), lddxf, ptr(da_n), ptr(da_o), ptr(ws), wsb, dev.index,
                                                stream_of(dev)), "att_backward_dropout")
-        return dx, da_n, da_o, None, None, None, None, None, None, None, None
+        return dx, da_n, da_o, None, None, None, None, None, None, None, None, None
 
 
 def _att(score: int, name: str, x, a_nbr, a_own, graph: Graph, H: int, Cc: int, slope: float, drop_edge,
          dropout_p: float = 0.0, seed: Optional[torch.Tensor] = None):
     """Pads heads to the kernel's channel count (torch ops on node-sized tensors, autograd-transparent), memoises
-    the no-grad call, applies the fused op.  seed: fused dropout at rate dropout_p (see dropout_mask)."""
+    the no-grad call, applies the fused op.  seed: fused dropout at rate dropout_p (see dropout_mask).  SD scales
+    its logit by 1/sqrt(Cc) of the unpadded head width."""
     Cp = _head_pad(H, Cc)
     N = x.size(0)
     xk = x if Cp == Cc else torch.nn.functional.pad(x.view(N, H, Cc), (0, Cp - Cc)).reshape(N, H * Cp)
     drop_csr = None if drop_edge is None else graph.to_csr_order(drop_edge)
+    ls = 1.0 / math.sqrt(Cc) if score == ATT_SD else 0.0
     if drop_csr is None and seed is None:
-        out = memo.cached(graph, (name, H, Cc, float(slope)), (xk, a_nbr, a_own), _work(graph, xk),
-                          lambda: _Att.apply(xk, a_nbr, a_own, graph, score, H, Cp, float(slope), None, None, 0.0))
+        ins = tuple(t for t in (xk, a_nbr, a_own) if t is not None)
+        out = memo.cached(graph, (name, H, Cc, float(slope)), ins, _work(graph, xk),
+                          lambda: _Att.apply(xk, a_nbr, a_own, graph, score, H, Cp, float(slope), None, None, 0.0, ls))
     else:
-        out = _Att.apply(xk, a_nbr, a_own, graph, score, H, Cp, float(slope), drop_csr, seed, float(dropout_p))
+        out = _Att.apply(xk, a_nbr, a_own, graph, score, H, Cp, float(slope), drop_csr, seed, float(dropout_p), ls)
     return out if Cp == Cc else out.view(N, H, Cp)[:, :, :Cc].reshape(N, H * Cc)
 
 
@@ -728,6 +748,23 @@ def supergat_mx(xp, a_l, a_r, graph: Graph, H: int, Cc: int, slope: float = 0.2,
         drop_edge = dropout_mask(graph, H, dropout_p, seed)
     logits = edge_sddmm(xp, xp, graph, H, Cc)
     alpha = torch.nn.functional.leaky_relu(edge_u_add_v(a_l, a_r, graph) * logits.sigmoid(), slope)
+    alpha = edge_softmax(alpha, graph)
+    if drop_edge is not None:
+        alpha = alpha * graph.to_csr_order(drop_edge)
+    return spmm_heads(alpha, xp, graph, H, Cc)
+
+
+def supergat_sd(xp, graph: Graph, H: int, Cc: int, slope: float = 0.2, drop_edge: Optional[torch.Tensor] = None,
+                dropout_p: float = 0.0, generator: Optional[torch.Generator] = None):
+    """SuperGATConv SD attention + aggregate (A12): alpha = softmax(leaky_relu(<x_i, x_j> / sqrt(Cc))) per head.
+    xp [N,H*C] float32 -> [N,H*C].  drop_edge / dropout_p / generator as in gat."""
+    _lib.require_f32(xp, "supergat_sd xp")
+    seed = _draw_dropout(graph, drop_edge, dropout_p, generator)
+    if att_fusable(ATT_SD, H, Cc):
+        return _att(ATT_SD, "supergat_sd", xp, None, None, graph, H, Cc, slope, drop_edge, dropout_p, seed)
+    if seed is not None:
+        drop_edge = dropout_mask(graph, H, dropout_p, seed)
+    alpha = torch.nn.functional.leaky_relu(edge_sddmm(xp, xp, graph, H, Cc) / math.sqrt(Cc), slope)
     alpha = edge_softmax(alpha, graph)
     if drop_edge is not None:
         alpha = alpha * graph.to_csr_order(drop_edge)

@@ -224,9 +224,9 @@ class GATConv(MessagePassing):
 
 
 class SuperGATConv(MessagePassing):
-    """A12, MX attention (models/supergat.py:15-21,26,29): scores, edge softmax and aggregate in ONE fused
-    kernel pass (ops.supergat_mx, csrc/att.cu; backward = one pass per orientation, nothing edge-sized is
-    allocated).  Edge sampling and the BCE loss on the sampled pairs stay PyTorch (node-pair sized) unless
+    """A12, MX and SD attention (models/supergat.py:15-21,26,29): scores, edge softmax and aggregate in ONE fused
+    kernel pass (ops.supergat_mx / ops.supergat_sd, csrc/att.cu; backward = one pass per orientation, nothing
+    edge-sized is allocated).  Edge sampling and the BCE loss on the sampled pairs stay PyTorch (node-pair sized) unless
     ops.FUSED_SUPERGAT_LOSS: then both run on the device (ops.supergat_att_loss) and nothing edge-sized is allocated."""
 
     def __init__(self, in_channels, out_channels, heads=1, concat=True, negative_slope=0.2, dropout=0.0,
@@ -292,14 +292,8 @@ class SuperGATConv(MessagePassing):
             a_l = (x3 * self.att_l).sum(-1)
             a_r = (x3 * self.att_r).sum(-1)
             out = ops.supergat_mx(xp, a_l, a_r, g, H, C, self.negative_slope, keep, dropout_p=p)      # one fused pass
-        else:                                                         # SD attention: not used by the reference
-            if p > 0:                                                 # the mask the seed stands for, edge order
-                keep = ops.dropout_mask(g, H, p, ops.dropout_seed(x.device))
-            alpha = F.leaky_relu(ops.edge_sddmm(xp, xp, g, H, C) / math.sqrt(C), self.negative_slope)
-            alpha = ops.edge_softmax(alpha, g)
-            if keep is not None:
-                alpha = alpha * g.to_csr_order(keep)
-            out = ops.spmm_heads(alpha, xp, g, H, C)
+        else:                                                         # SD attention (the reference's models use MX)
+            out = ops.supergat_sd(xp, g, H, C, self.negative_slope, keep, dropout_p=p)                # one fused pass
         if self.training and ops.FUSED_SUPERGAT_LOSS:                # sampling and BCE on the device
             scale = 1.0 / H if self.attention_type == "MX" else 1.0 / (H * math.sqrt(C))     # att_x.mean(-1)
             self._att_loss = ops.supergat_att_loss(xp, g, H, C, scale, self.edge_sample_ratio, self.neg_sample_ratio,
