@@ -35,7 +35,7 @@ extern "C" {
 #pragma GCC visibility push(default)   /* the library is built with -fvisibility=hidden */
 #endif
 
-#define RGBMP_VERSION 100
+#define RGBMP_VERSION 101
 
 /* argument errors */
 #define RGBMP_EINVAL   (-1)  /* null pointer / bad enum / negative size */
@@ -313,43 +313,35 @@ int rgbmp_peer_close(void* ptr, int device);
  *                  e = leaky_relu((a_nbr[j] + a_own[i]) * sigmoid(<X[i,h,:], X[j,h,:]>)), then as GAT
  *   RGBMP_ATT_FA   FAConv (fagcn.py:15,31; A13), H = 1:
  *                  out[i] = sum tanh(a_nbr[j] + a_own[i]) * dinv[j]*dinv[i] * mask * X[j]        (no softmax)
- *   RGBMP_ATT_SD   SuperGATConv, SD attention (A12), through rgbmp_att_sd_forward / _backward only:
+ *   RGBMP_ATT_SD   SuperGATConv, SD attention (A12):
  *                  e = leaky_relu(logit_scale * <X[i,h,:], X[j,h,:]>), then as GAT
  * X [n_cols, H*C] (ldx), a_nbr [n_cols,H] (a_src / att_l side), a_own [n_rows,H] (a_dst / att_r side).
  * Shapes: H == 1 with any C <= 128 (padding columns of X up to roundup(C,4) must be ZERO), or C a power of two in
  * 8..128 with any H (heads are tiled over the grid) -- rgbmp_att_supported() says which; the host layer pads heads.
- * drop (optional, forward-CSR order [nnz,H]) is the attention-dropout keep-mask already divided by (1-p).
+ * What each score reads:
+ *   GAT, MX  a_nbr, a_own (the backward writes da_nbr, da_own);
+ *   FA       a_nbr, a_own and dinv [n]; H == 1;
+ *   SD       no a_*, dinv or da_* (pass NULL); g square (X holds both endpoints), gT its transpose, logit_scale
+ *            finite -- 1/sqrt(C) of the UNPADDED head width when the caller pads heads to a supported C.
+ *            logit_scale is ignored by the other scores.
+ * Attention dropout: at most one of `drop` and `d` may be non-NULL.  drop is the explicit keep-mask in forward-CSR
+ * order [nnz,H], already divided by (1-p); the backward also needs tpos[k'] = forward-CSR position of transpose entry
+ * k'.  d generates the mask inside the kernels (rgbmp_dropout_t below): the forward reads d->eid, the backward
+ * d->eid_t (MX and SD also d->eid) and streams eid_t in its transpose pass -- no tpos, no random gather.
  * Softmax scores save rowmax,rowsum [n_rows,H].  TRAINING mode = out2 != NULL: GAT and FA accumulate a second
  * aggregate next to out (GAT: P_i = sum alpha*leaky'*mask*X[j] into out2 and q_i = sum alpha*leaky' into rowq;
  * FA: Q_i = sum (1-tanh^2)*dinv*dinv*mask*X[j]) from which the backward gets the gradient of the per-TARGET score
- * term without atomics (da_own[i] = <dout_i, P_i> - S_i q_i); MX needs none (out2 must be NULL).
- * Nothing edge-sized is written; the result is deterministic. */
+ * term without atomics (da_own[i] = <dout_i, P_i> - S_i q_i); MX and SD need none (out2 must be NULL).
+ * The backward: g = the forward CSR, gT = its transpose (rows = sources j).  It recomputes the edge weights from the
+ * saved per-target statistics; `out`/`out2`/`rowq` are the training-mode forward's results.  It writes dX [n, H*C]
+ * (lddx) and, but for SD, da_nbr [n_cols,H], da_own [n_rows,H].  MX and SD run one pass per orientation (the logit
+ * <x_i,x_j> feeds both endpoints) and need the scratch dXf [n_rows, lddxf]; GAT and FA run one transpose pass.
+ * An unsupported score / H / C is RGBMP_ERANGE; a NULL pointer a score reads, both dropout forms or a graph SD
+ * cannot take is RGBMP_EINVAL.  Nothing edge-sized is written; the result is deterministic. */
 #define RGBMP_ATT_GAT 0
 #define RGBMP_ATT_MX  1
 #define RGBMP_ATT_FA  2
 #define RGBMP_ATT_SD  3
-int rgbmp_att_supported(int score, int H, int C);
-size_t rgbmp_att_forward_workspace_bytes(const rgbmp_graph_t* g, int H, int C);
-int rgbmp_att_forward(const rgbmp_graph_t* g, int score, const float* X, int64_t ldx,
-                      const float* a_nbr, const float* a_own, const float* dinv, int H, int C, float slope,
-                      const float* drop, float* out, int64_t ldo, float* rowmax, float* rowsum,
-                      float* out2, int64_t ldo2, float* rowq,
-                      void* ws, size_t ws_bytes, int device, void* stream);
-
-/* Backward of rgbmp_att_forward.  g = the forward CSR, gT = its transpose (rows = sources j).  Recomputes the
- * edge weights from the saved per-target statistics; `out`/`out2`/`rowq` are the training-mode forward's results.
- * Writes dX [n, H*C] (lddx), da_nbr [n_cols,H], da_own [n_rows,H].  MX runs one pass per orientation (the logit
- * <x_i,x_j> feeds both endpoints) and needs the scratch dXf [n_rows, lddxf]; GAT and FA run one transpose pass.
- * tpos[k'] = forward-CSR position of transpose entry k' (only read when drop != NULL). */
-size_t rgbmp_att_backward_workspace_bytes(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int H, int C);
-int rgbmp_att_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int score, const float* X, int64_t ldx,
-                       const float* a_nbr, const float* a_own, const float* dinv, int H, int C, float slope,
-                       const float* drop, const int32_t* tpos,
-                       const float* rowmax, const float* rowsum, const float* rowq,
-                       const float* out, int64_t ldo, const float* out2, int64_t ldo2,
-                       const float* dout, int64_t ldd,
-                       float* dX, int64_t lddx, float* dXf, int64_t lddxf, float* da_nbr, float* da_own,
-                       void* ws, size_t ws_bytes, int device, void* stream);
 
 /* Attention dropout generated inside the kernels (csrc/philox.cuh): no mask tensor exists.  For edge e (its id in
  * the edited edge list) and head h (FA: h = 0):
@@ -366,39 +358,21 @@ typedef struct rgbmp_dropout {
   float    scale;
 } rgbmp_dropout_t;
 
-/* = rgbmp_att_forward with the dropout descriptor in place of `drop` (d->eid required). */
-int rgbmp_att_forward_dropout(const rgbmp_graph_t* g, int score, const float* X, int64_t ldx,
-                              const float* a_nbr, const float* a_own, const float* dinv, int H, int C, float slope,
-                              const rgbmp_dropout_t* d, float* out, int64_t ldo, float* rowmax, float* rowsum,
-                              float* out2, int64_t ldo2, float* rowq,
-                              void* ws, size_t ws_bytes, int device, void* stream);
-/* = rgbmp_att_backward with the dropout descriptor in place of `drop, tpos` (d->eid_t required; MX also d->eid).
- * The transpose pass streams eid_t: no tpos, no random gather. */
-int rgbmp_att_backward_dropout(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int score, const float* X, int64_t ldx,
-                               const float* a_nbr, const float* a_own, const float* dinv, int H, int C, float slope,
-                               const rgbmp_dropout_t* d,
-                               const float* rowmax, const float* rowsum, const float* rowq,
-                               const float* out, int64_t ldo, const float* out2, int64_t ldo2,
-                               const float* dout, int64_t ldd,
-                               float* dX, int64_t lddx, float* dXf, int64_t lddxf, float* da_nbr, float* da_own,
-                               void* ws, size_t ws_bytes, int device, void* stream);
-/* SuperGATConv's SD attention: the RGBMP_ATT_SD score with no score scalars.  g must be square (X holds both
- * endpoints), gT its transpose.  logit_scale is 1/sqrt(C) of the UNPADDED head width when the caller pads heads to a
- * supported C.  At most one of `drop` (explicit mask, forward-CSR order; the backward also needs tpos) and `d`
- * (dropout generated in the kernels; d->eid, and d->eid_t in the backward) may be non-NULL.  Workspaces: the
- * rgbmp_att_forward / backward_workspace_bytes queries.  The forward saves rowmax, rowsum [n,H]; the backward runs
- * one pass per orientation like MX (dXf = scratch [n, lddxf]) and writes dX.  Unsupported H / C, NULL pointers,
- * both dropout forms or a non-square graph: RGBMP_EINVAL.  rgbmp_att_forward / backward(_dropout) do not take
- * score 3. */
-int rgbmp_att_sd_forward(const rgbmp_graph_t* g, const float* X, int64_t ldx, int H, int C, float logit_scale,
-                         float slope, const float* drop, const rgbmp_dropout_t* d, float* out, int64_t ldo,
-                         float* rowmax, float* rowsum, void* ws, size_t ws_bytes, int device, void* stream);
-int rgbmp_att_sd_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, const float* X, int64_t ldx, int H, int C,
-                          float logit_scale, float slope, const float* drop, const int32_t* tpos,
-                          const rgbmp_dropout_t* d, const float* rowmax, const float* rowsum,
-                          const float* out, int64_t ldo, const float* dout, int64_t ldd,
-                          float* dX, int64_t lddx, float* dXf, int64_t lddxf,
-                          void* ws, size_t ws_bytes, int device, void* stream);
+int rgbmp_att_supported(int score, int H, int C);
+size_t rgbmp_att_forward_workspace_bytes(const rgbmp_graph_t* g, int H, int C);
+int rgbmp_att_forward(const rgbmp_graph_t* g, int score, const float* X, int64_t ldx,
+                      const float* a_nbr, const float* a_own, const float* dinv, int H, int C,
+                      float slope, float logit_scale, const float* drop, const rgbmp_dropout_t* d,
+                      float* out, int64_t ldo, float* rowmax, float* rowsum, float* out2, int64_t ldo2, float* rowq,
+                      void* ws, size_t ws_bytes, int device, void* stream);
+size_t rgbmp_att_backward_workspace_bytes(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int H, int C);
+int rgbmp_att_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int score, const float* X, int64_t ldx,
+                       const float* a_nbr, const float* a_own, const float* dinv, int H, int C,
+                       float slope, float logit_scale, const float* drop, const int32_t* tpos, const rgbmp_dropout_t* d,
+                       const float* rowmax, const float* rowsum, const float* rowq,
+                       const float* out, int64_t ldo, const float* out2, int64_t ldo2, const float* dout, int64_t ldd,
+                       float* dX, int64_t lddx, float* dXf, int64_t lddxf, float* da_nbr, float* da_own,
+                       void* ws, size_t ws_bytes, int device, void* stream);
 /* out[e*H + h] = the multiplier of edge e, head h, in EDGE order [nnz, H] (the mask of the unfused paths). */
 int rgbmp_dropout_mask(const rgbmp_dropout_t* d, int64_t nnz, int H, float* out, int device, void* stream);
 

@@ -95,22 +95,13 @@ def lib():
     optional = {
         "rgbmp_att_supported": (C.c_int, [C.c_int, C.c_int, C.c_int]),
         "rgbmp_att_forward_workspace_bytes": (c_sz, [GP, C.c_int, C.c_int]),
-        "rgbmp_att_forward": (C.c_int, [GP, C.c_int, c_vp, c_i64, c_vp, c_vp, c_vp, C.c_int, C.c_int, c_f32, c_vp, c_vp, c_i64,
-                                        c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_sz, C.c_int, c_vp]),
+        "rgbmp_att_forward": (C.c_int, [GP, C.c_int, c_vp, c_i64, c_vp, c_vp, c_vp, C.c_int, C.c_int, c_f32, c_f32, c_vp, DP,
+                                        c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_sz, C.c_int, c_vp]),
         "rgbmp_att_backward_workspace_bytes": (c_sz, [GP, GP, C.c_int, C.c_int]),
-        "rgbmp_att_backward": (C.c_int, [GP, GP, C.c_int, c_vp, c_i64, c_vp, c_vp, c_vp, C.c_int, C.c_int, c_f32, c_vp, c_vp,
-                                         c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64,
-                                         c_vp, c_vp, c_vp, c_sz, C.c_int, c_vp]),
-        "rgbmp_att_forward_dropout": (C.c_int, [GP, C.c_int, c_vp, c_i64, c_vp, c_vp, c_vp, C.c_int, C.c_int, c_f32, DP, c_vp,
-                                                c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_sz, C.c_int, c_vp]),
-        "rgbmp_att_backward_dropout": (C.c_int, [GP, GP, C.c_int, c_vp, c_i64, c_vp, c_vp, c_vp, C.c_int, C.c_int, c_f32, DP,
-                                                 c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp,
-                                                 c_i64, c_vp, c_vp, c_vp, c_sz, C.c_int, c_vp]),
+        "rgbmp_att_backward": (C.c_int, [GP, GP, C.c_int, c_vp, c_i64, c_vp, c_vp, c_vp, C.c_int, C.c_int, c_f32, c_f32, c_vp,
+                                         c_vp, DP, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp,
+                                         c_i64, c_vp, c_vp, c_vp, c_sz, C.c_int, c_vp]),
         "rgbmp_dropout_mask": (C.c_int, [DP, c_i64, C.c_int, c_vp, C.c_int, c_vp]),
-        "rgbmp_att_sd_forward": (C.c_int, [GP, c_vp, c_i64, C.c_int, C.c_int, c_f32, c_f32, c_vp, DP, c_vp, c_i64, c_vp, c_vp,
-                                           c_vp, c_sz, C.c_int, c_vp]),
-        "rgbmp_att_sd_backward": (C.c_int, [GP, GP, c_vp, c_i64, C.c_int, C.c_int, c_f32, c_f32, c_vp, c_vp, DP, c_vp, c_vp,
-                                            c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_sz, C.c_int, c_vp]),
         "rgbmp_sgat_negative_sampling_workspace_bytes": (c_sz, [c_i64]),
         "rgbmp_sgat_negative_sampling": (C.c_int, [c_vp, c_vp, c_i64, SP, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_sz, C.c_int,
                                                    c_vp]),
@@ -143,7 +134,7 @@ def lib():
     for name, (res, args) in optional.items():
         fn = getattr(L, name)
         fn.restype, fn.argtypes = res, args
-    if L.rgbmp_version() != 100:
+    if L.rgbmp_version() != 101:
         raise RuntimeError("librgbmp.so version mismatch")
     _lib = L
     return L

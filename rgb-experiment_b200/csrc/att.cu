@@ -31,6 +31,7 @@
 //   SD:   MX without the score scalars and the sigmoid gate: the same two passes, no da_l / da_r.
 #include <math.h>
 #include <stdlib.h>
+#include <type_traits>
 #include "common.cuh"
 #include "philox.cuh"
 
@@ -1119,6 +1120,25 @@ static int launch_bwdF(const AttParams& p, const Shape& s, cudaStream_t st) {
   return 0;
 }
 
+// the scores and shapes the kernels take; FA is single-head
+static bool att_ok(int score, int H, int C, Shape* s) {
+  return score >= RGBMP_ATT_GAT && score <= RGBMP_ATT_SD && (score != RGBMP_ATT_FA || H == 1) && att_shape(H, C, s);
+}
+
+// Calls f(SC, DR) -- the score as a std::integral_constant, "fused dropout" as a std::bool_constant -- for a score
+// att_ok admitted: the one place run-time arguments become kernel template arguments.  f guards with if constexpr
+// what a score has no kernels for (MX / SD: a training-mode forward; GAT / FA: the backward's pass F).
+template <class F>
+static int with_kernel(int score, bool dr, F&& f) {
+  const auto run = [&](auto sc) { return dr ? f(sc, std::true_type()) : f(sc, std::false_type()); };
+  switch (score) {
+    case RGBMP_ATT_GAT: return run(std::integral_constant<int, SC_GAT>());
+    case RGBMP_ATT_MX: return run(std::integral_constant<int, SC_MX>());
+    case RGBMP_ATT_FA: return run(std::integral_constant<int, SC_FA>());
+    default: return run(std::integral_constant<int, SC_SD>());
+  }
+}
+
 }  // namespace rgbmp
 
 using namespace rgbmp;
@@ -1127,9 +1147,7 @@ extern "C" {
 
 int rgbmp_att_supported(int score, int H, int C) {
   Shape s;
-  if (score < RGBMP_ATT_GAT || score > RGBMP_ATT_SD) return 0;
-  if (score == RGBMP_ATT_FA && H != 1) return 0;
-  return att_shape(H, C, &s) ? 1 : 0;
+  return att_ok(score, H, C, &s) ? 1 : 0;
 }
 
 size_t rgbmp_att_forward_workspace_bytes(const rgbmp_graph_t* g, int H, int C) {
@@ -1145,41 +1163,22 @@ static void set_dropout(AttParams& p, const rgbmp_dropout_t* d, const int32_t* e
   p.dscale = d->scale;
 }
 
-// The generic entry points take GAT / MX / FA (sd == false: score 3 stays unsupported there); SD comes through
-// rgbmp_att_sd_* only (sd == true, score == RGBMP_ATT_SD), which check its arguments first.  SD reads no score
-// scalars (a_nbr / a_own NULL) and scales the logit by logit_scale.
-static bool score_ok(int score, bool sd) { return sd ? score == RGBMP_ATT_SD : score >= RGBMP_ATT_GAT && score <= RGBMP_ATT_FA; }
-
-// What the SD entry points check before att_forward / att_backward (which check pointers and the dropout descriptor):
-// the shape (EINVAL here), a square graph -- X holds the features of both endpoints -- and gT its transpose, a finite
-// scale, and at most one dropout form.
-static int check_sd(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int H, int C, float logit_scale, const float* drop,
-                    const rgbmp_dropout_t* d, const char* fn) {
-  int rc = check_g(g, fn);
-  if (rc) return rc;
-  if (gT && (rc = check_g(gT, fn))) return rc;
-  Shape s;
-  if (!att_shape(H, C, &s))
-    return fail(RGBMP_EINVAL, "%s: unsupported H %d / C %d (H == 1 with C <= 128, or C in {8..128} a power of two)", fn, H, C);
-  if (g->n_rows != g->n_cols || (gT && (gT->n_rows != g->n_cols || gT->n_cols != g->n_rows || gT->nnz != g->nnz)))
-    return fail(RGBMP_EINVAL, "%s: SD needs a square graph (and its transpose)", fn);
-  if (!isfinite(logit_scale)) return fail(RGBMP_EINVAL, "%s: logit_scale must be finite", fn);
-  if (drop && d) return fail(RGBMP_EINVAL, "%s: at most one of drop / d", fn);
-  return 0;
-}
-
-// d == NULL: the explicit `drop` mask (or none); d != NULL: fused dropout
-static int att_forward(const char* fn, const rgbmp_graph_t* g, int score, const float* X, int64_t ldx, const float* a_nbr,
-                       const float* a_own, const float* dinv, int H, int C, float slope, const float* drop,
-                       const rgbmp_dropout_t* d, float* out, int64_t ldo, float* rowmax, float* rowsum, float* out2,
-                       int64_t ldo2, float* rowq, void* ws, size_t ws_bytes, int device, void* stream,
-                       bool sd = false, float logit_scale = 0.f) {
+int rgbmp_att_forward(const rgbmp_graph_t* g, int score, const float* X, int64_t ldx, const float* a_nbr,
+                      const float* a_own, const float* dinv, int H, int C, float slope, float logit_scale,
+                      const float* drop, const rgbmp_dropout_t* d, float* out, int64_t ldo, float* rowmax,
+                      float* rowsum, float* out2, int64_t ldo2, float* rowq, void* ws, size_t ws_bytes, int device,
+                      void* stream) {
+  const char* fn = "rgbmp_att_forward";
   int rc = check_g(g, fn);
   if (rc) return rc;
   Shape s;
-  if (!score_ok(score, sd) || (score == RGBMP_ATT_FA && H != 1) || !att_shape(H, C, &s))
+  if (!att_ok(score, H, C, &s))
     return fail(RGBMP_ERANGE, "%s: unsupported score %d / H %d / C %d (H == 1 with C <= 128, or C in {8..128} a power of two)",
                 fn, score, H, C);
+  const bool sd = score == RGBMP_ATT_SD;                   // X holds the features of both endpoints
+  if (sd && (g->n_rows != g->n_cols || !isfinite(logit_scale)))
+    return fail(RGBMP_EINVAL, "%s: SD needs a square graph and a finite logit_scale", fn);
+  if (drop && d) return fail(RGBMP_EINVAL, "%s: at most one of drop / d", fn);
   if (!X || (!sd && (!a_nbr || !a_own)) || !out || !ws) return fail(RGBMP_EINVAL, "%s: null pointer", fn);
   if (d && (!d->seed || (g->nnz > 0 && !d->eid))) return fail(RGBMP_EINVAL, "%s: dropout needs seed and eid", fn);
   const bool softmax = score != RGBMP_ATT_FA;
@@ -1209,40 +1208,20 @@ static int att_forward(const char* fn, const rgbmp_graph_t* g, int score, const 
   p.Xn = X; p.ldn = ldx; p.Xo = X; p.ldo_ = ldx; p.dinv = dinv; p.drop = drop;
   if (d) set_dropout(p, d, d->eid);
   p.out = out; p.ldo = ldo; p.out2 = out2; p.ldo2 = ldo2; p.rowmax = rowmax; p.rowsum = rowsum; p.rowq = rowq;
-  if (sd) return d ? launch_fwd<SC_SD, false, true>(p, s, st) : launch_fwd<SC_SD, false, false>(p, s, st);
-  if (softmax) {                                           // log2-domain copies of the score terms
+  if (score == RGBMP_ATT_FA) {
+    p.sn = a_nbr; p.so = a_own;
+  } else if (!sd) {                                        // log2-domain copies of the score terms
     att_scale_kernel<<<(unsigned)ceil_div(g->n_cols * H, 256), 256, 0, st>>>(a_nbr, g->n_cols * H, an2);
     att_scale_kernel<<<(unsigned)ceil_div(n * H, 256), 256, 0, st>>>(a_own, n * H, ao2);
     RGBMP_LAUNCH_CHECK("att_scale_kernel");
     p.sn = an2; p.so = ao2;
-  } else {
-    p.sn = a_nbr; p.so = a_own;
   }
-  if (d) {
-    if (score == RGBMP_ATT_GAT) return train ? launch_fwd<SC_GAT, true, true>(p, s, st) : launch_fwd<SC_GAT, false, true>(p, s, st);
-    if (score == RGBMP_ATT_MX) return launch_fwd<SC_MX, false, true>(p, s, st);
-    return train ? launch_fwd<SC_FA, true, true>(p, s, st) : launch_fwd<SC_FA, false, true>(p, s, st);
-  }
-  if (score == RGBMP_ATT_GAT) return train ? launch_fwd<SC_GAT, true, false>(p, s, st) : launch_fwd<SC_GAT, false, false>(p, s, st);
-  if (score == RGBMP_ATT_MX) return launch_fwd<SC_MX, false, false>(p, s, st);
-  return train ? launch_fwd<SC_FA, true, false>(p, s, st) : launch_fwd<SC_FA, false, false>(p, s, st);
-}
-
-int rgbmp_att_forward(const rgbmp_graph_t* g, int score, const float* X, int64_t ldx, const float* a_nbr,
-                      const float* a_own, const float* dinv, int H, int C, float slope, const float* drop, float* out,
-                      int64_t ldo, float* rowmax, float* rowsum, float* out2, int64_t ldo2, float* rowq, void* ws,
-                      size_t ws_bytes, int device, void* stream) {
-  return att_forward("rgbmp_att_forward", g, score, X, ldx, a_nbr, a_own, dinv, H, C, slope, drop, nullptr, out, ldo,
-                     rowmax, rowsum, out2, ldo2, rowq, ws, ws_bytes, device, stream);
-}
-
-int rgbmp_att_forward_dropout(const rgbmp_graph_t* g, int score, const float* X, int64_t ldx, const float* a_nbr,
-                              const float* a_own, const float* dinv, int H, int C, float slope, const rgbmp_dropout_t* d,
-                              float* out, int64_t ldo, float* rowmax, float* rowsum, float* out2, int64_t ldo2,
-                              float* rowq, void* ws, size_t ws_bytes, int device, void* stream) {
-  if (!d) return fail(RGBMP_EINVAL, "rgbmp_att_forward_dropout: null dropout descriptor");
-  return att_forward("rgbmp_att_forward_dropout", g, score, X, ldx, a_nbr, a_own, dinv, H, C, slope, nullptr, d, out,
-                     ldo, rowmax, rowsum, out2, ldo2, rowq, ws, ws_bytes, device, stream);
+  return with_kernel(score, d != nullptr, [&](auto sc, auto dr) {
+    constexpr int SC = decltype(sc)::value;
+    constexpr bool DR = decltype(dr)::value;
+    if constexpr (SC == SC_MX || SC == SC_SD) return launch_fwd<SC, false, DR>(p, s, st);
+    else return train ? launch_fwd<SC, true, DR>(p, s, st) : launch_fwd<SC, false, DR>(p, s, st);
+  });
 }
 
 size_t rgbmp_att_backward_workspace_bytes(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int H, int C) {
@@ -1252,20 +1231,25 @@ size_t rgbmp_att_backward_workspace_bytes(const rgbmp_graph_t* g, const rgbmp_gr
          split_bytes(items, H, H * C);
 }
 
-static int att_backward(const char* fn, const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int score, const float* X,
-                        int64_t ldx, const float* a_nbr, const float* a_own, const float* dinv, int H, int C, float slope,
-                        const float* drop, const int32_t* tpos, const rgbmp_dropout_t* d, const float* rowmax,
-                        const float* rowsum, const float* rowq, const float* out, int64_t ldo, const float* out2,
-                        int64_t ldo2, const float* dout, int64_t ldd, float* dX, int64_t lddx, float* dXf, int64_t lddxf,
-                        float* da_nbr, float* da_own, void* ws, size_t ws_bytes, int device, void* stream,
-                        bool sd = false, float logit_scale = 0.f) {
+int rgbmp_att_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int score, const float* X, int64_t ldx,
+                       const float* a_nbr, const float* a_own, const float* dinv, int H, int C, float slope,
+                       float logit_scale, const float* drop, const int32_t* tpos, const rgbmp_dropout_t* d,
+                       const float* rowmax, const float* rowsum, const float* rowq, const float* out, int64_t ldo,
+                       const float* out2, int64_t ldo2, const float* dout, int64_t ldd, float* dX, int64_t lddx,
+                       float* dXf, int64_t lddxf, float* da_nbr, float* da_own, void* ws, size_t ws_bytes, int device,
+                       void* stream) {
+  const char* fn = "rgbmp_att_backward";
   int rc = check_g(g, fn);
   if (rc) return rc;
   rc = check_g(gT, fn);
   if (rc) return rc;
   Shape s;
-  if (!score_ok(score, sd) || (score == RGBMP_ATT_FA && H != 1) || !att_shape(H, C, &s))
-    return fail(RGBMP_ERANGE, "%s: unsupported score %d / H %d / C %d", fn, score, H, C);
+  if (!att_ok(score, H, C, &s)) return fail(RGBMP_ERANGE, "%s: unsupported score %d / H %d / C %d", fn, score, H, C);
+  const bool sd = score == RGBMP_ATT_SD;
+  if (sd && (g->n_rows != g->n_cols || gT->n_rows != g->n_cols || gT->n_cols != g->n_rows || gT->nnz != g->nnz ||
+             !isfinite(logit_scale)))
+    return fail(RGBMP_EINVAL, "%s: SD needs a square graph, its transpose and a finite logit_scale", fn);
+  if (drop && d) return fail(RGBMP_EINVAL, "%s: at most one of drop / d", fn);
   if (!X || !dout || !dX || (!sd && (!a_nbr || !a_own || !da_nbr || !da_own)) || !ws || (drop && !tpos))
     return fail(RGBMP_EINVAL, "%s: null pointer", fn);
   const bool logit = score == RGBMP_ATT_MX || sd;             // one pass per orientation
@@ -1296,105 +1280,39 @@ static int att_backward(const char* fn, const rgbmp_graph_t* g, const rgbmp_grap
   if (!carve_split(pt, cv, HC, g->n_items > gT->n_items ? g->n_items : gT->n_items) || !cv.ok())
     return fail(RGBMP_EWORKSPACE, "%s: workspace carve", fn);
   const unsigned prep_grid = (unsigned)ceil_div(n_dst * H, 256);
-  if (score == RGBMP_ATT_GAT)
-    att_bwd_prep_kernel<SC_GAT><<<prep_grid, 256, 0, st>>>(dout, ldd, out, ldo, out2, ldo2, a_own, rowmax, rowsum, rowq, dinv, n_dst, H, C, stats, da_own);
-  else if (score == RGBMP_ATT_MX)
-    att_bwd_prep_kernel<SC_MX><<<prep_grid, 256, 0, st>>>(dout, ldd, out, ldo, out2, ldo2, a_own, rowmax, rowsum, rowq, dinv, n_dst, H, C, stats, da_own);
-  else if (sd)
-    att_bwd_prep_kernel<SC_SD><<<prep_grid, 256, 0, st>>>(dout, ldd, out, ldo, out2, ldo2, nullptr, rowmax, rowsum, rowq, dinv, n_dst, H, C, stats, nullptr);
-  else
-    att_bwd_prep_kernel<SC_FA><<<prep_grid, 256, 0, st>>>(dout, ldd, out, ldo, out2, ldo2, a_own, rowmax, rowsum, rowq, dinv, n_dst, H, C, stats, da_own);
-  RGBMP_LAUNCH_CHECK("att_bwd_prep_kernel");
-  if (score == RGBMP_ATT_MX) {
-    // pass F on the forward CSR: dXf_i = sum_j dlogit_ij x_j, da_r[i]
-    att_scale_kernel<<<(unsigned)ceil_div(g->n_cols * H, 256), 256, 0, st>>>(a_nbr, g->n_cols * H, an2);
-    RGBMP_LAUNCH_CHECK("att_scale_kernel");
-    AttParams pf = pt;
-    fill_graph(pf, g);
-    pf.Xn = X; pf.ldn = ldx; pf.sn = an2; pf.stats = stats; pf.Xo = X; pf.ldo_ = ldx; pf.Do = dout; pf.lddo = ldd;
-    pf.drop = drop; pf.out = dXf; pf.ldo = lddxf; pf.ds = da_own;
-    if (d) set_dropout(pf, d, d->eid);
-    rc = d ? launch_bwdF<SC_MX, true>(pf, s, st) : launch_bwdF<SC_MX, false>(pf, s, st);
-    if (rc) return rc;
-    pt.acc_in = dXf; pt.ld_acc = lddxf;
-    pt.Xn2 = X; pt.ldn2 = ldx;
-  }
-  if (sd) {
-    // SD has no score scalars, but the passes (att_bwd_combine_kernel among them) write a per-row ds: the zeros land
-    // in the slot of the scaled a_nbr copy, n_cols * H floats, which covers the rows of both orientations because
-    // check_sd admits square graphs only
-    AttParams pf = pt;
-    fill_graph(pf, g);
-    pf.Xn = X; pf.ldn = ldx; pf.stats = stats; pf.Xo = X; pf.ldo_ = ldx; pf.Do = dout; pf.lddo = ldd;
-    pf.drop = drop; pf.out = dXf; pf.ldo = lddxf; pf.ds = an2;
-    if (d) set_dropout(pf, d, d->eid);
-    rc = d ? launch_bwdF<SC_SD, true>(pf, s, st) : launch_bwdF<SC_SD, false>(pf, s, st);
-    if (rc) return rc;
-    pt.Xn = dout; pt.ldn = ldd; pt.stats = stats; pt.Xo = X; pt.ldo_ = ldx; pt.Xn2 = X; pt.ldn2 = ldx;
-    pt.drop = drop; pt.tpos = tpos; pt.out = dX; pt.ldo = lddx; pt.ds = an2; pt.acc_in = dXf; pt.ld_acc = lddxf;
+  return with_kernel(score, d != nullptr, [&](auto sc, auto dr) {
+    constexpr int SC = decltype(sc)::value;
+    constexpr bool DR = decltype(dr)::value;
+    att_bwd_prep_kernel<SC><<<prep_grid, 256, 0, st>>>(dout, ldd, out, ldo, out2, ldo2, a_own, rowmax, rowsum, rowq, dinv,
+                                                       n_dst, H, C, stats, da_own);
+    RGBMP_LAUNCH_CHECK("att_bwd_prep_kernel");
+    if constexpr (SC == SC_MX || SC == SC_SD) {
+      // pass F on the forward CSR: dXf_i = sum_j dlogit_ij x_j, da_r[i]
+      AttParams pf = pt;
+      fill_graph(pf, g);
+      if constexpr (SC == SC_MX) {
+        att_scale_kernel<<<(unsigned)ceil_div(g->n_cols * H, 256), 256, 0, st>>>(a_nbr, g->n_cols * H, an2);
+        RGBMP_LAUNCH_CHECK("att_scale_kernel");
+        pf.sn = an2;
+      }
+      pf.Xn = X; pf.ldn = ldx; pf.stats = stats; pf.Xo = X; pf.ldo_ = ldx; pf.Do = dout; pf.lddo = ldd;
+      // SD has no score scalars, but the passes (att_bwd_combine_kernel among them) write a per-row ds: the zeros
+      // land in the slot of the scaled a_nbr copy, n_cols * H floats, which covers the rows of both orientations
+      // because SD admits square graphs only
+      pf.drop = drop; pf.out = dXf; pf.ldo = lddxf; pf.ds = SC == SC_SD ? an2 : da_own;
+      if (d) set_dropout(pf, d, d->eid);
+      const int rc = launch_bwdF<SC, DR>(pf, s, st);
+      if (rc) return rc;
+      pt.acc_in = dXf; pt.ld_acc = lddxf;
+      pt.Xn2 = X; pt.ldn2 = ldx;
+    }
+    // pass T on the transpose CSR: dX_j, da_src[j]
+    pt.Xn = dout; pt.ldn = ldd; pt.stats = stats; pt.Xo = X; pt.ldo_ = ldx;
+    if constexpr (SC != SC_SD) { pt.dinv = dinv; pt.so = a_nbr; }
+    pt.drop = drop; pt.tpos = tpos; pt.out = dX; pt.ldo = lddx; pt.ds = SC == SC_SD ? an2 : da_nbr;
     if (d) set_dropout(pt, d, d->eid_t);
-    return d ? launch_bwdT<SC_SD, true>(pt, s, st) : launch_bwdT<SC_SD, false>(pt, s, st);
-  }
-  // pass T on the transpose CSR: dX_j, da_src[j]
-  pt.Xn = dout; pt.ldn = ldd; pt.stats = stats; pt.dinv = dinv; pt.Xo = X; pt.ldo_ = ldx; pt.so = a_nbr;
-  pt.drop = drop; pt.tpos = tpos; pt.out = dX; pt.ldo = lddx; pt.ds = da_nbr;
-  if (d) {
-    set_dropout(pt, d, d->eid_t);
-    if (score == RGBMP_ATT_GAT) return launch_bwdT<SC_GAT, true>(pt, s, st);
-    if (score == RGBMP_ATT_MX) return launch_bwdT<SC_MX, true>(pt, s, st);
-    return launch_bwdT<SC_FA, true>(pt, s, st);
-  }
-  if (score == RGBMP_ATT_GAT) return launch_bwdT<SC_GAT, false>(pt, s, st);
-  if (score == RGBMP_ATT_MX) return launch_bwdT<SC_MX, false>(pt, s, st);
-  return launch_bwdT<SC_FA, false>(pt, s, st);
-}
-
-int rgbmp_att_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int score, const float* X, int64_t ldx,
-                       const float* a_nbr, const float* a_own, const float* dinv, int H, int C, float slope,
-                       const float* drop, const int32_t* tpos, const float* rowmax, const float* rowsum,
-                       const float* rowq, const float* out, int64_t ldo, const float* out2, int64_t ldo2,
-                       const float* dout, int64_t ldd, float* dX, int64_t lddx, float* dXf, int64_t lddxf,
-                       float* da_nbr, float* da_own, void* ws, size_t ws_bytes, int device, void* stream) {
-  return att_backward("rgbmp_att_backward", g, gT, score, X, ldx, a_nbr, a_own, dinv, H, C, slope, drop, tpos, nullptr,
-                      rowmax, rowsum, rowq, out, ldo, out2, ldo2, dout, ldd, dX, lddx, dXf, lddxf, da_nbr, da_own, ws,
-                      ws_bytes, device, stream);
-}
-
-int rgbmp_att_backward_dropout(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int score, const float* X, int64_t ldx,
-                               const float* a_nbr, const float* a_own, const float* dinv, int H, int C, float slope,
-                               const rgbmp_dropout_t* d, const float* rowmax, const float* rowsum, const float* rowq,
-                               const float* out, int64_t ldo, const float* out2, int64_t ldo2, const float* dout,
-                               int64_t ldd, float* dX, int64_t lddx, float* dXf, int64_t lddxf, float* da_nbr,
-                               float* da_own, void* ws, size_t ws_bytes, int device, void* stream) {
-  if (!d) return fail(RGBMP_EINVAL, "rgbmp_att_backward_dropout: null dropout descriptor");
-  return att_backward("rgbmp_att_backward_dropout", g, gT, score, X, ldx, a_nbr, a_own, dinv, H, C, slope, nullptr,
-                      nullptr, d, rowmax, rowsum, rowq, out, ldo, out2, ldo2, dout, ldd, dX, lddx, dXf, lddxf, da_nbr,
-                      da_own, ws, ws_bytes, device, stream);
-}
-
-int rgbmp_att_sd_forward(const rgbmp_graph_t* g, const float* X, int64_t ldx, int H, int C, float logit_scale,
-                         float slope, const float* drop, const rgbmp_dropout_t* d, float* out, int64_t ldo,
-                         float* rowmax, float* rowsum, void* ws, size_t ws_bytes, int device, void* stream) {
-  const char* fn = "rgbmp_att_sd_forward";
-  int rc = check_sd(g, nullptr, H, C, logit_scale, drop, d, fn);
-  if (rc) return rc;
-  return att_forward(fn, g, RGBMP_ATT_SD, X, ldx, nullptr, nullptr, nullptr, H, C, slope, drop, d, out, ldo, rowmax,
-                     rowsum, nullptr, 0, nullptr, ws, ws_bytes, device, stream, true, logit_scale);
-}
-
-int rgbmp_att_sd_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, const float* X, int64_t ldx, int H, int C,
-                          float logit_scale, float slope, const float* drop, const int32_t* tpos,
-                          const rgbmp_dropout_t* d, const float* rowmax, const float* rowsum,
-                          const float* out, int64_t ldo, const float* dout, int64_t ldd,
-                          float* dX, int64_t lddx, float* dXf, int64_t lddxf,
-                          void* ws, size_t ws_bytes, int device, void* stream) {
-  const char* fn = "rgbmp_att_sd_backward";
-  if (!gT) return fail(RGBMP_EINVAL, "%s: null pointer", fn);
-  int rc = check_sd(g, gT, H, C, logit_scale, drop, d, fn);
-  if (rc) return rc;
-  return att_backward(fn, g, gT, RGBMP_ATT_SD, X, ldx, nullptr, nullptr, nullptr, H, C, slope, drop, tpos, d, rowmax,
-                      rowsum, nullptr, out, ldo, nullptr, 0, dout, ldd, dX, lddx, dXf, lddxf, nullptr, nullptr, ws,
-                      ws_bytes, device, stream, true, logit_scale);
+    return launch_bwdT<SC, DR>(pt, s, st);
+  });
 }
 
 int rgbmp_dropout_mask(const rgbmp_dropout_t* d, int64_t nnz, int H, float* out, int device, void* stream) {

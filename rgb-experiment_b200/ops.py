@@ -600,20 +600,10 @@ class _Att(torch.autograd.Function):
         L = lib()
         wsb = L.rgbmp_att_forward_workspace_bytes(graph.fwd.ref, H, Cc)
         ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
-        if score == ATT_SD:
-            d = None if seed is None else C.byref(_dropout_struct(p, seed, graph))
-            check(L.rgbmp_att_sd_forward(graph.fwd.ref, ptr(xb), ldx, H, Cc, logit_scale, slope, ptr(drop_csr), d,
-                                         ptr(out), ldo, ptr(rmax), ptr(rsum), ptr(ws), wsb, dev.index, stream_of(dev)),
-                  "att_sd_forward")
-        elif seed is None:
-            check(L.rgbmp_att_forward(graph.fwd.ref, score, ptr(xb), ldx, ptr(a_n), ptr(a_o), ptr(dinv), H, Cc, slope,
-                                      ptr(drop_csr), ptr(out), ldo, ptr(rmax), ptr(rsum), ptr(out2), ldo2, ptr(rowq),
-                                      ptr(ws), wsb, dev.index, stream_of(dev)), "att_forward")
-        else:
-            d = _dropout_struct(p, seed, graph)
-            check(L.rgbmp_att_forward_dropout(graph.fwd.ref, score, ptr(xb), ldx, ptr(a_n), ptr(a_o), ptr(dinv), H, Cc,
-                                              slope, C.byref(d), ptr(out), ldo, ptr(rmax), ptr(rsum), ptr(out2), ldo2,
-                                              ptr(rowq), ptr(ws), wsb, dev.index, stream_of(dev)), "att_forward_dropout")
+        d = None if seed is None else C.byref(_dropout_struct(p, seed, graph))
+        check(L.rgbmp_att_forward(graph.fwd.ref, score, ptr(xb), ldx, ptr(a_n), ptr(a_o), ptr(dinv), H, Cc, slope,
+                                  logit_scale, ptr(drop_csr), d, ptr(out), ldo, ptr(rmax), ptr(rsum), ptr(out2), ldo2,
+                                  ptr(rowq), ptr(ws), wsb, dev.index, stream_of(dev)), "att_forward")
         ctx.graph, ctx.score, ctx.H, ctx.Cc, ctx.slope, ctx.p, ctx.logit_scale = graph, score, H, Cc, slope, p, logit_scale
         ctx.save_for_backward(xb, a_n, a_o, rmax, rsum, rowq, out, out2, drop_csr, seed)
         return out
@@ -631,28 +621,16 @@ class _Att(torch.autograd.Function):
         L = lib()
         wsb = L.rgbmp_att_backward_workspace_bytes(g.fwd.ref, g.bwd.ref, H, Cc)
         ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
-        if score == ATT_SD:
-            d = None if seed is None else C.byref(_dropout_struct(ctx.p, seed, g, backward=True))
-            check(L.rgbmp_att_sd_backward(g.fwd.ref, g.bwd.ref, ptr(xb), xb.stride(0), H, Cc, ctx.logit_scale, ctx.slope,
-                                          ptr(drop), ptr(tpos), d, ptr(rmax), ptr(rsum), ptr(out), out.stride(0), ptr(db),
-                                          ldd, ptr(dx), lddx, ptr(dxf), lddxf, ptr(ws), wsb, dev.index, stream_of(dev)),
-                  "att_sd_backward")
-            return dx, None, None, None, None, None, None, None, None, None, None, None
-        da_n = torch.empty((N, H), dtype=torch.float32, device=dev)
-        da_o = torch.empty((N, H), dtype=torch.float32, device=dev)
+        da_n = da_o = None                                   # SD has no score scalars
+        if score != ATT_SD:
+            da_n = torch.empty((N, H), dtype=torch.float32, device=dev)
+            da_o = torch.empty((N, H), dtype=torch.float32, device=dev)
         ld2 = 0 if out2 is None else out2.stride(0)
-        if seed is None:
-            check(L.rgbmp_att_backward(g.fwd.ref, g.bwd.ref, score, ptr(xb), xb.stride(0), ptr(a_n), ptr(a_o), ptr(dinv), H,
-                                       Cc, ctx.slope, ptr(drop), ptr(tpos), ptr(rmax), ptr(rsum), ptr(rowq), ptr(out),
-                                       out.stride(0), ptr(out2), ld2, ptr(db), ldd, ptr(dx), lddx, ptr(dxf), lddxf,
-                                       ptr(da_n), ptr(da_o), ptr(ws), wsb, dev.index, stream_of(dev)), "att_backward")
-        else:
-            d = _dropout_struct(ctx.p, seed, g, backward=True)
-            check(L.rgbmp_att_backward_dropout(g.fwd.ref, g.bwd.ref, score, ptr(xb), xb.stride(0), ptr(a_n), ptr(a_o),
-                                               ptr(dinv), H, Cc, ctx.slope, C.byref(d), ptr(rmax), ptr(rsum), ptr(rowq),
-                                               ptr(out), out.stride(0), ptr(out2), ld2, ptr(db), ldd, ptr(dx), lddx,
-                                               ptr(dxf), lddxf, ptr(da_n), ptr(da_o), ptr(ws), wsb, dev.index,
-                                               stream_of(dev)), "att_backward_dropout")
+        d = None if seed is None else C.byref(_dropout_struct(ctx.p, seed, g, backward=True))
+        check(L.rgbmp_att_backward(g.fwd.ref, g.bwd.ref, score, ptr(xb), xb.stride(0), ptr(a_n), ptr(a_o), ptr(dinv), H, Cc,
+                                   ctx.slope, ctx.logit_scale, ptr(drop), ptr(tpos), d, ptr(rmax), ptr(rsum), ptr(rowq),
+                                   ptr(out), out.stride(0), ptr(out2), ld2, ptr(db), ldd, ptr(dx), lddx, ptr(dxf), lddxf,
+                                   ptr(da_n), ptr(da_o), ptr(ws), wsb, dev.index, stream_of(dev)), "att_backward")
         return dx, da_n, da_o, None, None, None, None, None, None, None, None, None
 
 

@@ -31,10 +31,10 @@ def test_every_declared_symbol_is_exported():
     assert not missing, missing
 
 
-def test_binding_loads_and_version_matches():
+def test_binding_loads_and_version_is_101():
     import rgb_experiment_b200 as R
     L = R._lib.lib()
-    assert L.rgbmp_version() == 100
+    assert L.rgbmp_version() == 101
     for n in declared_symbols():
         assert getattr(L, n).argtypes is not None or n in ("rgbmp_version", "rgbmp_last_error"), n
 

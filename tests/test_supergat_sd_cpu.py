@@ -1,6 +1,6 @@
 """SuperGATConv's SD attention without a GPU: a dense fp64 statement of the paper's equation agrees with the oracle
-layer; RGBMP_ATT_SD has the shape rules of MX; the SD entry points reject bad arguments with RGBMP_EINVAL before
-touching a device, and the generic attention entry points keep refusing score 3.
+layer; RGBMP_ATT_SD has the shape rules of MX; the attention entry points reject bad SD arguments before touching a
+device, and refuse unknown scores and bad dropout arguments for every score.
 
   SuperGAT  Kim & Oh 2021, eq. 3 (SD)   e_ij = (Wh_i . Wh_j) / sqrt(C),  alpha = softmax_j(leaky_relu(e_ij))
 """
@@ -68,63 +68,92 @@ def _drop(seed=FAKE, eid=FAKE, eid_t=FAKE):
     return DropoutStruct(seed, eid, eid_t, 1 << 31, 2.0)
 
 
-def _fwd(g=None, X=FAKE, H=8, Cc=8, drop=None, d=None, out=FAKE, rowmax=FAKE, rowsum=FAKE, ws=FAKE, scale=0.35):
+def _fwd(g=None, X=FAKE, H=8, Cc=8, drop=None, d=None, out=FAKE, rowmax=FAKE, rowsum=FAKE, ws=FAKE, scale=0.35,
+         score=3, a=None, dinv=None, out2=None, rowq=None):
     g = _graph() if g is None else g
-    return L().rgbmp_att_sd_forward(C.byref(g) if g is not False else None, X, 64, H, Cc, scale, 0.2, drop,
-                                    None if d is None else C.byref(d), out, 64, rowmax, rowsum, ws, 1 << 30, 0, None)
+    return L().rgbmp_att_forward(C.byref(g) if g is not False else None, score, X, 64, a, a, dinv, H, Cc, 0.2, scale,
+                                 drop, None if d is None else C.byref(d), out, 64, rowmax, rowsum, out2, 64, rowq, ws,
+                                 1 << 30, 0, None)
 
 
 def _bwd(g=None, gT=None, X=FAKE, H=8, Cc=8, drop=None, tpos=None, d=None, out=FAKE, dout=FAKE, dX=FAKE, dXf=FAKE,
-         ws=FAKE, scale=0.35):
+         ws=FAKE, scale=0.35, score=3, a=None, dinv=None, out2=None, rowq=None):
     g = _graph() if g is None else g
     gT = _graph() if gT is None else gT
-    return L().rgbmp_att_sd_backward(C.byref(g), C.byref(gT) if gT is not False else None, X, 64, H, Cc, scale, 0.2,
-                                     drop, tpos, None if d is None else C.byref(d), FAKE, FAKE, out, 64, dout, 64,
-                                     dX, 64, dXf, 64, ws, 1 << 30, 0, None)
+    return L().rgbmp_att_backward(C.byref(g), C.byref(gT) if gT is not False else None, score, X, 64, a, a, dinv, H, Cc,
+                                  0.2, scale, drop, tpos, None if d is None else C.byref(d), FAKE, FAKE, rowq, out, 64,
+                                  out2, 64, dout, 64, dX, 64, dXf, 64, a, a, ws, 1 << 30, 0, None)
 
 
-def _einval(rc, fn):
+def _rc(rc, code, fn, msg=b""):
+    assert rc == code
+    err = L().rgbmp_last_error()
+    assert fn.encode() in err and msg in err and b"bad device" not in err, err
+
+
+def _einval(rc, fn, msg=b""):
     from rgb_experiment_b200._lib import EINVAL
-    assert rc == EINVAL
-    assert fn.encode() in L().rgbmp_last_error()
+    _rc(rc, EINVAL, fn, msg)
 
 
-def test_sd_forward_argument_errors():
-    fn = "rgbmp_att_sd_forward"
+def _erange(rc, fn):
+    from rgb_experiment_b200._lib import ERANGE
+    _rc(rc, ERANGE, fn, b"unsupported score")
+
+
+def test_att_forward_sd_argument_errors():
+    fn = "rgbmp_att_forward"
     _einval(_fwd(g=False), fn)
     for kw in ({"X": None}, {"out": None}, {"rowmax": None}, {"rowsum": None}, {"ws": None}):
         _einval(_fwd(**kw), fn)
     _einval(_fwd(drop=FAKE, d=_drop()), fn)                 # both dropout forms
     for H, Cc in ((8, 12), (2, 130), (1, 129), (3, 7), (0, 8)):
-        _einval(_fwd(H=H, Cc=Cc), fn)
+        _erange(_fwd(H=H, Cc=Cc), fn)
     _einval(_fwd(d=_drop(eid=None)), fn)
     _einval(_fwd(d=_drop(seed=None)), fn)
     _einval(_fwd(g=_graph(square=False)), fn)
     _einval(_fwd(scale=float("nan")), fn)
+    _einval(_fwd(out2=FAKE, rowq=FAKE), fn)                # SD has no second aggregate
 
 
-def test_sd_backward_argument_errors():
-    fn = "rgbmp_att_sd_backward"
+def test_att_backward_sd_argument_errors():
+    fn = "rgbmp_att_backward"
     _einval(_bwd(gT=False), fn)
     for kw in ({"X": None}, {"out": None}, {"dout": None}, {"dX": None}, {"dXf": None}, {"ws": None},
                {"drop": FAKE}):                            # an explicit mask needs tpos
         _einval(_bwd(**kw), fn)
     _einval(_bwd(drop=FAKE, tpos=FAKE, d=_drop()), fn)
     for H, Cc in ((8, 12), (2, 130), (1, 129), (3, 7)):
-        _einval(_bwd(H=H, Cc=Cc), fn)
+        _erange(_bwd(H=H, Cc=Cc), fn)
     _einval(_bwd(d=_drop(eid_t=None)), fn)
     _einval(_bwd(d=_drop(eid=None)), fn)
     _einval(_bwd(gT=_graph(n=5)), fn)                       # not the transpose of g
+    _einval(_bwd(scale=float("inf")), fn)
 
 
-def test_generic_entry_points_still_refuse_score_3():
-    from rgb_experiment_b200._lib import ERANGE
-    lib = L()
-    g = _graph()
-    rc = lib.rgbmp_att_forward(C.byref(g), 3, FAKE, 64, FAKE, FAKE, None, 8, 8, 0.2, None, FAKE, 64, FAKE, FAKE, None,
-                               0, None, FAKE, 1 << 30, 0, None)
-    assert rc == ERANGE and b"unsupported score 3" in lib.rgbmp_last_error()
-    rc = lib.rgbmp_att_backward(C.byref(g), C.byref(g), 3, FAKE, 64, FAKE, FAKE, None, 8, 8, 0.2, None, None, FAKE,
-                                FAKE, None, FAKE, 64, None, 0, FAKE, 64, FAKE, 64, FAKE, 64, FAKE, FAKE, FAKE, 1 << 30,
-                                0, None)
-    assert rc == ERANGE and b"unsupported score 3" in lib.rgbmp_last_error()
+# every argument the score reads, so that only the one under test is wrong: GAT / MX / FA read a_nbr, a_own;
+# FA is single-head and reads dinv; the GAT / FA backward reads the training-mode forward's out2 (GAT also rowq)
+SCORES = {0: dict(H=8, a=FAKE, out2=FAKE, rowq=FAKE), 1: dict(H=8, a=FAKE),
+          2: dict(H=1, a=FAKE, dinv=FAKE, out2=FAKE)}
+
+
+def test_unknown_scores_are_out_of_range():
+    for score in (-1, 4):
+        _erange(_fwd(score=score, a=FAKE), "rgbmp_att_forward")
+        _erange(_bwd(score=score, a=FAKE), "rgbmp_att_backward")
+
+
+@pytest.mark.parametrize("score", sorted(SCORES))
+def test_gat_mx_fa_dropout_argument_errors(score):
+    kw = SCORES[score]
+    fwd_kw = {k: v for k, v in kw.items() if k not in ("out2", "rowq")}   # inference forward
+    fn, both, seed_eid = "rgbmp_att_forward", b"at most one of drop / d", b"dropout needs seed"
+    _einval(_fwd(score=score, drop=FAKE, d=_drop(), **fwd_kw), fn, both)
+    _einval(_fwd(score=score, d=_drop(seed=None), **fwd_kw), fn, seed_eid)
+    _einval(_fwd(score=score, d=_drop(eid=None), **fwd_kw), fn, seed_eid)
+    fn = "rgbmp_att_backward"
+    _einval(_bwd(score=score, drop=FAKE, tpos=FAKE, d=_drop(), **kw), fn, both)
+    _einval(_bwd(score=score, d=_drop(seed=None), **kw), fn, seed_eid)
+    _einval(_bwd(score=score, d=_drop(eid_t=None), **kw), fn, seed_eid)
+    if score == 1:                                          # MX also runs a pass on the forward CSR
+        _einval(_bwd(score=score, d=_drop(eid=None), **kw), fn, seed_eid)
