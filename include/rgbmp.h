@@ -166,8 +166,16 @@ typedef struct rgbmp_graph {
   const int64_t* item_start;   /* [n_items]                                                         */
   const int32_t* row_order;    /* [n_rows] schedule of the short-row kernel, or NULL = natural order */
   int32_t        col_tagged;   /* 1: bit 31 of col[k] marks a frequently gathered ("hot") column, see
-                                  rgbmp_col_tag; only rgbmp_spmm / rgbmp_khop accept it      */
+                                  rgbmp_col_tag                                                     */
 } rgbmp_graph_t;
+/* Every entry point that takes an rgbmp_graph_t checks it before it selects a device:
+ *   RGBMP_EINVAL  NULL descriptor or rowptr, n_rows < 0, nnz < 0, or col NULL with nnz > 0;
+ *   RGBMP_EINVAL  n_items > 0 without chunk > 0, long_chunk > 0 and all four long-row lists (never run unsplit);
+ *   RGBMP_ERANGE  n_cols >= 2^31;
+ *   RGBMP_EINVAL  col_tagged = 1, except in rgbmp_spmm, rgbmp_khop and rgbmp_appnp_host, whose kernels strip the tag;
+ *   RGBMP_EINVAL  n_rows != n_cols where the graph must be square: rgbmp_khop, rgbmp_appnp_host, RGBMP_ATT_SD's g,
+ *                 rgbmp_cluster_lpa and rgbmp_cluster_connectivity.
+ * n_items <= 0 means no long rows: the long-row fields are then ignored. */
 
 
 /* Fused epilogue applied to every output row i after the segmented sum s_i (all optional):

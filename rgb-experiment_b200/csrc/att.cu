@@ -17,9 +17,9 @@
 //   * heads are independent, so wide layers (H*C > 128) are tiled over blockIdx.y in groups of HT heads;
 //   * logits live in the log2 domain (a_src/a_dst pre-multiplied by log2 e; leaky_relu and the product with
 //     sigmoid > 0 commute with a positive scale), exp is a bare ex2.approx;
-//   * the SpMM machinery is reused: degree/locality row schedule, one coalesced load of G column ids per batch +
-//     shuffle broadcast, software-pipelined full batches (forward), rows longer than `chunk` split into CTA work
-//     items whose partial (max, sum, acc) states are merged in item order.
+//   * SpMM's row-split schedule (csr_work.cuh): degree/locality row schedule, one coalesced load of G column ids per
+//     batch broadcast through shared memory, rows longer than `chunk` split into CTA work items whose partial
+//     (max, sum, acc) states are merged in item order; software-pipelined full batches (forward).
 // DETERMINISTIC, no atomics anywhere.  The gradient of the per-TARGET score term (da_dst / da_r) is a sum over a
 // target's in-edges while the backward walks the transpose CSR; instead of atomics it uses linearity:
 //   GAT:  da_dst[i] = sum_j alpha_ij l'_ij (mask_ij <dout_i, x_j> - S_i) = <dout_i, P_i> - S_i q_i
@@ -32,7 +32,7 @@
 #include <math.h>
 #include <stdlib.h>
 #include <type_traits>
-#include "common.cuh"
+#include "csr_work.cuh"
 #include "philox.cuh"
 
 namespace rgbmp {
@@ -75,17 +75,7 @@ __device__ __forceinline__ float dot4(const float4& a, const float4& b) {
 __device__ __forceinline__ float4 zero4() { return make_float4(0.f, 0.f, 0.f, 0.f); }
 
 struct AttParams {
-  // graph (the orientation of this pass)
-  const int64_t* rowptr;
-  const int32_t* col;
-  const int32_t* row_order;
-  int64_t n_rows;
-  int32_t chunk, long_chunk;
-  const int32_t* long_rows;
-  const int32_t* long_item_ptr;
-  const int32_t* item_long;
-  const int64_t* item_start;
-  int64_t n_long, n_items;
+  CsrWork w;                          // the graph in the orientation of this pass
   // geometry: H heads of C channels, HT heads per blockIdx.y tile, LPH lanes per head
   int H, HT, C, LPH;
   float slope;
@@ -175,36 +165,6 @@ __device__ __forceinline__ void load_own(const float* X, int64_t ld, int64_t row
   x[1] = L.nact > 1 ? __ldg(reinterpret_cast<const float4*>(X + row * ld + L.f + 4)) : zero4();
 }
 
-__device__ __forceinline__ bool row_of_group(const AttParams& p, int G, int64_t& row, int64_t& k0, int64_t& k1) {
-  const int GPB = ATT_THREADS / G;
-  const int64_t gid = (int64_t)blockIdx.x * GPB + threadIdx.x / G;
-  row = -1;
-  k0 = k1 = 0;
-  if (gid < p.n_rows) {
-    row = p.row_order ? (int64_t)__ldg(p.row_order + gid) : gid;
-    k0 = __ldg(p.rowptr + row);
-    k1 = __ldg(p.rowptr + row + 1);
-    if (p.n_items > 0 && k1 - k0 > p.chunk) row = -1;       // long row: the *_long kernel owns it
-  }
-  if (row < 0) k1 = k0;
-  return row >= 0;
-}
-
-__device__ __forceinline__ void item_range(const AttParams& p, int G, int64_t& row, int64_t& k0, int64_t& k1) {
-  const int Q = ATT_THREADS / G;
-  const int q = threadIdx.x / G;
-  const int64_t item = blockIdx.x;
-  row = p.long_rows[p.item_long[item]];
-  const int64_t rs = p.item_start[item];
-  const int64_t rend = __ldg(p.rowptr + row + 1);
-  const int64_t re = (rs + p.long_chunk < rend) ? rs + p.long_chunk : rend;
-  const int64_t per = (re - rs + Q - 1) / Q;
-  k0 = rs + (int64_t)q * per;
-  k1 = k0 + per;
-  if (k0 > re) k0 = re;
-  if (k1 > re) k1 = re;
-}
-
 // =============================================================================================
 // forward
 // =============================================================================================
@@ -212,20 +172,6 @@ struct FwdState {
   float m, s, q;            // running max (log2 domain), running sum, running sum of alpha*l'
   float4 acc[2], acc2[2];
 };
-
-// Column ids of a batch reach the lanes of a group through shared memory (one STS per lane, then broadcast LDS of
-// the UU ids of a step) instead of one SHFL per edge: a SHFL occupies the LSU data pipe for 4 wavefronts, the
-// same pipe that serves the gathers (profiles/r02_spmm_l1_wavefronts.txt).
-template <int N>
-__device__ __forceinline__ void lds_ids(const int32_t* p, uint32_t (&c)[N]) {
-  if constexpr (N == 4) {
-    const int4 v = *reinterpret_cast<const int4*>(p);
-    c[0] = v.x; c[1] = v.y; c[2] = v.z; c[3] = v.w;
-  } else {
-    const int2 v = *reinterpret_cast<const int2*>(p);
-    c[0] = v.x; c[1] = v.y;
-  }
-}
 
 template <int SC, bool TRAIN, int UU, bool DR>
 __device__ __forceinline__ void fwd_consume(const AttParams& p, const float4 (&x)[UU][2], const float (&sn)[UU], const float (&dn)[UU],
@@ -309,7 +255,7 @@ __device__ __forceinline__ void fwd_range(const AttParams& p, int64_t k0, int64_
   const int len = (k1 > k0) ? (int)(k1 - k0) : 0;
   const int maxlen = __reduce_max_sync(FULLMASK, len);
   if (maxlen == 0) return;
-  const int32_t* __restrict__ col = p.col + k0;
+  const int32_t* __restrict__ col = p.w.col + k0;
   const char* xb0 = reinterpret_cast<const char*>(p.Xn + L.f);
   const char* xb1 = reinterpret_cast<const char*>(p.Xn + L.f + 4);
   const bool a0 = L.nact > 0, a1 = L.nact > 1;             // lanes beyond the row issue no feature load
@@ -415,7 +361,7 @@ __global__ void __launch_bounds__(ATT_THREADS, fwd_minb<SC, TRAIN>()) att_fwd_ro
   __shared__ __align__(16) int32_t sm_ids[ATT_THREADS];
   const int gl = threadIdx.x % G;
   int64_t row, k0, k1;
-  const bool live = row_of_group(p, G, row, k0, k1);
+  const bool live = short_row<G, ATT_THREADS>(p.w, row, k0, k1);
   const Lane L = lane_of(p, gl);
   float so = 0.f, d_own = 0.f;
   float4 xi[2] = {zero4(), zero4()};
@@ -462,7 +408,7 @@ __global__ void __launch_bounds__(ATT_THREADS, fwd_minb<SC, TRAIN>()) att_fwd_lo
   __shared__ float sm_m[Q][G], sm_s[Q][G], sm_q[Q][G];      // heads per tile <= lanes per group
   const int gl = threadIdx.x % G, q = threadIdx.x / G;
   int64_t row, k0, k1;
-  item_range(p, G, row, k0, k1);
+  long_item<G, ATT_THREADS>(p.w, row, k0, k1);
   const Lane L = lane_of(p, gl);
   const float so = (SC == SC_SD) ? 0.f : __ldg(p.so + row * p.H + L.h);
   float d_own = 0.f;
@@ -545,10 +491,10 @@ __global__ void __launch_bounds__(256) att_fwd_combine_kernel(const AttParams p)
   const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t slot = t / HC;
   const int f = (int)(t - slot * HC);
-  if (slot >= p.n_long) return;
-  const int64_t row = p.long_rows[slot];
+  if (slot >= p.w.n_long) return;
+  const int64_t row = p.w.long_rows[slot];
   const int h = (p.H == 1) ? 0 : f / p.C;
-  const int32_t i0 = p.long_item_ptr[slot], i1 = p.long_item_ptr[slot + 1];
+  const int32_t i0 = p.w.long_item_ptr[slot], i1 = p.w.long_item_ptr[slot + 1];
   float acc = 0.f, acc2 = 0.f, s = 0.f, qv = 0.f, M = -INFINITY, inv = 1.0f;
   if constexpr (SC == SC_FA) {
     for (int32_t it = i0; it < i1; ++it) {
@@ -654,7 +600,7 @@ __device__ __forceinline__ void bwdT_range(const AttParams& p, int64_t k0, int64
   const int len = (k1 > k0) ? (int)(k1 - k0) : 0;
   const int maxlen = __reduce_max_sync(FULLMASK, len);
   if (maxlen == 0) return;
-  const int32_t* __restrict__ col = p.col + k0;
+  const int32_t* __restrict__ col = p.w.col + k0;
   const char* db0 = reinterpret_cast<const char*>(p.Xn + L.f);
   const char* db1 = reinterpret_cast<const char*>(p.Xn + L.f + 4);
   const uint32_t d_bytes = (uint32_t)(p.ldn * 4);
@@ -749,7 +695,7 @@ __global__ void __launch_bounds__(ATT_THREADS, bwdT_minb<SC>()) att_bwdT_rows_ke
   __shared__ __align__(16) int32_t sm_ids[ATT_THREADS];
   const int gl = threadIdx.x % G;
   int64_t row, k0, k1;
-  const bool live = row_of_group(p, G, row, k0, k1);
+  const bool live = short_row<G, ATT_THREADS>(p.w, row, k0, k1);
   const Lane L = lane_of(p, gl);
   float so2 = 0.f, d_own = 0.f;
   float4 xj[2] = {zero4(), zero4()}, acc[2] = {zero4(), zero4()};
@@ -813,7 +759,7 @@ __global__ void __launch_bounds__(ATT_THREADS, bwdT_minb<SC>()) att_bwdT_long_ke
   __shared__ float sm_s[Q][G];
   const int gl = threadIdx.x % G, q = threadIdx.x / G;
   int64_t row, k0, k1;
-  item_range(p, G, row, k0, k1);
+  long_item<G, ATT_THREADS>(p.w, row, k0, k1);
   const Lane L = lane_of(p, gl);
   const float so2 = (SC == SC_SD) ? 0.f : __ldg(p.so + row * p.H + L.h) * (SC == SC_FA ? 1.0f : LOG2E);
   float d_own = 0.f;
@@ -830,11 +776,11 @@ __global__ void __launch_bounds__(256) att_bwd_combine_kernel(const AttParams p)
   const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t slot = t / HC;
   const int f = (int)(t - slot * HC);
-  if (slot >= p.n_long) return;
-  const int64_t row = p.long_rows[slot];
+  if (slot >= p.w.n_long) return;
+  const int64_t row = p.w.long_rows[slot];
   const int h = (p.H == 1) ? 0 : f / p.C;
   float acc = 0.f, s = 0.f;
-  for (int32_t it = p.long_item_ptr[slot]; it < p.long_item_ptr[slot + 1]; ++it) {
+  for (int32_t it = p.w.long_item_ptr[slot]; it < p.w.long_item_ptr[slot + 1]; ++it) {
     acc += p.part_acc[(int64_t)it * p.ldp + f];
     s += p.part_s[(int64_t)it * p.H + h];
   }
@@ -852,7 +798,7 @@ __device__ __forceinline__ void bwdF_range(const AttParams& p, int64_t k0, int64
   const int len = (k1 > k0) ? (int)(k1 - k0) : 0;
   const int maxlen = __reduce_max_sync(FULLMASK, len);
   if (maxlen == 0) return;
-  const int32_t* __restrict__ col = p.col + k0;
+  const int32_t* __restrict__ col = p.w.col + k0;
   const char* xb0 = reinterpret_cast<const char*>(p.Xn + L.f);
   const char* xb1 = reinterpret_cast<const char*>(p.Xn + L.f + 4);
   const uint32_t row_bytes = (uint32_t)(p.ldn * 4);
@@ -922,7 +868,7 @@ __global__ void __launch_bounds__(ATT_THREADS, RGBMP_ATT_OCC >= 1 ? 3 : 2) att_b
   __shared__ __align__(16) int32_t sm_ids[ATT_THREADS];
   const int gl = threadIdx.x % G;
   int64_t row, k0, k1;
-  const bool live = row_of_group(p, G, row, k0, k1);
+  const bool live = short_row<G, ATT_THREADS>(p.w, row, k0, k1);
   const Lane L = lane_of(p, gl);
   float4 xi[2] = {zero4(), zero4()}, di[2] = {zero4(), zero4()}, acc[2] = {zero4(), zero4()};
   float4 st_own = zero4();
@@ -948,7 +894,7 @@ __global__ void __launch_bounds__(ATT_THREADS, RGBMP_ATT_OCC >= 1 ? 3 : 2) att_b
   __shared__ float sm_s[Q][G];
   const int gl = threadIdx.x % G, q = threadIdx.x / G;
   int64_t row, k0, k1;
-  item_range(p, G, row, k0, k1);
+  long_item<G, ATT_THREADS>(p.w, row, k0, k1);
   const Lane L = lane_of(p, gl);
   float4 xi[2], di[2], acc[2] = {zero4(), zero4()};
   load_own(p.Xo, p.ldo_, row, L, xi);
@@ -985,32 +931,6 @@ static bool att_shape(int H, int C, Shape* s) {
   return g <= 16;
 }
 
-static inline bool al16(const void* p, int64_t ld) { return (((uintptr_t)p) & 15) == 0 && (ld % 4) == 0; }
-
-static void fill_graph(AttParams& p, const rgbmp_graph_t* g) {
-  p.rowptr = g->rowptr;
-  p.col = g->col;
-  p.row_order = g->row_order;
-  p.n_rows = g->n_rows;
-  const bool split = g->n_items > 0 && g->long_rows && g->long_item_ptr && g->item_long && g->item_start &&
-                     g->chunk > 0 && g->long_chunk > 0;
-  p.chunk = split ? g->chunk : 0;
-  p.long_chunk = g->long_chunk;
-  p.long_rows = g->long_rows;
-  p.long_item_ptr = g->long_item_ptr;
-  p.item_long = g->item_long;
-  p.item_start = g->item_start;
-  p.n_long = split ? g->n_long : 0;
-  p.n_items = split ? g->n_items : 0;
-}
-
-static int check_g(const rgbmp_graph_t* g, const char* fn) {
-  if (!g || !g->rowptr || g->n_rows < 0 || g->nnz < 0 || (g->nnz > 0 && !g->col))
-    return fail(RGBMP_EINVAL, "%s: bad graph descriptor", fn);
-  if (g->col_tagged) return fail(RGBMP_EINVAL, "%s: hot-tagged column ids are not accepted here", fn);
-  return 0;
-}
-
 // scratch of the long-row split: part_m | part_s | part_q [n_items,H] and part_acc | part_acc2 [n_items, ldp]
 static size_t split_bytes(int64_t n_items, int H, int HC) {
   if (n_items <= 0) return 0;
@@ -1029,8 +949,15 @@ static bool carve_split(AttParams& p, Carver& cv, int HC, int64_t n_items) {
   return cv.ok();
 }
 
-#define ATT_G_SWITCH(G_, CALL4, CALL8, CALL16) \
-  switch (G_) { case 4: CALL4; break; case 8: CALL8; break; default: CALL16; break; }
+// Calls f(G) for the lanes per row att_shape chose, G as a std::integral_constant
+template <class F>
+static int with_group(int G, F&& f) {
+  switch (G) {
+    case 4: return f(std::integral_constant<int, 4>());
+    case 8: return f(std::integral_constant<int, 8>());
+    default: return f(std::integral_constant<int, 16>());
+  }
+}
 
 // forward loop variant: 0 = 2 edges per step, software-pipelined (round 1's shape); 1 = 4 edges per step, plain;
 // 2 = 2 edges per step, plain (default).  Measured on the Reddit-shaped 8x8 layer with the ids staged in shared
@@ -1048,22 +975,14 @@ static int att_fwd_variant() {
 
 template <int SC, bool TRAIN, int UU, bool PIPE, bool DR>
 static int launch_fwd_v(const AttParams& p, const Shape& s, cudaStream_t st) {
-  const int HC = p.H * p.C;
-  dim3 grid_rows((unsigned)ceil_div(p.n_rows, ATT_THREADS / s.G), (unsigned)s.tiles);
-  ATT_G_SWITCH(s.G, (att_fwd_rows_kernel<SC, TRAIN, 4, UU, PIPE, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
-               (att_fwd_rows_kernel<SC, TRAIN, 8, UU, PIPE, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
-               (att_fwd_rows_kernel<SC, TRAIN, 16, UU, PIPE, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)))
-  RGBMP_LAUNCH_CHECK("att_fwd_rows_kernel");
-  if (p.n_items > 0) {
-    dim3 grid_items((unsigned)p.n_items, (unsigned)s.tiles);
-    ATT_G_SWITCH(s.G, (att_fwd_long_kernel<SC, TRAIN, 4, UU, PIPE, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
-                 (att_fwd_long_kernel<SC, TRAIN, 8, UU, PIPE, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
-                 (att_fwd_long_kernel<SC, TRAIN, 16, UU, PIPE, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)))
-    RGBMP_LAUNCH_CHECK("att_fwd_long_kernel");
-    att_fwd_combine_kernel<SC, TRAIN><<<(unsigned)ceil_div(p.n_long * HC, 256), 256, 0, st>>>(p);
-    RGBMP_LAUNCH_CHECK("att_fwd_combine_kernel");
-  }
-  return 0;
+  return with_group(s.G, [&](auto g) {
+    constexpr int G = decltype(g)::value;
+    return launch_phases(
+        p.w, ATT_THREADS / G, s.tiles, p.H * p.C, "att_fwd kernels",
+        [&](dim3 grid) { att_fwd_rows_kernel<SC, TRAIN, G, UU, PIPE, DR><<<grid, ATT_THREADS, 0, st>>>(p); },
+        [&](dim3 grid) { att_fwd_long_kernel<SC, TRAIN, G, UU, PIPE, DR><<<grid, ATT_THREADS, 0, st>>>(p); },
+        [&](unsigned blocks) { att_fwd_combine_kernel<SC, TRAIN><<<blocks, 256, 0, st>>>(p); });
+  });
 }
 
 // the fused-dropout and the SD forwards exist in the default loop variant only (SD spills in the other two)
@@ -1082,42 +1001,26 @@ static int launch_fwd(const AttParams& p, const Shape& s, cudaStream_t st) {
 
 template <int SC, bool DR>
 static int launch_bwdT(const AttParams& p, const Shape& s, cudaStream_t st) {
-  const int HC = p.H * p.C;
-  dim3 grid_rows((unsigned)ceil_div(p.n_rows, ATT_THREADS / s.G), (unsigned)s.tiles);
-  ATT_G_SWITCH(s.G, (att_bwdT_rows_kernel<SC, 4, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
-               (att_bwdT_rows_kernel<SC, 8, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
-               (att_bwdT_rows_kernel<SC, 16, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)))
-  RGBMP_LAUNCH_CHECK("att_bwdT_rows_kernel");
-  if (p.n_items > 0) {
-    dim3 grid_items((unsigned)p.n_items, (unsigned)s.tiles);
-    ATT_G_SWITCH(s.G, (att_bwdT_long_kernel<SC, 4, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
-                 (att_bwdT_long_kernel<SC, 8, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
-                 (att_bwdT_long_kernel<SC, 16, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)))
-    RGBMP_LAUNCH_CHECK("att_bwdT_long_kernel");
-    att_bwd_combine_kernel<<<(unsigned)ceil_div(p.n_long * HC, 256), 256, 0, st>>>(p);
-    RGBMP_LAUNCH_CHECK("att_bwd_combine_kernel");
-  }
-  return 0;
+  return with_group(s.G, [&](auto g) {
+    constexpr int G = decltype(g)::value;
+    return launch_phases(
+        p.w, ATT_THREADS / G, s.tiles, p.H * p.C, "att_bwdT kernels",
+        [&](dim3 grid) { att_bwdT_rows_kernel<SC, G, DR><<<grid, ATT_THREADS, 0, st>>>(p); },
+        [&](dim3 grid) { att_bwdT_long_kernel<SC, G, DR><<<grid, ATT_THREADS, 0, st>>>(p); },
+        [&](unsigned blocks) { att_bwd_combine_kernel<<<blocks, 256, 0, st>>>(p); });
+  });
 }
 
 template <int SC, bool DR>
 static int launch_bwdF(const AttParams& p, const Shape& s, cudaStream_t st) {
-  const int HC = p.H * p.C;
-  dim3 grid_rows((unsigned)ceil_div(p.n_rows, ATT_THREADS / s.G), (unsigned)s.tiles);
-  ATT_G_SWITCH(s.G, (att_bwdF_rows_kernel<SC, 4, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
-               (att_bwdF_rows_kernel<SC, 8, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)),
-               (att_bwdF_rows_kernel<SC, 16, DR><<<grid_rows, ATT_THREADS, 0, st>>>(p)))
-  RGBMP_LAUNCH_CHECK("att_bwdF_rows_kernel");
-  if (p.n_items > 0) {
-    dim3 grid_items((unsigned)p.n_items, (unsigned)s.tiles);
-    ATT_G_SWITCH(s.G, (att_bwdF_long_kernel<SC, 4, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
-                 (att_bwdF_long_kernel<SC, 8, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)),
-                 (att_bwdF_long_kernel<SC, 16, DR><<<grid_items, ATT_THREADS, 0, st>>>(p)))
-    RGBMP_LAUNCH_CHECK("att_bwdF_long_kernel");
-    att_bwd_combine_kernel<<<(unsigned)ceil_div(p.n_long * HC, 256), 256, 0, st>>>(p);
-    RGBMP_LAUNCH_CHECK("att_bwd_combine_kernel");
-  }
-  return 0;
+  return with_group(s.G, [&](auto g) {
+    constexpr int G = decltype(g)::value;
+    return launch_phases(
+        p.w, ATT_THREADS / G, s.tiles, p.H * p.C, "att_bwdF kernels",
+        [&](dim3 grid) { att_bwdF_rows_kernel<SC, G, DR><<<grid, ATT_THREADS, 0, st>>>(p); },
+        [&](dim3 grid) { att_bwdF_long_kernel<SC, G, DR><<<grid, ATT_THREADS, 0, st>>>(p); },
+        [&](unsigned blocks) { att_bwd_combine_kernel<<<blocks, 256, 0, st>>>(p); });
+  });
 }
 
 // the scores and shapes the kernels take; FA is single-head
@@ -1169,15 +1072,14 @@ int rgbmp_att_forward(const rgbmp_graph_t* g, int score, const float* X, int64_t
                       float* rowsum, float* out2, int64_t ldo2, float* rowq, void* ws, size_t ws_bytes, int device,
                       void* stream) {
   const char* fn = "rgbmp_att_forward";
-  int rc = check_g(g, fn);
+  const bool sd = score == RGBMP_ATT_SD;                   // X holds the features of both endpoints
+  int rc = check_graph(g, fn, sd ? GRAPH_SQUARE : 0);
   if (rc) return rc;
   Shape s;
   if (!att_ok(score, H, C, &s))
     return fail(RGBMP_ERANGE, "%s: unsupported score %d / H %d / C %d (H == 1 with C <= 128, or C in {8..128} a power of two)",
                 fn, score, H, C);
-  const bool sd = score == RGBMP_ATT_SD;                   // X holds the features of both endpoints
-  if (sd && (g->n_rows != g->n_cols || !isfinite(logit_scale)))
-    return fail(RGBMP_EINVAL, "%s: SD needs a square graph and a finite logit_scale", fn);
+  if (sd && !isfinite(logit_scale)) return fail(RGBMP_EINVAL, "%s: SD needs a finite logit_scale", fn);
   if (drop && d) return fail(RGBMP_EINVAL, "%s: at most one of drop / d", fn);
   if (!X || (!sd && (!a_nbr || !a_own)) || !out || !ws) return fail(RGBMP_EINVAL, "%s: null pointer", fn);
   if (d && (!d->seed || (g->nnz > 0 && !d->eid))) return fail(RGBMP_EINVAL, "%s: dropout needs seed and eid", fn);
@@ -1199,12 +1101,12 @@ int rgbmp_att_forward(const rgbmp_graph_t* g, int score, const float* X, int64_t
   const int64_t n = g->n_rows;
   if (n == 0) return 0;
   AttParams p = {};
-  fill_graph(p, g);
+  p.w = csr_work(g);
   p.H = H; p.HT = s.HT; p.C = C; p.LPH = s.LPH; p.slope = slope; p.logit_scale = logit_scale;
   Carver cv(ws, ws_bytes);
   float* an2 = cv.take<float>((size_t)g->n_cols * H);
   float* ao2 = cv.take<float>((size_t)n * H);
-  if (!carve_split(p, cv, HC, p.n_items) || !cv.ok()) return fail(RGBMP_EWORKSPACE, "%s: workspace carve", fn);
+  if (!carve_split(p, cv, HC, p.w.n_items) || !cv.ok()) return fail(RGBMP_EWORKSPACE, "%s: workspace carve", fn);
   p.Xn = X; p.ldn = ldx; p.Xo = X; p.ldo_ = ldx; p.dinv = dinv; p.drop = drop;
   if (d) set_dropout(p, d, d->eid);
   p.out = out; p.ldo = ldo; p.out2 = out2; p.ldo2 = ldo2; p.rowmax = rowmax; p.rowsum = rowsum; p.rowq = rowq;
@@ -1239,16 +1141,15 @@ int rgbmp_att_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int scor
                        float* dXf, int64_t lddxf, float* da_nbr, float* da_own, void* ws, size_t ws_bytes, int device,
                        void* stream) {
   const char* fn = "rgbmp_att_backward";
-  int rc = check_g(g, fn);
+  const bool sd = score == RGBMP_ATT_SD;
+  int rc = check_graph(g, fn, sd ? GRAPH_SQUARE : 0);
   if (rc) return rc;
-  rc = check_g(gT, fn);
+  rc = check_graph(gT, fn);
   if (rc) return rc;
   Shape s;
   if (!att_ok(score, H, C, &s)) return fail(RGBMP_ERANGE, "%s: unsupported score %d / H %d / C %d", fn, score, H, C);
-  const bool sd = score == RGBMP_ATT_SD;
-  if (sd && (g->n_rows != g->n_cols || gT->n_rows != g->n_cols || gT->n_cols != g->n_rows || gT->nnz != g->nnz ||
-             !isfinite(logit_scale)))
-    return fail(RGBMP_EINVAL, "%s: SD needs a square graph, its transpose and a finite logit_scale", fn);
+  if (sd && (gT->n_rows != g->n_cols || gT->n_cols != g->n_rows || gT->nnz != g->nnz || !isfinite(logit_scale)))
+    return fail(RGBMP_EINVAL, "%s: SD needs the transpose of g and a finite logit_scale", fn);
   if (drop && d) return fail(RGBMP_EINVAL, "%s: at most one of drop / d", fn);
   if (!X || !dout || !dX || (!sd && (!a_nbr || !a_own || !da_nbr || !da_own)) || !ws || (drop && !tpos))
     return fail(RGBMP_EINVAL, "%s: null pointer", fn);
@@ -1275,7 +1176,7 @@ int rgbmp_att_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int scor
   float4* stats = cv.take<float4>((size_t)n_dst * H);
   float* an2 = cv.take<float>((size_t)g->n_cols * H);
   AttParams pt = {};
-  fill_graph(pt, gT);
+  pt.w = csr_work(gT);
   pt.H = H; pt.HT = s.HT; pt.C = C; pt.LPH = s.LPH; pt.slope = slope; pt.logit_scale = logit_scale;
   if (!carve_split(pt, cv, HC, g->n_items > gT->n_items ? g->n_items : gT->n_items) || !cv.ok())
     return fail(RGBMP_EWORKSPACE, "%s: workspace carve", fn);
@@ -1289,7 +1190,7 @@ int rgbmp_att_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, int scor
     if constexpr (SC == SC_MX || SC == SC_SD) {
       // pass F on the forward CSR: dXf_i = sum_j dlogit_ij x_j, da_r[i]
       AttParams pf = pt;
-      fill_graph(pf, g);
+      pf.w = csr_work(g);
       if constexpr (SC == SC_MX) {
         att_scale_kernel<<<(unsigned)ceil_div(g->n_cols * H, 256), 256, 0, st>>>(a_nbr, g->n_cols * H, an2);
         RGBMP_LAUNCH_CHECK("att_scale_kernel");

@@ -5,7 +5,7 @@
 // CSR (all in-edges of one target, or all out-edges of one source for the transpose) is owned by a
 // warp; reductions over a row's edges are sequential per lane + warp shuffles, so results are
 // deterministic.
-#include "common.cuh"
+#include "csr_work.cuh"
 
 namespace rgbmp {
 
@@ -149,14 +149,6 @@ spmm_heads_kernel(const int64_t* __restrict__ rowptr, const int32_t* __restrict_
   }
 }
 
-static int check_g(const rgbmp_graph_t* g, const char* fn) {
-  if (!g || !g->rowptr || g->n_rows < 0 || g->nnz < 0 || (g->nnz > 0 && !g->col))
-    return fail(RGBMP_EINVAL, "%s: bad graph descriptor", fn);
-  return 0;
-}
-
-static inline bool al16(const void* p, int64_t ld) { return (((uintptr_t)p) & 15) == 0 && (ld % 4) == 0; }
-
 }  // namespace rgbmp
 
 using namespace rgbmp;
@@ -178,7 +170,7 @@ int rgbmp_rowdot(const float* A, int64_t lda, const float* B, int64_t ldb, int64
 
 int rgbmp_sddmm(const rgbmp_graph_t* g, const float* A, int64_t lda, const float* B, int64_t ldb, int H, int C,
                 float* out, int device, void* stream) {
-  int rc = check_g(g, "rgbmp_sddmm");
+  int rc = check_graph(g, "rgbmp_sddmm");
   if (rc) return rc;
   if (!A || !B || (g->nnz > 0 && !out) || H <= 0 || C <= 0) return fail(RGBMP_EINVAL, "rgbmp_sddmm: bad argument");
   DeviceGuard dg(device);
@@ -190,7 +182,7 @@ int rgbmp_sddmm(const rgbmp_graph_t* g, const float* A, int64_t lda, const float
 }
 
 int rgbmp_u_add_v(const rgbmp_graph_t* g, const float* u, const float* v, int H, float* out, int device, void* stream) {
-  int rc = check_g(g, "rgbmp_u_add_v");
+  int rc = check_graph(g, "rgbmp_u_add_v");
   if (rc) return rc;
   if (!u || !v || (g->nnz > 0 && !out) || H <= 0) return fail(RGBMP_EINVAL, "rgbmp_u_add_v: bad argument");
   DeviceGuard dg(device);
@@ -202,7 +194,7 @@ int rgbmp_u_add_v(const rgbmp_graph_t* g, const float* u, const float* v, int H,
 }
 
 int rgbmp_seg_softmax(const rgbmp_graph_t* g, const float* in, int H, float* out, int device, void* stream) {
-  int rc = check_g(g, "rgbmp_seg_softmax");
+  int rc = check_graph(g, "rgbmp_seg_softmax");
   if (rc) return rc;
   if ((g->nnz > 0 && (!in || !out)) || H <= 0) return fail(RGBMP_EINVAL, "rgbmp_seg_softmax: bad argument");
   DeviceGuard dg(device);
@@ -215,7 +207,7 @@ int rgbmp_seg_softmax(const rgbmp_graph_t* g, const float* in, int H, float* out
 
 int rgbmp_seg_softmax_backward(const rgbmp_graph_t* g, const float* alpha, const float* dalpha, int H, float* dlogit,
                                int device, void* stream) {
-  int rc = check_g(g, "rgbmp_seg_softmax_backward");
+  int rc = check_graph(g, "rgbmp_seg_softmax_backward");
   if (rc) return rc;
   if ((g->nnz > 0 && (!alpha || !dalpha || !dlogit)) || H <= 0)
     return fail(RGBMP_EINVAL, "rgbmp_seg_softmax_backward: bad argument");
@@ -228,7 +220,7 @@ int rgbmp_seg_softmax_backward(const rgbmp_graph_t* g, const float* alpha, const
 }
 
 int rgbmp_seg_sum(const rgbmp_graph_t* g, const float* in, int H, float* out, int device, void* stream) {
-  int rc = check_g(g, "rgbmp_seg_sum");
+  int rc = check_graph(g, "rgbmp_seg_sum");
   if (rc) return rc;
   if ((g->nnz > 0 && !in) || !out || H <= 0) return fail(RGBMP_EINVAL, "rgbmp_seg_sum: bad argument");
   DeviceGuard dg(device);
@@ -241,7 +233,7 @@ int rgbmp_seg_sum(const rgbmp_graph_t* g, const float* in, int H, float* out, in
 
 int rgbmp_spmm_heads(const rgbmp_graph_t* g, const float* w, const float* X, int64_t ldx, int H, int C, float* out,
                      int64_t ldo, int device, void* stream) {
-  int rc = check_g(g, "rgbmp_spmm_heads");
+  int rc = check_graph(g, "rgbmp_spmm_heads");
   if (rc) return rc;
   if ((g->nnz > 0 && !w) || !X || !out || H <= 0 || C <= 0) return fail(RGBMP_EINVAL, "rgbmp_spmm_heads: bad argument");
   DeviceGuard dg(device);

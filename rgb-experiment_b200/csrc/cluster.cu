@@ -17,7 +17,7 @@
 //      leaves settle first, hubs wait for their own leaves instead of copying a bigger hub across a hub-hub edge;
 //   3. W[a][b] = number of edges from group b into group a; the host orders the groups so that strongly connected
 //      ones are adjacent (graph.py), rows are then sorted by (group rank, -degree) by rgbmp_row_order_grouped.
-#include "common.cuh"
+#include "csr_work.cuh"
 
 namespace rgbmp {
 
@@ -130,9 +130,10 @@ size_t rgbmp_cluster_workspace_bytes(int64_t n_rows) {
 
 int rgbmp_cluster_lpa(const rgbmp_graph_t* g, const int32_t* deg_order, int32_t n_seeds, int iters, const float* taus,
                       int32_t* label, void* ws, size_t ws_bytes, int device, void* stream) {
-  if (!g || !g->rowptr || g->n_rows <= 0 || (g->nnz > 0 && !g->col) || !deg_order || !label || !taus || iters < 1 || !ws)
+  int rc = check_graph(g, "rgbmp_cluster_lpa", GRAPH_SQUARE);
+  if (rc) return rc;
+  if (g->n_rows <= 0 || !deg_order || !label || !taus || iters < 1 || !ws)
     return fail(RGBMP_EINVAL, "rgbmp_cluster_lpa: bad argument");
-  if (g->n_rows != g->n_cols) return fail(RGBMP_EINVAL, "rgbmp_cluster_lpa: needs a square graph");
   if (n_seeds < 1 || n_seeds > 4096 || n_seeds > g->n_rows) return fail(RGBMP_ERANGE, "rgbmp_cluster_lpa: n_seeds must be in 1..min(4096, n_rows)");
   if (ws_bytes < rgbmp_cluster_workspace_bytes(g->n_rows)) return fail(RGBMP_EWORKSPACE, "rgbmp_cluster_lpa: workspace");
   DeviceGuard dg(device);
@@ -165,8 +166,9 @@ int rgbmp_cluster_lpa(const rgbmp_graph_t* g, const int32_t* deg_order, int32_t 
 
 int rgbmp_cluster_connectivity(const rgbmp_graph_t* g, const int32_t* label, int32_t n_groups, int row_stride, uint32_t* W,
                                int device, void* stream) {
-  if (!g || !g->rowptr || g->n_rows <= 0 || (g->nnz > 0 && !g->col) || !label || !W || row_stride < 1)
-    return fail(RGBMP_EINVAL, "rgbmp_cluster_connectivity: bad argument");
+  int rc = check_graph(g, "rgbmp_cluster_connectivity", GRAPH_SQUARE);
+  if (rc) return rc;
+  if (g->n_rows <= 0 || !label || !W || row_stride < 1) return fail(RGBMP_EINVAL, "rgbmp_cluster_connectivity: bad argument");
   if (n_groups < 1 || n_groups > 4096) return fail(RGBMP_ERANGE, "rgbmp_cluster_connectivity: n_groups must be in 1..4096");
   DeviceGuard dg(device);
   if (!dg.ok) return fail(RGBMP_EINVAL, "rgbmp_cluster_connectivity: bad device");

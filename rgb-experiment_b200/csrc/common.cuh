@@ -56,6 +56,8 @@ constexpr int kSMs = 148;  // B200: 2 dies x 74 SMs
 
 inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
+// fp32 rows read as float4: 16-byte aligned base, ld a multiple of 4
+inline bool al16(const void* p, int64_t ld) { return (((uintptr_t)p) & 15) == 0 && (ld % 4) == 0; }
 
 // carve aligned regions out of a caller workspace
 struct Carver {

@@ -71,16 +71,6 @@ static void choose_shape(int nvec, bool hbm_regime, int* G, int* V, int* U) {
   *U = nvec > 2 ? 4 : 20;
 }
 
-static int check_graph(const rgbmp_graph_t* g, const char* fn) {
-  if (!g || !g->rowptr || g->n_rows < 0 || g->nnz < 0 || (g->nnz > 0 && !g->col))
-    return fail(RGBMP_EINVAL, "%s: bad graph descriptor", fn);
-  if (g->n_items > 0 && (!g->long_rows || !g->long_item_ptr || !g->item_long || !g->item_start || g->chunk <= 0 ||
-                         g->long_chunk <= 0))
-    return fail(RGBMP_EINVAL, "%s: incomplete long-row lists", fn);
-  if (g->n_cols >= (1ll << 31)) return fail(RGBMP_ERANGE, "%s: n_cols exceeds int32", fn);
-  return 0;
-}
-
 struct Prepared {
   SpmmParams p;
   int G, V, U, epv;
@@ -89,20 +79,9 @@ struct Prepared {
 static int spmm_prepare(const rgbmp_graph_t* g, const float* val, const void* X, int64_t ldx, void* Y, int64_t ldy, int F,
                         int dtype, const rgbmp_epilogue_t* ep, int tune, void* ws, size_t ws_bytes, Prepared* out) {
   SpmmParams& p = out->p;
-  p.rowptr = g->rowptr;
-  p.col = g->col;
+  p.w = csr_work(g);
   p.val = val;
-  p.row_order = g->row_order;
   p.push_bulk = push_bulk_default();
-  p.n_rows = g->n_rows;
-  p.chunk = g->n_items > 0 ? g->chunk : 0;
-  p.long_chunk = g->long_chunk;
-  p.long_rows = g->long_rows;
-  p.long_item_ptr = g->long_item_ptr;
-  p.item_long = g->item_long;
-  p.item_start = g->item_start;
-  p.n_long = g->n_items > 0 ? g->n_long : 0;
-  p.n_items = g->n_items;
   p.X = X;
   p.ldx = ldx;
   p.Y = Y;
@@ -139,9 +118,9 @@ static int spmm_prepare(const rgbmp_graph_t* g, const float* val, const void* X,
 
   p.partial = nullptr;
   p.ldpart = 0;
-  if (p.n_items > 0) {
+  if (p.w.n_items > 0) {
     p.ldpart = (int64_t)align_up(F, 4);
-    const size_t need = (size_t)p.n_items * p.ldpart * sizeof(float);
+    const size_t need = (size_t)p.w.n_items * p.ldpart * sizeof(float);
     if (!ws || ws_bytes < need) return fail(RGBMP_EWORKSPACE, "rgbmp_spmm: workspace %zu < %zu", ws_bytes, need);
     p.partial = (float*)ws;
   }
@@ -205,7 +184,7 @@ int rgbmp_set_push_bulk(int on) {
 
 int rgbmp_spmm(const rgbmp_graph_t* g, const float* val, const void* X, int64_t ldx, void* Y, int64_t ldy, int F,
                int dtype, const rgbmp_epilogue_t* ep, int tune, void* ws, size_t ws_bytes, int device, void* stream) {
-  int rc = check_graph(g, "rgbmp_spmm");
+  int rc = check_graph(g, "rgbmp_spmm", GRAPH_TAGS_OK);
   if (rc) return rc;
   if (!X || F <= 0 || ldx < F || (Y && ldy < F)) return fail(RGBMP_EINVAL, "rgbmp_spmm: bad feature arguments");
   if (dtype != RGBMP_F32 && dtype != RGBMP_BF16) return fail(RGBMP_EINVAL, "rgbmp_spmm: bad dtype %d", dtype);
@@ -217,7 +196,7 @@ int rgbmp_spmm(const rgbmp_graph_t* g, const float* val, const void* X, int64_t 
 int rgbmp_khop(const rgbmp_graph_t* g, const float* val, const void* X0, int64_t ldx0, void* ping, void* pong,
                int64_t ldp, void* out, int64_t ldo, void* hops, int64_t ld_hops, int64_t hop_stride, int F, int dtype,
                int K, const rgbmp_epilogue_t* ep, int tune, void* ws, size_t ws_bytes, int device, void* stream) {
-  int rc = check_graph(g, "rgbmp_khop");
+  int rc = check_graph(g, "rgbmp_khop", GRAPH_TAGS_OK | GRAPH_SQUARE);
   if (rc) return rc;
   if (!X0 || (!out && !hops) || F <= 0 || K < 1 || ldx0 < F || (out && ldo < F))
     return fail(RGBMP_EINVAL, "rgbmp_khop: bad arguments");
@@ -226,7 +205,6 @@ int rgbmp_khop(const rgbmp_graph_t* g, const float* val, const void* X0, int64_t
     if (!through_hops) return fail(RGBMP_EINVAL, "rgbmp_khop: K > 1 needs ping/pong buffers");
   }
   if (dtype != RGBMP_F32 && dtype != RGBMP_BF16) return fail(RGBMP_EINVAL, "rgbmp_khop: bad dtype %d", dtype);
-  if (g->n_rows != g->n_cols) return fail(RGBMP_EINVAL, "rgbmp_khop: needs a square graph");
   DeviceGuard dg(device);
   if (!dg.ok) return fail(RGBMP_EINVAL, "rgbmp_khop: bad device %d", device);
   cudaStream_t st = (cudaStream_t)stream;
@@ -352,7 +330,7 @@ int rgbmp_stage_rows(const float* X, int64_t ldx, const float* scale, float* Z0,
 int rgbmp_appnp_host(const rgbmp_graph_t* g, const float* dinv, const float* z0_host, float* out_host, int F, int K,
                      float alpha, float* dev_z0, float* dev_ping, float* dev_pong, float* dev_out, int64_t ld, void* ws,
                      size_t ws_bytes, int device, void* stream) {
-  int rc = check_graph(g, "rgbmp_appnp_host");
+  int rc = check_graph(g, "rgbmp_appnp_host", GRAPH_TAGS_OK | GRAPH_SQUARE);
   if (rc) return rc;
   if (!dinv || !z0_host || !out_host || !dev_z0 || !dev_ping || !dev_pong || !dev_out || F <= 0 || K < 1 || ld < F)
     return fail(RGBMP_EINVAL, "rgbmp_appnp_host: bad argument");

@@ -15,25 +15,13 @@
 //   * the epilogue (row scale, teleport, clamp, reset rows, pre-scaled second output) is applied
 //     in registers before the single store of the row.
 #pragma once
-#include "common.cuh"
+#include "csr_work.cuh"
 
 namespace rgbmp {
 
 struct SpmmParams {
-  // graph
-  const int64_t* rowptr;
-  const int32_t* col;
+  CsrWork w;
   const float* val;
-  const int32_t* row_order;  // nullable: schedule of the short-row kernel
-  int64_t n_rows;
-  int32_t chunk;
-  // long rows
-  int32_t long_chunk;
-  const int32_t* long_rows;
-  const int32_t* long_item_ptr;
-  const int32_t* item_long;
-  const int64_t* item_start;
-  int64_t n_long, n_items;
   float* partial;  // [n_items, ldpart]
   int64_t ldpart;
   // features
@@ -232,22 +220,6 @@ struct IdStage {
 };
 
 template <int N>
-__device__ __forceinline__ void lds_ids(const int32_t* p, uint32_t (&c)[N]) {
-  if constexpr (N == 8) {
-    const int4 v = *reinterpret_cast<const int4*>(p), w = *reinterpret_cast<const int4*>(p + 4);
-    c[0] = v.x; c[1] = v.y; c[2] = v.z; c[3] = v.w; c[4] = w.x; c[5] = w.y; c[6] = w.z; c[7] = w.w;
-  } else if constexpr (N == 4) {
-    const int4 v = *reinterpret_cast<const int4*>(p);
-    c[0] = v.x; c[1] = v.y; c[2] = v.z; c[3] = v.w;
-  } else if constexpr (N == 2) {
-    const int2 v = *reinterpret_cast<const int2*>(p);
-    c[0] = v.x; c[1] = v.y;
-  } else {
-#pragma unroll
-    for (int i = 0; i < N; ++i) c[i] = p[i];
-  }
-}
-template <int N>
 __device__ __forceinline__ void lds_wts(const float* p, float (&w)[N]) {
   if constexpr (N == 8) {
     const float4 v = *reinterpret_cast<const float4*>(p), x = *reinterpret_cast<const float4*>(p + 4);
@@ -279,7 +251,7 @@ __device__ __forceinline__ void accumulate_range(const SpmmParams& p, int64_t k0
   constexpr int UE = (U < G) ? U : G;   // edges per inner step (a batch holds G ids)
   const uint32_t row_bytes = (uint32_t)(p.ldx * (int64_t)sizeof(T));
   const uint64_t pol_hot = make_policy(p.pol_hot), pol_cold = make_policy(p.pol_cold);
-  const int32_t* __restrict__ col = p.col + k0;
+  const int32_t* __restrict__ col = p.w.col + k0;
   const float* __restrict__ val = HASW ? p.val + k0 : nullptr;
   const int len = (k1 > k0) ? (int)(k1 - k0) : 0;          // <= chunk / long sub-range, fits int
   const int maxlen = __reduce_max_sync(FULL, len);
@@ -461,17 +433,9 @@ __device__ __forceinline__ void lane_bases(const SpmmParams& p, int f0, const ch
 // groups sharing a warp run rows of equal length -- no idle issue slots from divergent trip counts.
 template <typename T, int EPV, int G, int V, int U, bool HASW, bool PIPE>
 __global__ void __launch_bounds__(SPMM_THREADS, spmm_minb<EPV, V, U, PIPE>()) spmm_rows_kernel(const SpmmParams p) {
-  constexpr int GPB = SPMM_THREADS / G;
   const int gl = threadIdx.x % G;
-  const int64_t gid = (int64_t)blockIdx.x * GPB + threadIdx.x / G;
-  int64_t row = -1, k0 = 0, k1 = 0;
-  if (gid < p.n_rows) {
-    row = p.row_order ? (int64_t)__ldg(p.row_order + gid) : gid;
-    k0 = __ldg(p.rowptr + row);
-    k1 = __ldg(p.rowptr + row + 1);
-    if (p.chunk > 0 && k1 - k0 > p.chunk) row = -1;  // long row: handled by spmm_long_kernel
-  }
-  if (row < 0) k1 = k0;                               // idle group: stays in the warp-uniform loop with no edges
+  int64_t row, k0, k1;
+  short_row<G, SPMM_THREADS>(p.w, row, k0, k1);
   const int f0 = blockIdx.y * (G * V * EPV) + gl * EPV;
   const char* xb[V];
   bool active[V];
@@ -531,16 +495,8 @@ __global__ void __launch_bounds__(SPMM_THREADS, spmm_minb<EPV, V, U, PIPE>()) sp
   extern __shared__ float sm[];            // [Q][W]
   const int gl = threadIdx.x % G, q = threadIdx.x / G;
   const int64_t item = blockIdx.x;
-  const int32_t slot = p.item_long[item];
-  const int64_t row = p.long_rows[slot];
-  const int64_t rs = p.item_start[item];
-  const int64_t rend = __ldg(p.rowptr + row + 1);
-  const int64_t re = (rs + p.long_chunk < rend) ? rs + p.long_chunk : rend;
-  const int64_t len = re - rs;
-  const int64_t per = (len + Q - 1) / Q;
-  int64_t k0 = rs + (int64_t)q * per, k1 = k0 + per;
-  if (k0 > re) k0 = re;
-  if (k1 > re) k1 = re;
+  int64_t row, k0, k1;
+  long_item<G, SPMM_THREADS>(p.w, row, k0, k1);
   const int ftile = blockIdx.y * W;
   const int f0 = ftile + gl * EPV;
   const char* xb[V];
@@ -574,10 +530,10 @@ __global__ void __launch_bounds__(256) spmm_combine_kernel(const SpmmParams p) {
   const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t slot = t / p.F;
   const int f = (int)(t - slot * p.F);
-  if (slot >= p.n_long) return;
-  const int64_t row = p.long_rows[slot];
+  if (slot >= p.w.n_long) return;
+  const int64_t row = p.w.long_rows[slot];
   float s[1] = {0.f};
-  for (int32_t it = p.long_item_ptr[slot]; it < p.long_item_ptr[slot + 1]; ++it)
+  for (int32_t it = p.w.long_item_ptr[slot]; it < p.w.long_item_ptr[slot + 1]; ++it)
     s[0] = __fadd_rn(s[0], p.partial[(int64_t)it * p.ldpart + f]);
   epilogue_store<T, 1>(p, row, f, s);
 }
@@ -603,23 +559,14 @@ row_scale_kernel(const T* __restrict__ X, int64_t ldx, const float* __restrict__
 template <typename T, int EPV, int G, int V, int U, bool HASW, bool PIPE>
 int launch_cfg(const SpmmParams& p, cudaStream_t st) {
   constexpr int W = G * V * EPV;
-  const unsigned ytiles = (unsigned)ceil_div(p.F, W);
-  constexpr int GPB = SPMM_THREADS / G;
-  if (p.n_rows > 0) {
-    dim3 grid((unsigned)ceil_div(p.n_rows, GPB), ytiles);
-    const size_t push_smem = (EPV > 1 && p.push_bulk && p.ep.n_peers > 0) ? (size_t)SPMM_THREADS * V * 16 : 0;
-    spmm_rows_kernel<T, EPV, G, V, U, HASW, PIPE><<<grid, SPMM_THREADS, push_smem, st>>>(p);
-    RGBMP_LAUNCH_CHECK("spmm_rows_kernel");
-  }
-  if (p.n_items > 0) {
-    constexpr int Q = SPMM_THREADS / G;
-    dim3 grid((unsigned)p.n_items, ytiles);
-    spmm_long_kernel<T, EPV, G, V, U, HASW, PIPE><<<grid, SPMM_THREADS, Q * W * sizeof(float), st>>>(p);
-    RGBMP_LAUNCH_CHECK("spmm_long_kernel");
-    spmm_combine_kernel<T><<<(unsigned)ceil_div(p.n_long * p.F, 256), 256, 0, st>>>(p);
-    RGBMP_LAUNCH_CHECK("spmm_combine_kernel");
-  }
-  return 0;
+  const size_t push_smem = (EPV > 1 && p.push_bulk && p.ep.n_peers > 0) ? (size_t)SPMM_THREADS * V * 16 : 0;
+  return launch_phases(
+      p.w, SPMM_THREADS / G, (unsigned)ceil_div(p.F, W), p.F, "spmm kernels",
+      [&](dim3 grid) { spmm_rows_kernel<T, EPV, G, V, U, HASW, PIPE><<<grid, SPMM_THREADS, push_smem, st>>>(p); },
+      [&](dim3 grid) {
+        spmm_long_kernel<T, EPV, G, V, U, HASW, PIPE><<<grid, SPMM_THREADS, (SPMM_THREADS / G) * W * sizeof(float), st>>>(p);
+      },
+      [&](unsigned blocks) { spmm_combine_kernel<T><<<blocks, 256, 0, st>>>(p); });
 }
 
 template <typename T, int EPV, int G, int V, int U, bool PIPE>

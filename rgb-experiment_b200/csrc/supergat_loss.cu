@@ -12,7 +12,7 @@
 // per-row fp32 partials which a fixed-shape two-stage fp64 reduction turns into the scalar; the backward is one pass
 // over target rows (forward CSR + negatives' CSR) that writes dx' and one over source rows (transpose CSRs) that adds
 // into its own rows.  No atomics anywhere: every result is bit-reproducible.
-#include "common.cuh"
+#include "csr_work.cuh"
 #include "philox.cuh"
 
 namespace rgbmp {
@@ -361,8 +361,8 @@ void choose_groups(int nvec, int* G, int* V) {
 }
 
 int check_rows(const rgbmp_graph_t* g, int64_t n, const char* fn, const char* what) {
-  if (!g || !g->rowptr || g->n_rows != n || g->nnz < 0 || (g->nnz > 0 && !g->col))
-    return fail(RGBMP_EINVAL, "%s: bad %s descriptor (rows must equal the node count)", fn, what);
+  if (int rc = check_graph(g, fn)) return rc;
+  if (g->n_rows != n) return fail(RGBMP_EINVAL, "%s: bad %s descriptor (rows must equal the node count)", fn, what);
   return 0;
 }
 
@@ -469,10 +469,10 @@ int rgbmp_sgat_loss_forward(const rgbmp_graph_t* g, const rgbmp_graph_t* gneg, c
                             const float* X, int64_t ldx, int F, float scale, float* loss, int64_t* npairs,
                             void* ws, size_t ws_bytes, int device, void* stream) {
   const char* fn = "rgbmp_sgat_loss_forward";
-  if (!g) return fail(RGBMP_EINVAL, "%s: graph is NULL", fn);
+  int rc = check_graph(g, fn);
+  if (rc) return rc;
   const int64_t n = g->n_rows;
-  int rc;
-  if ((rc = check_rows(g, n, fn, "graph")) || (rc = check_rows(gneg, n, fn, "negatives")) ||
+  if ((rc = check_rows(gneg, n, fn, "negatives")) ||
       (rc = check_features(X, ldx, F, fn)) || (rc = check_sample(s, false, fn)))
     return rc;
   if (!loss || !npairs || !ws) return fail(RGBMP_EINVAL, "%s: NULL output or workspace", fn);
@@ -511,10 +511,10 @@ int rgbmp_sgat_loss_backward(const rgbmp_graph_t* g, const rgbmp_graph_t* gT, co
                              float scale, const int64_t* npairs, const float* dloss, float* dX, int64_t lddx,
                              int device, void* stream) {
   const char* fn = "rgbmp_sgat_loss_backward";
-  if (!g) return fail(RGBMP_EINVAL, "%s: graph is NULL", fn);
+  int rc = check_graph(g, fn);
+  if (rc) return rc;
   const int64_t n = g->n_rows;
-  int rc;
-  if ((rc = check_rows(g, n, fn, "graph")) || (rc = check_rows(gT, n, fn, "transpose graph")) ||
+  if ((rc = check_rows(gT, n, fn, "transpose graph")) ||
       (rc = check_rows(gneg, n, fn, "negatives")) || (rc = check_rows(gnegT, n, fn, "negatives' transpose")) ||
       (rc = check_features(X, ldx, F, fn)) || (rc = check_sample(s, true, fn)))
     return rc;
