@@ -187,7 +187,8 @@ typedef struct rgbmp_graph {
  *                                                                    PTA pta.py:83, LP A15)
  *   if clamp: v = min(max(v,lo),hi)                                  (C&S post_step, A15)
  *   if reset_when==2 and reset_mask[i]: v = reset_val[i,:]           (C&S autoscale=False)
- *   Y[i,:] = v (if Y) ;  Y2[i,:] = out2_scale[i]*v (if Y2)           (pre-scaled copy for the next hop)
+ *   Y[row_map ? row_map[i] : i,:] = v (if Y)                         (row_map: the graph's nodes are renamed)
+ *   Y2[i,:] = out2_scale[i]*v (if Y2)                                (pre-scaled copy for the next hop)
  *   peer_out[q][peer_row0+i,:] = out2_scale ? out2_scale[i]*v : v    (fused all-gather, see below)
  */
 #define RGBMP_MAX_PEERS 8
@@ -219,6 +220,11 @@ typedef struct rgbmp_epilogue {
   int32_t        n_peers;
   int64_t        peer_row0;
   int64_t        ld_peer;
+  /* optional int32 [n_rows]: row i of the graph is row row_map[i] of Y.  A graph whose nodes are renamed in schedule
+   * order stores its result under the original names this way; only the Y store is redirected (Y2, T, row_scale
+   * and out2_scale stay indexed by i).  Not accepted with peers, acc_in or reset rows; rgbmp_khop applies it to
+   * the last hop only and rejects it with `hops`. */
+  const int32_t* row_map;
 } rgbmp_epilogue_t;
 
 /* CSR SpMM  Y[i,:] = epilogue( sum_k val[k] * X[col[k],:] ), k in rowptr[i]..rowptr[i+1].
@@ -292,10 +298,12 @@ int rgbmp_cluster_lpa(const rgbmp_graph_t* g, const int32_t* deg_order, int32_t 
 int rgbmp_cluster_connectivity(const rgbmp_graph_t* g, const int32_t* label, int32_t n_groups, int row_stride,
                                uint32_t* W, int device, void* stream);
 
-/* One pass that prepares a folded K-hop call from an unpadded input: Z0[i, 0:ld] = X[i, 0:F] zero-padded to the
- * 16-byte aligned leading dimension ld (the teleport term) and U0[i,:] = scale[i] * Z0[i,:] (what hop 1 gathers). fp32. */
-int rgbmp_stage_rows(const float* X, int64_t ldx, const float* scale, float* Z0, float* U0, int64_t ld,
-                     int64_t n_rows, int F, int device, void* stream);
+/* One pass that prepares a folded K-hop call from an unpadded input: Z0[i, 0:ld] = X[s, 0:F] zero-padded to the
+ * 16-byte aligned leading dimension ld (the teleport term) and U0[i,:] = scale[i] * Z0[i,:] (what hop 1 gathers),
+ * with s = src_map ? src_map[i] : i (src_map renames the input into a renamed graph's node order).  Z0 may be NULL
+ * when no teleport term is needed.  fp32. */
+int rgbmp_stage_rows(const float* X, int64_t ldx, const int32_t* src_map, const float* scale, float* Z0, float* U0,
+                     int64_t ld, int64_t n_rows, int F, int device, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * (b2) peer memory for the row-partitioned multi-GPU path (one process per GPU, NVLink P2P)
@@ -474,6 +482,13 @@ int rgbmp_appnp_host(const rgbmp_graph_t* g, const float* dinv,
                      const float* z0_host, float* out_host, int F, int K, float alpha,
                      float* dev_z0, float* dev_ping, float* dev_pong, float* dev_out, int64_t ld,
                      void* ws, size_t ws_bytes, int device, void* stream);
+/* The same on a graph whose nodes are renamed: row i of g (and dinv[i]) is node row_map[i] of z0_host and out_host
+ * (int32 [n_rows], device).  The staging pass reads the input in the renamed order and the last hop stores the result
+ * under the original names, so the hops read and write their rows in order.  row_map = NULL: rgbmp_appnp_host. */
+int rgbmp_appnp_host_mapped(const rgbmp_graph_t* g, const int32_t* row_map, const float* dinv,
+                            const float* z0_host, float* out_host, int F, int K, float alpha,
+                            float* dev_z0, float* dev_ping, float* dev_pong, float* dev_out, int64_t ld,
+                            void* ws, size_t ws_bytes, int device, void* stream);
 
 #if defined(__GNUC__)
 #pragma GCC visibility pop

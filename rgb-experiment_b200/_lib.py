@@ -29,7 +29,8 @@ class Epilogue(C.Structure):
                 ("ld_reset", c_i64), ("reset_when", c_i32), ("a", c_f32), ("b", c_f32), ("T", c_vp),
                 ("ldt", c_i64), ("clamp", c_i32), ("lo", c_f32), ("hi", c_f32), ("out2_scale", c_vp),
                 ("Y2", c_vp), ("ldy2", c_i64), ("acc_in", c_vp), ("ld_acc", c_i64), ("skip_empty", c_i32),
-                ("peer_out", c_vp * 8), ("n_peers", c_i32), ("peer_row0", c_i64), ("ld_peer", c_i64)]
+                ("peer_out", c_vp * 8), ("n_peers", c_i32), ("peer_row0", c_i64), ("ld_peer", c_i64),
+                ("row_map", c_vp)]
 
 
 class DropoutStruct(C.Structure):
@@ -88,9 +89,11 @@ def lib():
         "rgbmp_khop": (C.c_int, [GP, c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_i64, C.c_int,
                                  C.c_int, C.c_int, EP, C.c_int, c_vp, c_sz, C.c_int, c_vp]),
         "rgbmp_row_scale": (C.c_int, [c_vp, c_i64, c_vp, C.c_int, c_vp, c_i64, c_i64, C.c_int, C.c_int, C.c_int, c_vp]),
-        "rgbmp_stage_rows": (C.c_int, [c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_i64, C.c_int, C.c_int, c_vp]),
+        "rgbmp_stage_rows": (C.c_int, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, C.c_int, C.c_int, c_vp]),
         "rgbmp_appnp_host": (C.c_int, [GP, c_vp, c_vp, c_vp, C.c_int, C.c_int, c_f32, c_vp, c_vp, c_vp, c_vp, c_i64,
                                        c_vp, c_sz, C.c_int, c_vp]),
+        "rgbmp_appnp_host_mapped": (C.c_int, [GP, c_vp, c_vp, c_vp, c_vp, C.c_int, C.c_int, c_f32, c_vp, c_vp, c_vp, c_vp,
+                                              c_i64, c_vp, c_sz, C.c_int, c_vp]),
     }
     optional = {
         "rgbmp_att_supported": (C.c_int, [C.c_int, C.c_int, C.c_int]),

@@ -448,14 +448,14 @@ static int kc_launch(const KhopCtaParams& p, cudaStream_t st, int device) {
 
 // *handled = 1 when the call was taken (return value = its status), 0 = not eligible: the caller runs the K-launch path.
 // Eligible: fp32, 16-byte aligned padded rows everywhere, at most KC_MAX_GATHER_BYTES gathered per hop and KC_MAX_ROWS
-// rows, rows of at most 4 vectors (KC_MAX_LD), K >= 2, no peer / partial-sum / skip-empty epilogue, no hot tags.
+// rows, rows of at most 4 vectors (KC_MAX_LD), K >= 2, no peer / partial-sum / skip-empty / row-map epilogue, no hot tags.
 int khop_cta_try(const rgbmp_graph_t* g, const float* val, const void* X0, int64_t ldx0, void* ping, void* pong, int64_t ldp,
                  void* out, int64_t ldo, void* hops, int64_t ld_hops, int64_t hop_stride, int F, int dtype, int K,
                  const rgbmp_epilogue_t* ep, cudaStream_t st, int device, int* handled) {
   *handled = 0;
   const int on = g_kc_override >= 0 ? g_kc_override : kc_enabled();
   if (!on || dtype != RGBMP_F32 || g->col_tagged || g->n_rows < 1 || g->n_rows > KC_MAX_ROWS || g->nnz >= (1ll << 30)) return 0;
-  if (ep && (ep->n_peers > 0 || ep->acc_in || ep->skip_empty || ep->Y2)) return 0;
+  if (ep && (ep->n_peers > 0 || ep->acc_in || ep->skip_empty || ep->Y2 || ep->row_map)) return 0;
   const int ld = (int)align_up((size_t)F, 4);
   if (ld > KC_MAX_LD || K < 2) return 0;
   if ((double)g->nnz * ld * 4.0 > KC_MAX_GATHER_BYTES) return 0;

@@ -9,17 +9,18 @@ int khop_cta_try(const rgbmp_graph_t* g, const float* val, const void* X0, int64
                  void* out, int64_t ldo, void* hops, int64_t ld_hops, int64_t hop_stride, int F, int dtype, int K,
                  const rgbmp_epilogue_t* ep, cudaStream_t st, int device, int* handled);   // khop_cta.cu
 
-// packed [n,F] -> pitched z0 [n,ld] and u0 = scale*z0 [n,ld]  (host entry point staging)
+// packed [n,F] -> pitched z0 [n,ld] (optional) and u0 = scale*z0 [n,ld]; row r reads X row src_map[r] when mapped
 __global__ void __launch_bounds__(256)
-stage_rows_kernel(const float* __restrict__ X, int64_t ldx, const float* __restrict__ scale, float* __restrict__ Z0,
-                  float* __restrict__ U0, int64_t ld, int64_t n_rows, int F) {
+stage_rows_kernel(const float* __restrict__ X, int64_t ldx, const int32_t* __restrict__ src_map, const float* __restrict__ scale,
+                  float* __restrict__ Z0, float* __restrict__ U0, int64_t ld, int64_t n_rows, int F) {
   const int64_t total = n_rows * ld;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += stride) {
     const int64_t r = t / ld;
     const int f = (int)(t - r * ld);
-    const float v = (f < F) ? X[r * ldx + f] : 0.f;
-    Z0[t] = v;
+    const int64_t sr = src_map ? (int64_t)src_map[r] : r;
+    const float v = (f < F) ? X[sr * ldx + f] : 0.f;
+    if (Z0) Z0[t] = v;
     U0[t] = __fmul_rn(scale[r], v);
   }
 }
@@ -98,6 +99,8 @@ static int spmm_prepare(const rgbmp_graph_t* g, const float* val, const void* X,
     return fail(RGBMP_EINVAL, "rgbmp_spmm: reset_when set without reset_mask/reset_val");
   if (p.ep.Y2 && !p.ep.out2_scale) return fail(RGBMP_EINVAL, "rgbmp_spmm: Y2 without out2_scale");
   if (!Y && !p.ep.Y2 && p.ep.n_peers <= 0) return fail(RGBMP_EINVAL, "rgbmp_spmm: no output");
+  if (p.ep.row_map && (p.ep.n_peers > 0 || p.ep.acc_in || p.ep.reset_when != 0))
+    return fail(RGBMP_EINVAL, "rgbmp_spmm: row_map does not combine with peers, acc_in or reset rows");
   if (p.ep.n_peers < 0 || p.ep.n_peers > RGBMP_MAX_PEERS) return fail(RGBMP_EINVAL, "rgbmp_spmm: bad n_peers");
   for (int q = 0; q < p.ep.n_peers; ++q)
     if (!p.ep.peer_out[q]) return fail(RGBMP_EINVAL, "rgbmp_spmm: null peer buffer %d", q);
@@ -205,6 +208,7 @@ int rgbmp_khop(const rgbmp_graph_t* g, const float* val, const void* X0, int64_t
     if (!through_hops) return fail(RGBMP_EINVAL, "rgbmp_khop: K > 1 needs ping/pong buffers");
   }
   if (dtype != RGBMP_F32 && dtype != RGBMP_BF16) return fail(RGBMP_EINVAL, "rgbmp_khop: bad dtype %d", dtype);
+  if (ep && ep->row_map && hops) return fail(RGBMP_EINVAL, "rgbmp_khop: row_map does not combine with hops");
   DeviceGuard dg(device);
   if (!dg.ok) return fail(RGBMP_EINVAL, "rgbmp_khop: bad device %d", device);
   cudaStream_t st = (cudaStream_t)stream;
@@ -227,6 +231,7 @@ int rgbmp_khop(const rgbmp_graph_t* g, const float* val, const void* X0, int64_t
     void* y = nullptr;
     int64_t ldy = 0;
     rgbmp_epilogue_t ek = e;
+    ek.row_map = last ? e.row_map : nullptr;     // the iterate stays in the graph's own naming until the last store
     if (hops) { y = (char*)hops + (size_t)k * hop_stride * esz; ldy = ld_hops; }
     if (last && !hops) { y = out; ldy = ldo; }
     if (folded) {
@@ -316,13 +321,13 @@ int rgbmp_row_scale(const void* X, int64_t ldx, const float* scale, int divide, 
   return 0;
 }
 
-int rgbmp_stage_rows(const float* X, int64_t ldx, const float* scale, float* Z0, float* U0, int64_t ld, int64_t n_rows, int F,
-                     int device, void* stream) {
-  if (!X || !scale || !Z0 || !U0 || n_rows < 0 || F <= 0 || ldx < F || ld < F) return fail(RGBMP_EINVAL, "rgbmp_stage_rows: bad argument");
+int rgbmp_stage_rows(const float* X, int64_t ldx, const int32_t* src_map, const float* scale, float* Z0, float* U0, int64_t ld,
+                     int64_t n_rows, int F, int device, void* stream) {
+  if (!X || !scale || !U0 || n_rows < 0 || F <= 0 || ldx < F || ld < F) return fail(RGBMP_EINVAL, "rgbmp_stage_rows: bad argument");
   DeviceGuard dg(device);
   if (!dg.ok) return fail(RGBMP_EINVAL, "rgbmp_stage_rows: bad device");
   if (n_rows == 0) return 0;
-  stage_rows_kernel<<<kSMs * 8, 256, 0, (cudaStream_t)stream>>>(X, ldx, scale, Z0, U0, ld, n_rows, F);
+  stage_rows_kernel<<<kSMs * 8, 256, 0, (cudaStream_t)stream>>>(X, ldx, src_map, scale, Z0, U0, ld, n_rows, F);
   RGBMP_LAUNCH_CHECK("stage_rows_kernel");
   return 0;
 }
@@ -330,6 +335,13 @@ int rgbmp_stage_rows(const float* X, int64_t ldx, const float* scale, float* Z0,
 int rgbmp_appnp_host(const rgbmp_graph_t* g, const float* dinv, const float* z0_host, float* out_host, int F, int K,
                      float alpha, float* dev_z0, float* dev_ping, float* dev_pong, float* dev_out, int64_t ld, void* ws,
                      size_t ws_bytes, int device, void* stream) {
+  return rgbmp_appnp_host_mapped(g, nullptr, dinv, z0_host, out_host, F, K, alpha, dev_z0, dev_ping, dev_pong, dev_out, ld, ws,
+                                 ws_bytes, device, stream);
+}
+
+int rgbmp_appnp_host_mapped(const rgbmp_graph_t* g, const int32_t* row_map, const float* dinv, const float* z0_host,
+                            float* out_host, int F, int K, float alpha, float* dev_z0, float* dev_ping, float* dev_pong,
+                            float* dev_out, int64_t ld, void* ws, size_t ws_bytes, int device, void* stream) {
   int rc = check_graph(g, "rgbmp_appnp_host", GRAPH_TAGS_OK | GRAPH_SQUARE);
   if (rc) return rc;
   if (!dinv || !z0_host || !out_host || !dev_z0 || !dev_ping || !dev_pong || !dev_out || F <= 0 || K < 1 || ld < F)
@@ -340,10 +352,10 @@ int rgbmp_appnp_host(const rgbmp_graph_t* g, const float* dinv, const float* z0_
   const int64_t N = g->n_rows;
   // One contiguous H2D at full PCIe rate into dev_out (used as the packed [N,F] staging area; a
   // pitched 2-D copy of 188-byte rows runs ~15x slower), then one kernel re-pitches to ld and
-  // writes both z0 and u0 = D^-1/2 z0.
+  // writes both z0 and u0 = D^-1/2 z0 (in the graph's node order when it is renamed).
   float* stage = dev_out;
   RGBMP_CUDA(cudaMemcpyAsync(stage, z0_host, (size_t)N * F * sizeof(float), cudaMemcpyHostToDevice, st));
-  stage_rows_kernel<<<kSMs * 8, 256, 0, st>>>(stage, F, dinv, dev_z0, dev_pong, ld, N, F);
+  stage_rows_kernel<<<kSMs * 8, 256, 0, st>>>(stage, F, row_map, dinv, dev_z0, dev_pong, ld, N, F);
   RGBMP_LAUNCH_CHECK("stage_rows_kernel");
   rgbmp_epilogue_t e = {};
   e.row_scale = dinv;
@@ -352,6 +364,7 @@ int rgbmp_appnp_host(const rgbmp_graph_t* g, const float* dinv, const float* z0_
   e.T = dev_z0;
   e.ldt = ld;
   e.out2_scale = dinv;
+  e.row_map = row_map;
   // hop 1 reads u0 from pong and writes ping; the last hop writes the unscaled result to dev_out
   rc = rgbmp_khop(g, nullptr, dev_pong, ld, dev_ping, dev_pong, ld, dev_out, ld, nullptr, 0, 0, F, RGBMP_F32, K, &e, 0, ws,
                   ws_bytes, device, stream);

@@ -391,7 +391,10 @@ __device__ __forceinline__ void epilogue_store(const SpmmParams& p, int64_t row,
     if (reset && ep.reset_when == 2) v = rv[i];
     s[i] = v;
   }
-  if (p.Y) Raw<T, EPV>::store(reinterpret_cast<T*>(p.Y) + row * p.ldy + f, s, p.stream);
+  if (p.Y) {
+    const int64_t yrow = ep.row_map ? (int64_t)__ldg(ep.row_map + row) : row;
+    Raw<T, EPV>::store(reinterpret_cast<T*>(p.Y) + yrow * p.ldy + f, s, p.stream);
+  }
   if (ep.out2_scale) {                     // pre-scaled copy (folded D^-1/2): what the NEXT hop gathers
     const float s2 = __ldg(ep.out2_scale + row);
 #pragma unroll

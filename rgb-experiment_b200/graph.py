@@ -61,7 +61,7 @@ class CSR:
 
     def __init__(self, key: torch.Tensor, other: torch.Tensor, n_rows: int, n_cols: int,
                  chunk: Optional[int] = None, long_chunk: Optional[int] = None, window: Optional[int] = None,
-                 groups=None, finish: bool = True):
+                 groups=None, finish: bool = True, named: bool = False):
         L = lib()
         dev = key.device
         st = stream_of(dev)
@@ -76,7 +76,7 @@ class CSR:
                                 ptr(ws), ws.numel(), dev.index, st), "csr_build")
         self.col, self.eid = self.col[:nnz], self.eid[:nnz]
         if finish:
-            self._finish(chunk, long_chunk, window, groups)
+            self._finish(chunk, long_chunk, window, groups, named=named)
 
     @classmethod
     def from_arrays(cls, rowptr: torch.Tensor, col: torch.Tensor, n_cols: int, chunk: Optional[int] = None,
@@ -103,9 +103,12 @@ class CSR:
                                 self.device.index, stream_of(self.device)), "row_order")
         return order
 
-    def _finish(self, chunk: int, long_chunk: int, window: Optional[int], groups=None, deg_order=None):
+    def _finish(self, chunk: int, long_chunk: int, window: Optional[int], groups=None, deg_order=None,
+                named: bool = False):
         """Row schedule, long-row work lists, descriptor.  groups = (group int32 [n_rows], n_groups): schedule by
-        (group, -degree) and list the long rows in that order too (locality groups, see Graph)."""
+        (group, -degree) and list the long rows in that order too (locality groups, see Graph).  named: the rows are
+        already numbered in that schedule (Graph.named_fwd) -- identity schedule, long rows in id order, and like
+        any locality-grouped schedule no hot tags."""
         L = lib()
         dev, n_rows, nnz = self.device, self.n_rows, self.nnz
         st = stream_of(dev)
@@ -114,11 +117,11 @@ class CSR:
         self.n_long = self.n_items = 0
         self.long_rows = self.long_item_ptr = self.item_long = self.item_start = None
         self.row_order = None
-        self.clustered = groups is not None
+        self.clustered = groups is not None or named
         window = DEFAULT_WINDOW if window is None else int(window)
         if window < 0:
             window = n_rows
-        if n_rows > 1 and nnz > 0:
+        if n_rows > 1 and nnz > 0 and not named:
             if groups is not None:
                 grp, n_groups = groups
                 self.row_order = torch.empty(n_rows, dtype=torch.int32, device=dev)
@@ -319,6 +322,7 @@ class Graph:
         self.groups = locality_groups(self.fwd, deg_order) if deg_order is not None else None
         self.fwd._finish(chunk, long_chunk, window, self.groups, deg_order)
         self._bwd: Optional[CSR] = None
+        self._named: Optional[CSR] = None
         self._lock = threading.Lock()
         self._vals = {}
         self._perm_memo = {}
@@ -332,6 +336,26 @@ class Graph:
                     self._bwd = CSR(self.e_src, self.e_dst, self.N, self.N, self._chunk, self._long_chunk, self._window,
                                     groups=self.groups)     # the groups are a property of the NODES: same for both orientations
         return self._bwd
+
+    @property
+    def named_fwd(self) -> Optional[CSR]:
+        """The forward CSR under the node naming pos = inverse(fwd.row_order), or None when the graph has no
+        locality-grouped schedule.  Row i of it is node fwd.row_order[i]; its schedule is the identity, so a K-hop call
+        on it reads and writes the iterate, the teleport term and the output rows in order and every group's feature
+        rows form one contiguous slice.  Built from the same edited edge list by the same stable sort, every row keeps
+        its edges in the same order: sums, long-row splits and results are bit-identical to those on fwd.  No edge
+        ids (eid is None): only the K-hop paths use it."""
+        if self._named is None and self.groups is not None and self.fwd.row_order is not None:
+            with self._lock:
+                if self._named is None:
+                    order = self.fwd.row_order.long()
+                    pos = torch.empty(self.N, dtype=torch.int32, device=self.device)
+                    pos[order] = torch.arange(self.N, dtype=torch.int32, device=self.device)
+                    csr = CSR(pos.index_select(0, self.e_dst), pos.index_select(0, self.e_src), self.N, self.N,
+                              self.fwd.chunk, self.fwd.long_chunk, named=True)
+                    csr.eid = None
+                    self._named = csr
+        return self._named
 
     def dinv(self) -> torch.Tensor:
         """deg_in^-1/2 with inf -> 0 (gcn_norm, dagnn.py:27-30; unit edge weights)."""
@@ -455,9 +479,11 @@ def cache_bytes() -> int:
 
 def _build_nbytes(g: "Graph") -> int:
     """Bytes a freshly built Graph holds, plus what its lazily built parts will add (transpose CSR, weights in
-    both orientations, one hot-tagged column copy each): the cap is about what an entry may grow to."""
+    both orientations, one hot-tagged column copy each, the renamed forward CSR of a locality-grouped graph): the cap
+    is about what an entry may grow to."""
     nnz, n = g.nnz, g.N
-    return 2 * 4 * nnz + 2 * (8 * (n + 1) + 8 * nnz + 4 * n) + 2 * 4 * nnz + 2 * 4 * nnz
+    named = 8 * (n + 1) + 4 * nnz + 4 * n if g.groups is not None else 0
+    return 2 * 4 * nnz + 2 * (8 * (n + 1) + 8 * nnz + 4 * n) + 2 * 4 * nnz + 2 * 4 * nnz + named
 
 
 def oom_retry(fn):

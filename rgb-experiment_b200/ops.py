@@ -69,7 +69,7 @@ def alloc_rows(N: int, F: int, dtype, device) -> Tuple[torch.Tensor, int]:
 def make_epilogue(*, row_scale=None, row_div=False, a=1.0, b=0.0, T=None, ldt=0, clamp=None,
                   reset_mask=None, reset_val=None, ld_reset=0, reset_when=RESET_NONE,
                   out2_scale=None, acc_in=None, ld_acc=0, skip_empty=False, peers=(), peer_row0=0,
-                  ld_peer=0) -> Epilogue:
+                  ld_peer=0, row_map=None) -> Epilogue:
     e = Epilogue()
     e.row_scale, e.row_div = ptr(row_scale), int(bool(row_div))
     e.reset_mask, e.reset_val, e.ld_reset, e.reset_when = ptr(reset_mask), ptr(reset_val), ld_reset, reset_when
@@ -83,6 +83,7 @@ def make_epilogue(*, row_scale=None, row_div=False, a=1.0, b=0.0, T=None, ldt=0,
     for q, pp in enumerate(peers):          # raw device pointers (ints) of peer-mapped buffers
         e.peer_out[q] = int(pp)
     e.n_peers, e.peer_row0, e.ld_peer = len(peers), int(peer_row0), int(ld_peer)
+    e.row_map = ptr(row_map)
     return e
 
 
@@ -231,6 +232,9 @@ def propagate_weighted(x, w, graph: Graph):
 # ------------------------------------------------------------------------------------------
 FOLD_KHOP = True     # K-hop families apply D^-1/2 (A+I) D^-1/2 as row scalings around an unweighted sum (no per-edge
                      # weight stream, 4 B/edge less and adds instead of FMAs); False: per-edge gcn_norm weights as PyG multiplies them
+NAMED_KHOP = True    # folded fp32 K-hop forwards (APPNP, SGC, K >= 2) on a locality-grouped graph run on Graph.named_fwd, the
+                     # nodes renamed in schedule order: the iterate, teleport and output rows are read and written in order
+                     # and each group's feature rows are contiguous (bit-identical results); False: on fwd, ids as given
 FUSED_DROPOUT = False  # GATConv / SuperGATConv / FAConv in training mode: True = attention dropout generated inside the
                        # attention kernels (counter-based, keyed by edge id, nothing edge-sized allocated); False = a torch
                        # F.dropout mask per call, so the same torch.manual_seed draws the same masks as it always has
@@ -249,21 +253,45 @@ def _khop_gcn(csr: CSR, graph: Graph, x0b: torch.Tensor, K: int, transpose: bool
     return khop_raw(csr, x0b, K, val=graph.gcn_val(transpose), ep=make_epilogue(**epkw))
 
 
-def _staged(x: torch.Tensor, d: torch.Tensor):
+def _staged(x: torch.Tensor, d: torch.Tensor, src_map: Optional[torch.Tensor] = None, teleport: bool = True):
     """(z0 padded to an aligned row stride, u0 = D^-1/2 z0) from an UNALIGNED fp32 input in ONE kernel (instead of a zero
-    fill, a copy and a row scale): the case of every class count that is not a multiple of four (47, 10, ...)."""
+    fill, a copy and a row scale): the case of every class count that is not a multiple of four (47, 10, ...).
+    src_map: row i is input row src_map[i] (a renamed graph's node order); teleport=False: no z0 (None)."""
     N, F = x.shape
     Fp = padded_width(F, x.dtype)
-    z0 = torch.empty((N, Fp), dtype=x.dtype, device=x.device)
+    z0 = torch.empty((N, Fp), dtype=x.dtype, device=x.device) if teleport else None
     u0 = torch.empty((N, Fp), dtype=x.dtype, device=x.device)
     xc = x if x.stride(1) == 1 else x.contiguous()
     dev = x.device
-    check(lib().rgbmp_stage_rows(ptr(xc), xc.stride(0), ptr(d), ptr(z0), ptr(u0), Fp, N, F, dev.index, stream_of(dev)), "stage_rows")
-    return z0[:, :F], u0[:, :F], Fp
+    check(lib().rgbmp_stage_rows(ptr(xc), xc.stride(0), ptr(src_map), ptr(d), ptr(z0), ptr(u0), Fp, N, F, dev.index,
+                                 stream_of(dev)), "stage_rows")
+    return (None if z0 is None else z0[:, :F]), u0[:, :F], Fp
+
+
+def _named_csr(graph: Graph, x: torch.Tensor, K: int, transpose: bool, fold: bool) -> Optional[CSR]:
+    """graph.named_fwd when this K-hop call runs on the renamed graph (NAMED_KHOP), else None."""
+    if not (NAMED_KHOP and fold and not transpose and K >= 2 and x.dim() == 2 and x.dtype == torch.float32
+            and x.size(0) > 0 and x.size(0) == getattr(graph, "N", -1)):
+        return None
+    return getattr(graph, "named_fwd", None)
+
+
+def _khop_named(nf: CSR, graph: Graph, x: torch.Tensor, K: int, a: float = 1.0, b: Optional[float] = None):
+    """Folded K hops of z <- a * A_hat z (+ b * x) on the renamed graph nf: the staging pass reads x in nf's node order,
+    the last hop stores under the original ids.  Same operator, same per-row sums and roundings as on graph.fwd."""
+    d = nf.norm(NORM_INV_SQRT)              # dinv in the renamed order
+    order = graph.fwd.row_order             # row i of nf is node order[i]
+    z0, u0, ld = _staged(x, d, order, teleport=b is not None)
+    ep = make_epilogue(row_scale=d, out2_scale=d, a=a, b=0.0 if b is None else b, T=z0, ldt=ld if z0 is not None else 0,
+                       row_map=order)
+    return khop_raw(nf, u0, K, ep=ep, keep=(z0, d, order))
 
 
 def _appnp_khop(csr: CSR, graph: Graph, x: torch.Tensor, K: int, alpha: float, transpose: bool, fold: bool):
     _lib.require_cuda(x, "x")
+    nf = _named_csr(graph, x, K, transpose, fold)
+    if nf is not None:
+        return _khop_named(nf, graph, x, K, a=1.0 - alpha, b=alpha)
     if fold and x.dim() == 2 and x.dtype == torch.float32 and x.size(1) % 4 != 0 and x.size(0) > 0:
         d = graph.dinv()
         z0, u0, ld = _staged(x, d)
@@ -303,6 +331,10 @@ class _PowerHops(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, graph: Graph, K: int, fold: bool):
         ctx.graph, ctx.K, ctx.fold = graph, K, fold
+        _lib.require_cuda(x, "x")
+        nf = _named_csr(graph, x, K, False, fold)
+        if nf is not None:
+            return _khop_named(nf, graph, x, K)
         return _khop_gcn(graph.fwd, graph, as_rows(x)[0], K, False, fold)
 
     @staticmethod
@@ -981,8 +1013,11 @@ class HostAppnpPlan:
         N, dev = graph.N, graph.device
         self.graph, self.F, self.ld = graph, F, padded_width(F)
         self.bufs = [torch.empty((N, self.ld), dtype=torch.float32, device=dev) for _ in range(4)]
-        self.ws = graph.fwd.spmm_workspace(F)
-        self.dinv = graph.dinv()
+        nf = graph.named_fwd if NAMED_KHOP else None      # the renamed graph, as in _appnp_khop
+        self.csr = graph.fwd if nf is None else nf
+        self.row_map = None if nf is None else graph.fwd.row_order
+        self.ws = self.csr.spmm_workspace(F)
+        self.dinv = self.csr.norm(NORM_INV_SQRT)
 
 
 def appnp_host(graph: Graph, z0_host: torch.Tensor, out_host: torch.Tensor, K: int, alpha: float,
@@ -998,7 +1033,8 @@ def appnp_host(graph: Graph, z0_host: torch.Tensor, out_host: torch.Tensor, K: i
         plan = HostAppnpPlan(graph, F)
     dev = graph.device
     z0d, ping, pong, outd = plan.bufs
-    check(lib().rgbmp_appnp_host(graph.fwd.hot_ref(plan.ld * 4), ptr(plan.dinv), z0_host.data_ptr(), out_host.data_ptr(), F, K,
-                                 float(alpha), ptr(z0d), ptr(ping), ptr(pong), ptr(outd), plan.ld, ptr(plan.ws),
-                                 0 if plan.ws is None else plan.ws.numel(), dev.index, stream_of(dev)), "appnp_host")
+    check(lib().rgbmp_appnp_host_mapped(plan.csr.hot_ref(plan.ld * 4), ptr(plan.row_map), ptr(plan.dinv), z0_host.data_ptr(),
+                                        out_host.data_ptr(), F, K, float(alpha), ptr(z0d), ptr(ping), ptr(pong), ptr(outd),
+                                        plan.ld, ptr(plan.ws), 0 if plan.ws is None else plan.ws.numel(), dev.index,
+                                        stream_of(dev)), "appnp_host")
     return out_host
