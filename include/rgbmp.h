@@ -222,10 +222,19 @@ typedef struct rgbmp_epilogue {
   int64_t        ld_peer;
   /* optional int32 [n_rows]: row i of the graph is row row_map[i] of Y.  A graph whose nodes are renamed in schedule
    * order stores its result under the original names this way; only the Y store is redirected (Y2, T, row_scale
-   * and out2_scale stay indexed by i).  Not accepted with peers, acc_in or reset rows; rgbmp_khop applies it to
-   * the last hop only and rejects it with `hops`. */
+   * and out2_scale stay indexed by i).  rgbmp_khop applies it to the last hop only. */
   const int32_t* row_map;
 } rgbmp_epilogue_t;
+/* rgbmp_spmm and rgbmp_khop check the epilogue before they select a device; NULL stands for {a = 1}, nothing else set:
+ *   RGBMP_EINVAL  reset_when not 0, 1 or 2; reset_when != 0 without reset_mask, reset_val and ld_reset >= F;
+ *   RGBMP_EINVAL  T with ldt < F; Y2 without out2_scale or with ldy2 < F; acc_in with ld_acc < F;
+ *   RGBMP_EINVAL  n_peers outside [0, RGBMP_MAX_PEERS], a NULL peer_out[q] for q < n_peers, or peers with ld_peer < F;
+ *   RGBMP_EALIGN  a peer_out[q] that is not 16-byte aligned;
+ *   RGBMP_EINVAL  row_map together with peers, acc_in or reset rows;
+ *   RGBMP_EINVAL  rgbmp_spmm only: no output (Y NULL, no Y2 and no peers).
+ * K-hop only (rgbmp_khop owns every hop's stores, and every hop rewrites every row):
+ *   RGBMP_EINVAL  Y2, acc_in, skip_empty or peers;
+ *   RGBMP_EINVAL  row_map together with `hops`. */
 
 /* CSR SpMM  Y[i,:] = epilogue( sum_k val[k] * X[col[k],:] ), k in rowptr[i]..rowptr[i+1].
  * Replaces MessagePassing.propagate = index_select -> message -> scatter
@@ -268,7 +277,7 @@ int rgbmp_khop(const rgbmp_graph_t* g, const float* val, const void* X0, int64_t
                void* ws, size_t ws_bytes, int device, void* stream);
 /* Small graphs take ONE launch of ONE thread-block cluster (16 CTAs, 8 where 16 cannot be placed) for all K hops
  * (csrc/khop_cta.cu; hops separated by the hardware cluster barrier, the iterate stays in ping / pong, i.e. in L2): fp32,
- * 16-byte aligned padded rows, K >= 2, F <= 16, at most 8 MB gathered per hop, n_rows <= 200,000, no peer / acc_in / skip_empty
+ * 16-byte aligned padded rows, K >= 2, F <= 16, at most 8 MB gathered per hop, n_rows <= 200,000, no row_map in the
  * epilogue.  Same operator, same per-row summation order.  rgbmp_set_khop_cta(0 | 1) turns the path off / on process-wide
  * (default on; environment RGBMP_KHOP_CTA=0 turns it off) and returns the previous setting; other values only query. */
 int rgbmp_set_khop_cta(int on);

@@ -19,9 +19,9 @@
 //   * a hop barrier built from one remote mbarrier arrive per CTA (one release fence per CTA instead of one per thread)
 //     in place of barrier.cluster: within noise of it (56 vs 54 us for APPNP K=10).
 // Edges of a row accumulate sequentially in stable CSR order exactly as in spmm_rows_kernel (bit-identical for rows
-// neither path splits); the epilogue is rgbmp_epilogue_t's.
+// neither path splits); the epilogue is rgbmp_epilogue_t's, applied by the same ep_apply.
 #include <stdlib.h>
-#include "common.cuh"
+#include "epilogue.cuh"
 
 namespace rgbmp {
 
@@ -116,16 +116,7 @@ __device__ __forceinline__ float4 kc_epilogue(const KhopCtaParams& p, const KcRo
 #pragma unroll
     for (int i = 0; i < 4; ++i) rv[i] = (f + i < p.F) ? ep.reset_val[(int64_t)r.row * ep.ld_reset + f + i] : 0.f;
   }
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    float x = ep.row_scale ? (ep.row_div ? __fdiv_rn(v[i], r.rs) : __fmul_rn(r.rs, v[i])) : v[i];
-    if (r.reset && ep.reset_when == 1) x = rv[i];
-    x = __fmul_rn(ep.a, x);
-    if (ep.T) x = __fadd_rn(x, __fmul_rn(ep.b, t[i]));
-    if (ep.clamp) x = fminf(fmaxf(x, ep.lo), ep.hi);
-    if (r.reset && ep.reset_when == 2) x = rv[i];
-    v[i] = x;
-  }
+  ep_apply<4>(ep, v, r.rs, r.reset, rv, t);
   if (y) {
     float* q = y + (int64_t)r.row * ldy + f;
     if ((ldy & 3) == 0 && ((reinterpret_cast<uintptr_t>(y) & 15) == 0)) {
@@ -447,21 +438,22 @@ static int kc_launch(const KhopCtaParams& p, cudaStream_t st, int device) {
 }
 
 // *handled = 1 when the call was taken (return value = its status), 0 = not eligible: the caller runs the K-launch path.
-// Eligible: fp32, 16-byte aligned padded rows everywhere, at most KC_MAX_GATHER_BYTES gathered per hop and KC_MAX_ROWS
-// rows, rows of at most 4 vectors (KC_MAX_LD), K >= 2, no peer / partial-sum / skip-empty / row-map epilogue, no hot tags.
+// ep passed check_epilogue with EP_KHOP.  Eligible: fp32, 16-byte aligned padded rows everywhere, at most
+// KC_MAX_GATHER_BYTES gathered per hop and KC_MAX_ROWS rows, rows of at most 4 vectors (KC_MAX_LD), K >= 2, no row map,
+// no hot tags.
 int khop_cta_try(const rgbmp_graph_t* g, const float* val, const void* X0, int64_t ldx0, void* ping, void* pong, int64_t ldp,
                  void* out, int64_t ldo, void* hops, int64_t ld_hops, int64_t hop_stride, int F, int dtype, int K,
-                 const rgbmp_epilogue_t* ep, cudaStream_t st, int device, int* handled) {
+                 const rgbmp_epilogue_t& ep, cudaStream_t st, int device, int* handled) {
   *handled = 0;
   const int on = g_kc_override >= 0 ? g_kc_override : kc_enabled();
   if (!on || dtype != RGBMP_F32 || g->col_tagged || g->n_rows < 1 || g->n_rows > KC_MAX_ROWS || g->nnz >= (1ll << 30)) return 0;
-  if (ep && (ep->n_peers > 0 || ep->acc_in || ep->skip_empty || ep->Y2 || ep->row_map)) return 0;
+  if (ep.row_map) return 0;
   const int ld = (int)align_up((size_t)F, 4);
   if (ld > KC_MAX_LD || K < 2) return 0;
   if ((double)g->nnz * ld * 4.0 > KC_MAX_GATHER_BYTES) return 0;
   auto rows_ok = [&](const void* q, int64_t l) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0 && (l & 3) == 0 && l >= ld; };
   if (!rows_ok(X0, ldx0)) return 0;
-  if (ep && ep->T && !rows_ok(ep->T, ep->ldt)) return 0;
+  if (ep.T && !rows_ok(ep.T, ep.ldt)) return 0;
   if (K > 1 && (!ping || !pong || !rows_ok(ping, ldp) || !rows_ok(pong, ldp))) return 0;
   KhopCtaParams p;
   p.rowptr = g->rowptr;
@@ -483,8 +475,7 @@ int khop_cta_try(const rgbmp_graph_t* g, const float* val, const void* X0, int64
   p.hops = (float*)hops;
   p.ld_hops = ld_hops;
   p.hop_stride = hop_stride;
-  if (ep) p.ep = *ep;
-  else { p.ep = rgbmp_epilogue_t{}; p.ep.a = 1.0f; }
+  p.ep = ep;
   const int nvec = ld / 4;
   const int rc = nvec <= 1 ? kc_launch<1>(p, st, device) : (nvec <= 2 ? kc_launch<2>(p, st, device) : kc_launch<4>(p, st, device));
   if (rc != 0) {               // no 8-CTA cluster can be placed on this device / partition: leave the path off for good

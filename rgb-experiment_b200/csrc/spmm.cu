@@ -7,7 +7,7 @@ namespace rgbmp {
 
 int khop_cta_try(const rgbmp_graph_t* g, const float* val, const void* X0, int64_t ldx0, void* ping, void* pong, int64_t ldp,
                  void* out, int64_t ldo, void* hops, int64_t ld_hops, int64_t hop_stride, int F, int dtype, int K,
-                 const rgbmp_epilogue_t* ep, cudaStream_t st, int device, int* handled);   // khop_cta.cu
+                 const rgbmp_epilogue_t& ep, cudaStream_t st, int device, int* handled);   // khop_cta.cu
 
 // packed [n,F] -> pitched z0 [n,ld] (optional) and u0 = scale*z0 [n,ld]; row r reads X row src_map[r] when mapped
 __global__ void __launch_bounds__(256)
@@ -77,8 +77,9 @@ struct Prepared {
   int G, V, U, epv;
 };
 
+// ep passed check_epilogue
 static int spmm_prepare(const rgbmp_graph_t* g, const float* val, const void* X, int64_t ldx, void* Y, int64_t ldy, int F,
-                        int dtype, const rgbmp_epilogue_t* ep, int tune, void* ws, size_t ws_bytes, Prepared* out) {
+                        int dtype, const rgbmp_epilogue_t& ep, int tune, void* ws, size_t ws_bytes, Prepared* out) {
   SpmmParams& p = out->p;
   p.w = csr_work(g);
   p.val = val;
@@ -88,22 +89,7 @@ static int spmm_prepare(const rgbmp_graph_t* g, const float* val, const void* X,
   p.Y = Y;
   p.ldy = ldy;
   p.F = F;
-  if (ep) {
-    p.ep = *ep;
-  } else {
-    rgbmp_epilogue_t z = {};
-    z.a = 1.0f;
-    p.ep = z;
-  }
-  if (p.ep.reset_when != 0 && (!p.ep.reset_mask || !p.ep.reset_val))
-    return fail(RGBMP_EINVAL, "rgbmp_spmm: reset_when set without reset_mask/reset_val");
-  if (p.ep.Y2 && !p.ep.out2_scale) return fail(RGBMP_EINVAL, "rgbmp_spmm: Y2 without out2_scale");
-  if (!Y && !p.ep.Y2 && p.ep.n_peers <= 0) return fail(RGBMP_EINVAL, "rgbmp_spmm: no output");
-  if (p.ep.row_map && (p.ep.n_peers > 0 || p.ep.acc_in || p.ep.reset_when != 0))
-    return fail(RGBMP_EINVAL, "rgbmp_spmm: row_map does not combine with peers, acc_in or reset rows");
-  if (p.ep.n_peers < 0 || p.ep.n_peers > RGBMP_MAX_PEERS) return fail(RGBMP_EINVAL, "rgbmp_spmm: bad n_peers");
-  for (int q = 0; q < p.ep.n_peers; ++q)
-    if (!p.ep.peer_out[q]) return fail(RGBMP_EINVAL, "rgbmp_spmm: null peer buffer %d", q);
+  p.ep = ep;
 
   const int esz = dtype == RGBMP_BF16 ? 2 : 4;
   const int epv_vec = 16 / esz;
@@ -113,8 +99,6 @@ static int spmm_prepare(const rgbmp_graph_t* g, const float* val, const void* X,
   const bool vec_ok = aligned(X, ldx) && aligned(Y, ldy) && aligned(p.ep.T, p.ep.ldt) && aligned(p.ep.Y2, p.ep.ldy2) &&
                       aligned(p.ep.acc_in, p.ep.ld_acc) &&
                       (p.ep.n_peers == 0 || ((p.ep.ld_peer % epv_vec) == 0 && ((p.ep.peer_row0 * p.ep.ld_peer) % epv_vec) == 0));
-  for (int q = 0; q < p.ep.n_peers; ++q)
-    if ((((uintptr_t)p.ep.peer_out[q]) & 15) != 0) return fail(RGBMP_EALIGN, "rgbmp_spmm: peer buffer %d not 16-byte aligned", q);
   const int epv = vec_ok ? epv_vec : 1;
   if (dtype == RGBMP_BF16 && !vec_ok)
     return fail(RGBMP_EALIGN, "rgbmp_spmm: bf16 needs 16-byte aligned pointers and ld %% 8 == 0");
@@ -159,7 +143,7 @@ static int spmm_prepare(const rgbmp_graph_t* g, const float* val, const void* X,
 }
 
 static int spmm_impl(const rgbmp_graph_t* g, const float* val, const void* X, int64_t ldx, void* Y, int64_t ldy, int F,
-                     int dtype, const rgbmp_epilogue_t* ep, int tune, void* ws, size_t ws_bytes, cudaStream_t st) {
+                     int dtype, const rgbmp_epilogue_t& ep, int tune, void* ws, size_t ws_bytes, cudaStream_t st) {
   Prepared pr;
   const int rc = spmm_prepare(g, val, X, ldx, Y, ldy, F, dtype, ep, tune, ws, ws_bytes, &pr);
   if (rc) return rc;
@@ -191,9 +175,12 @@ int rgbmp_spmm(const rgbmp_graph_t* g, const float* val, const void* X, int64_t 
   if (rc) return rc;
   if (!X || F <= 0 || ldx < F || (Y && ldy < F)) return fail(RGBMP_EINVAL, "rgbmp_spmm: bad feature arguments");
   if (dtype != RGBMP_F32 && dtype != RGBMP_BF16) return fail(RGBMP_EINVAL, "rgbmp_spmm: bad dtype %d", dtype);
+  rgbmp_epilogue_t e;
+  rc = check_epilogue(ep, F, Y != nullptr, "rgbmp_spmm", 0, &e);
+  if (rc) return rc;
   DeviceGuard dg(device);
   if (!dg.ok) return fail(RGBMP_EINVAL, "rgbmp_spmm: bad device %d", device);
-  return spmm_impl(g, val, X, ldx, Y, ldy, F, dtype, ep, tune, ws, ws_bytes, (cudaStream_t)stream);
+  return spmm_impl(g, val, X, ldx, Y, ldy, F, dtype, e, tune, ws, ws_bytes, (cudaStream_t)stream);
 }
 
 int rgbmp_khop(const rgbmp_graph_t* g, const float* val, const void* X0, int64_t ldx0, void* ping, void* pong,
@@ -208,20 +195,19 @@ int rgbmp_khop(const rgbmp_graph_t* g, const float* val, const void* X0, int64_t
     if (!through_hops) return fail(RGBMP_EINVAL, "rgbmp_khop: K > 1 needs ping/pong buffers");
   }
   if (dtype != RGBMP_F32 && dtype != RGBMP_BF16) return fail(RGBMP_EINVAL, "rgbmp_khop: bad dtype %d", dtype);
-  if (ep && ep->row_map && hops) return fail(RGBMP_EINVAL, "rgbmp_khop: row_map does not combine with hops");
+  rgbmp_epilogue_t e;
+  rc = check_epilogue(ep, F, true /* out or hops */, "rgbmp_khop", EP_KHOP | (hops ? EP_HOPS : 0), &e);
+  if (rc) return rc;
   DeviceGuard dg(device);
   if (!dg.ok) return fail(RGBMP_EINVAL, "rgbmp_khop: bad device %d", device);
   cudaStream_t st = (cudaStream_t)stream;
   if (!(tune & RGBMP_TUNE_NO_CTA)) {     // small graphs: all K hops in one launch of one thread-block cluster
     int handled = 0;
-    rc = khop_cta_try(g, val, X0, ldx0, ping, pong, ldp, out, ldo, hops, ld_hops, hop_stride, F, dtype, K, ep, st, device,
+    rc = khop_cta_try(g, val, X0, ldx0, ping, pong, ldp, out, ldo, hops, ld_hops, hop_stride, F, dtype, K, e, st, device,
                       &handled);
     if (handled) return rc;
   }
   const size_t esz = dtype == RGBMP_BF16 ? 2 : 4;
-  rgbmp_epilogue_t e;
-  if (ep) e = *ep;
-  else { e = rgbmp_epilogue_t{}; e.a = 1.0f; }
   const bool folded = e.out2_scale != nullptr;  // iterate lives in the pre-scaled copy
   const void* in = X0;
   int64_t ldin = ldx0;
@@ -237,11 +223,11 @@ int rgbmp_khop(const rgbmp_graph_t* g, const float* val, const void* X0, int64_t
     if (folded) {
       ek.Y2 = last ? nullptr : buf;
       ek.ldy2 = ldp;
-    } else {
-      ek.Y2 = nullptr;
-      if (!y) { y = buf; ldy = ldp; }
+    } else if (!y) {
+      y = buf;
+      ldy = ldp;
     }
-    rc = spmm_impl(g, val, in, ldin, y, ldy, F, dtype, &ek, tune, ws, ws_bytes, st);
+    rc = spmm_impl(g, val, in, ldin, y, ldy, F, dtype, ek, tune, ws, ws_bytes, st);
     if (rc) return rc;
     if (folded) { in = buf; ldin = ldp; }
     else { in = y; ldin = ldy; }

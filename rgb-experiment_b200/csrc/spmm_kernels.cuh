@@ -16,6 +16,7 @@
 //     in registers before the single store of the row.
 #pragma once
 #include "csr_work.cuh"
+#include "epilogue.cuh"
 
 namespace rgbmp {
 
@@ -381,16 +382,7 @@ __device__ __forceinline__ void epilogue_store(const SpmmParams& p, int64_t row,
     else tr.load(reinterpret_cast<const T*>(ep.T) + row * ep.ldt + f);
     tr.unpack(t);
   }
-#pragma unroll
-  for (int i = 0; i < EPV; ++i) {
-    float v = ep.row_scale ? (ep.row_div ? __fdiv_rn(s[i], rs) : __fmul_rn(rs, s[i])) : s[i];
-    if (reset && ep.reset_when == 1) v = rv[i];
-    v = __fmul_rn(ep.a, v);
-    if (ep.T) v = __fadd_rn(v, __fmul_rn(ep.b, t[i]));
-    if (ep.clamp) v = fminf(fmaxf(v, ep.lo), ep.hi);
-    if (reset && ep.reset_when == 2) v = rv[i];
-    s[i] = v;
-  }
+  ep_apply<EPV>(ep, s, rs, reset, rv, t);
   if (p.Y) {
     const int64_t yrow = ep.row_map ? (int64_t)__ldg(ep.row_map + row) : row;
     Raw<T, EPV>::store(reinterpret_cast<T*>(p.Y) + yrow * p.ldy + f, s, p.stream);

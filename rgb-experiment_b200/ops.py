@@ -87,6 +87,15 @@ def make_epilogue(*, row_scale=None, row_div=False, a=1.0, b=0.0, T=None, ldt=0,
     return e
 
 
+def reset_rows(mask: torch.Tensor, vals: torch.Tensor, F: int) -> dict:
+    """make_epilogue keywords of label propagation's fixed-scale post-step: after the clamp, the rows where `mask` is set
+    take the first F columns of their `vals` (RESET_AFTER_CLAMP).  The epilogue reads a byte per row and the values as
+    float32 rows whatever the feature dtype; tensors already in that form are used without a copy."""
+    _lib.require_cuda(mask, "reset mask")
+    rv, ldr = as_rows(vals[:, :F].float())
+    return dict(reset_mask=mask.to(torch.uint8).contiguous(), reset_val=rv, ld_reset=ldr, reset_when=RESET_AFTER_CLAMP)
+
+
 def _graph_ref(csr, row_bytes: int, hot: bool = True):
     if hot and hasattr(csr, "hot_ref"):
         return csr.hot_ref(row_bytes)
@@ -386,12 +395,8 @@ def label_propagation(graph: Graph, out0: torch.Tensor, num_layers: int, alpha: 
         return out0
     xb, ldx = as_rows(out0)
     kw = {}
-    keep = [xb]
     if reset_mask is not None:
-        m = reset_mask.to(torch.uint8).contiguous()
-        rv, ldr = as_rows(reset_val.float())      # the epilogue reads reset rows as float32 whatever the feature dtype
-        kw = dict(reset_mask=m, reset_val=rv, ld_reset=ldr, reset_when=RESET_AFTER_CLAMP)
-        keep += [m, rv]
+        kw = reset_rows(reset_mask, reset_val, out0.size(1))
         clamp = None
     return _khop_gcn(graph.fwd, graph, xb, num_layers, False, bool(FOLD_KHOP if fold is None else fold),
                      a=alpha, b=1.0 - alpha, T=xb, ldt=ldx, clamp=clamp, **kw)

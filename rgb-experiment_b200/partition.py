@@ -347,25 +347,6 @@ def _wrap(ptr: int, nbytes: int, device) -> torch.Tensor:
     return torch.as_tensor(_RawCuda(ptr, nbytes), device=device)
 
 
-def _reset_rows(reset, F: int):
-    """(mask [R], values [R, >= F]) -> (uint8 mask, float32 values with 16-byte aligned rows), once per run: the
-    epilogue reads a byte per row and the values as float32 whatever the feature dtype (as ops.label_propagation)."""
-    from . import _lib, ops
-    mask, vals = reset
-    _lib.require_cuda(mask, "reset mask")
-    rv, _ = ops.as_rows(vals[:, :F].float())
-    return mask.to(torch.uint8).contiguous(), rv
-
-
-def _post_epilogue(clamp, reset) -> dict:
-    """make_epilogue keywords of label propagation's post-step (`reset` as _reset_rows returns it)."""
-    from . import ops
-    kw = {} if clamp is None else dict(clamp=clamp)
-    if reset is not None:
-        kw.update(reset_mask=reset[0], reset_val=reset[1], ld_reset=reset[1].stride(0), reset_when=ops.RESET_AFTER_CLAMP)
-    return kw
-
-
 class PartitionedAPPNP:
     """APPNP / LP-style K-hop propagation over a LocalBlock.
 
@@ -404,8 +385,9 @@ class PartitionedAPPNP:
             out = self.pong if self._flip else self.ping
             self._flip = not self._flip
             tele = dict(b=b, T=z0_local, ldt=z0_local.stride(0)) if b != 0.0 else {}
-            ep = ops.make_epilogue(a=a, **tele, **_post_epilogue(clamp, reset))
-            ops.spmm_raw(block.csr, x_full[:, :F], block.val, ep=ep, keep=(z0_local, reset), out=out[:, :F])
+            post = {} if reset is None else ops.reset_rows(*reset, F)     # run() converted the rows: no copy here
+            ep = ops.make_epilogue(a=a, clamp=clamp, **tele, **post)
+            ops.spmm_raw(block.csr, x_full[:, :F], block.val, ep=ep, keep=(z0_local,), out=out[:, :F])
             return out
 
         self.driver = PartitionedPropagator(block.N, block.rank, block.world, spmm, group)
@@ -426,12 +408,13 @@ class PartitionedAPPNP:
             _lib.dtype_code(z0_local)
             raise RuntimeError(f"z0_local is {z0_local.dtype}; this propagation was built for {self.dtype}")
         a, b = (1.0 - alpha, alpha) if teleport is None else (float(teleport[0]), float(teleport[1]))
-        check_post_step(self.block.R, clamp, reset)
-        if reset is not None:
-            reset = _reset_rows(reset, self.F)
-        if self.mode != "push":
-            return self.driver.run(z0_local, K, a, b, self.full, clamp=clamp, reset=reset)
         from . import ops
+        check_post_step(self.block.R, clamp, reset)
+        post = {} if reset is None else ops.reset_rows(*reset, self.F)    # once per run
+        if self.mode != "push":
+            if reset is not None:
+                reset = (post["reset_mask"], post["reset_val"])
+            return self.driver.run(z0_local, K, a, b, self.full, clamp=clamp, reset=reset)
         blk, F, R = self.block, self.F, self.block.R
         full = self.peers.local
         d = blk.dinv_local
@@ -443,17 +426,16 @@ class PartitionedAPPNP:
         dbg_self_only = os.environ.get("RGBMP_DEBUG_PUSH") == "self"
         dbg_no_tick = os.environ.get("RGBMP_DEBUG_TICK") == "0"
         tele = dict(b=b, T=z0_local, ldt=z0_local.stride(0)) if b != 0.0 else {}
-        post = _post_epilogue(clamp, reset)
         for k in range(K):
             src, nxt, last = full[k & 1], (k + 1) & 1, k == K - 1
             if last:                       # the result stays local and unscaled: no push, no tick
-                ep = ops.make_epilogue(row_scale=d, a=a, **tele, **post)
-                ops.spmm_raw(blk.csr, src[:, :F], None, ep=ep, keep=(z0_local, d, reset), out=self.out[:, :F])
+                ep = ops.make_epilogue(row_scale=d, a=a, clamp=clamp, **tele, **post)
+                ops.spmm_raw(blk.csr, src[:, :F], None, ep=ep, keep=(z0_local, d), out=self.out[:, :F])
                 break
             peers = [self.peers.ptrs[nxt][blk.rank]] if dbg_self_only else self.peers.ptrs[nxt]
             ep = ops.make_epilogue(row_scale=d, a=a, out2_scale=d, peers=peers, peer_row0=blk.rank * R,
-                                   ld_peer=self.ld, **tele, **post)
-            ops.spmm_raw(blk.csr, src[:, :F], None, ep=ep, keep=(z0_local, d, reset), store_local=False)
+                                   ld_peer=self.ld, clamp=clamp, **tele, **post)
+            ops.spmm_raw(blk.csr, src[:, :F], None, ep=ep, keep=(z0_local, d), store_local=False)
             if not dbg_no_tick:
                 dist.all_reduce(self.tick, group=self.group)     # orders the hops: every push has landed
         return self.out
