@@ -59,13 +59,17 @@ static int push_bulk_default() {
 //     U4 0.307 vs 0.459); rows wider than 64 vectors are tiled over blockIdx.y;
 //   * narrow rows: 8 lanes x 8 edges for 5-8 vectors (F=24/32: 1.81 / 1.74 ms), 4 lanes below that -- pipelined
 //     for 1-2 vectors, where two idle lanes still beat the 2-lane group (F=8: 0.86 vs 1.08 ms).
-//   * when the gathers come from HBM (feature matrix well beyond L2) 4 edges in flight at 5 CTAs per SM (40 registers)
-//     edge out 8 at 4 CTAs: products F=47 2.74 vs 2.83 ms per hop under the locality schedule; L2-resident matrices
-//     (arxiv F=40, bf16 F=128) keep 8.
-static void choose_shape(int nvec, bool hbm_regime, int* G, int* V, int* U) {
+//   * rows of 9-16 vectors whose gathers come from HBM (feature matrix well beyond L2), with the round-4 loop (one plain
+//     load per vector on untagged graphs; profiles/r04_spmm_untagged_gather.txt, bench.py on one B200 at 1000 W):
+//     rows of 32 edges and more on average keep 8 edges in flight at 4 CTAs/SM (62 registers) -- products F=47
+//     55.5 GTEPS vs 54.6 with 4 edges at 5 CTAs/SM (48 registers; 8 edges at 5 CTAs spill 224 bytes); shorter rows
+//     (papers100M-shaped block, 29.5 edges per row on average, bf16 F=128) keep 4 at 5 CTAs/SM, 22.2 vs 21.9 GTEPS
+//     with 8 (both with the two-loop weighted bf16 kernel, since replaced).  The cut-off of 32 only separates these two measured graphs (29.5 and 51.5 edges per row); it has not
+//     been swept.  L2-resident matrices (arxiv F=40, bf16 F=128) keep 8.
+static void choose_shape(int nvec, bool hbm_short_rows, int* G, int* V, int* U) {
   if (nvec > 32) { *G = 32; *V = 2; *U = 4; return; }
   if (nvec > 16) { *G = 16; *V = 2; *U = 4; return; }
-  if (nvec > 8) { *G = 16; *V = 1; *U = hbm_regime ? 4 : 8; return; }
+  if (nvec > 8) { *G = 16; *V = 1; *U = hbm_short_rows ? 4 : 8; return; }
   if (nvec > 4) { *G = 8; *V = 1; *U = 8; return; }
   *G = 4;
   *V = 1;
@@ -116,9 +120,11 @@ static int spmm_prepare(const rgbmp_graph_t* g, const float* val, const void* X,
   const int nvec = (int)ceil_div(F, epv);
   // gathered rows mostly come from HBM once the feature matrix is well beyond the 126 MB L2
   const bool hbm_regime = (double)g->n_cols * (double)ldx * esz > 96e6;
-  choose_shape(nvec, hbm_regime, &G, &V, &U);
+  const bool short_rows = g->nnz < 32 * g->n_rows;   // mean row shorter than two 16-edge batches
+  choose_shape(nvec, hbm_regime && short_rows, &G, &V, &U);
   p.stream = (tune & RGBMP_TUNE_NO_STREAM) ? 0 : 1;
   // gathered rows: ids tagged hot by rgbmp_col_tag stay in L2 (evict-last), the rest leave first
+  p.hinted = (g->col_tagged || (tune & RGBMP_TUNE_POLICY)) ? 1 : 0;
   p.pol_hot = g->col_tagged ? 2 : 0;
   p.pol_cold = g->col_tagged ? 1 : 0;
   if (tune & RGBMP_TUNE_POLICY) {

@@ -34,9 +34,10 @@ struct SpmmParams {
   // cache policy: 1 = column ids, weights, teleport rows and outputs are touched once per launch ->
   // streaming (evict-first) loads/stores, so that L2 keeps the gathered feature rows instead
   int stream;
-  // L2 eviction priority of the gathered feature rows (0 normal, 1 evict-first, 2 evict-last):
-  // pol_hot for column ids tagged hot (bit 31 set by rgbmp_col_tag), pol_cold for the rest.  With
-  // an untagged graph every row takes pol_cold.
+  // hinted = 1 (hot-tagged graph, or a policy set in the tune word): each gathered row carries an L2 eviction priority
+  // (0 normal, 1 evict-first, 2 evict-last), pol_hot for column ids tagged hot (bit 31 set by rgbmp_col_tag), pol_cold
+  // for the rest.  hinted = 0: one plain load per vector, no tag mask, no policy descriptor.
+  int hinted;
   int pol_hot, pol_cold;
   // fused all-gather: 1 = the short-row kernel stages each finished row in shared memory and pushes it to every peer with
   // one bulk asynchronous copy (cp.async.bulk, TMA) instead of 16-byte st.global per lane
@@ -193,18 +194,25 @@ __device__ __forceinline__ uint64_t make_policy(int kind) {
   return pol;
 }
 
-// gather one 16-byte vector of feature row `ctag & 0x7fffffff`; bit 31 of the id selects the policy.
-// The L2 policy travels in a memory DESCRIPTOR, which is warp-uniform on sm_100 (ptxas moves a
-// per-lane policy through R2UR, i.e. silently applies one lane's choice to the whole warp), so the
-// choice is expressed as two predicated loads with kernel-uniform policies.
-// `act` = this lane owns an existing vector of the row (lane-constant): lanes beyond F issue NO load -- a
-// predicated-off lane costs nothing in the LSU, while a dummy load of vector 0 touched a second cache line per
-// gathered row (one more L1 wavefront and two more sectors per edge for F = 47; profiles/r02_spmm_l1_wavefronts.txt).
-template <typename T, int EPV>
+// gather one 16-byte vector of feature row `ctag` (act = false: no load, zeros; the tail batches pass it -- without the
+// zero fill the predicated load's destination would stay live through the full-batch loop: +6 registers, spills).  Every lane
+// loads: a lane beyond F has its base on the row's LAST vector (lane_bases), so there is no predicate, branch or zero fill
+// in the full-batch loop.  Where another lane of the same instruction reads that vector anyway (every tile whose v-th
+// slice holds at least one vector of the row -- all shapes choose_shape() picks for rows of at most 64 vectors) this
+// costs no extra line or L1 wavefront.  A slice wholly beyond F (G32 V2: the last tile of a row wider than 64 vectors
+// with at most 32 vectors left, e.g. F = 602 fp32, tile 3; or V2 tune words on narrow rows) issues one extra load of an
+// already-requested line per edge, which the parent predicated off.
+// (Round 1's dummy load of vector 0 did cost a second line per gathered row; profiles/r02_spmm_l1_wavefronts.txt.)
+// HINTED: bit 31 of the id selects the policy.  The L2 policy travels in a memory DESCRIPTOR, which is warp-uniform on
+// sm_100 (ptxas moves a per-lane policy through R2UR, i.e. silently applies one lane's choice to the whole warp), so
+// the choice is expressed as two predicated loads with kernel-uniform policies.  Without HINTED: one plain load, no
+// tag mask, no policy descriptor.
+template <typename T, int EPV, bool HINTED>
 __device__ __forceinline__ void gather_vec(Raw<T, EPV>& raw, const char* base, uint32_t ctag, uint32_t row_bytes,
                                            uint64_t pol_hot, uint64_t pol_cold, bool act) {
-  const T* q = reinterpret_cast<const T*>(row_addr(base, ctag & 0x7fffffffu, row_bytes));
+  const T* q = reinterpret_cast<const T*>(row_addr(base, HINTED ? ctag & 0x7fffffffu : ctag, row_bytes));
   if (!act) raw.zero();
+  else if (!HINTED) raw.load(q);
   else if (ctag & 0x80000000u) raw.load_hint(q, pol_hot);
   else raw.load_hint(q, pol_cold);
 }
@@ -240,18 +248,26 @@ __device__ __forceinline__ void lds_wts(const float* p, float (&w)[N]) {
 // The loop is WARP-uniform: every lane of the warp runs the same number of batches (the maximum
 // over the warp's groups; with the degree-sorted row schedule the groups of a warp have equal
 // lengths, so nothing is wasted), which lets full batches run without a single predicate.
-// xb[v]: this lane's base pointer for its v-th vector; active[v]: the vector exists (lane-constant).
+// xb[v]: this lane's base pointer for its v-th vector (a lane beyond F: the row's last vector, see gather_vec).
 // PIPE: software-pipelined main loop -- the features of step j+1 are requested BEFORE the math of
 // step j and consumed in the next loop iteration, so UE*V loads per lane are always in flight
 // whatever order ptxas picks inside one iteration (without it, ptxas 12.9 sinks each LDG next to
 // its FFMA2 and serialises the gathers).
-template <typename T, int EPV, int G, int V, int U, bool HASW, bool PIPE>
-__device__ __forceinline__ void accumulate_range(const SpmmParams& p, int64_t k0, int64_t k1, const char* const (&xb)[V],
+template <typename T, int EPV, int G, int V, int U, bool HASW, bool PIPE, bool HINTED>
+__device__ __forceinline__ void accumulate_edges(const SpmmParams& p, int64_t k0, int64_t k1, const char* const (&xb)[V],
                                                  const bool (&active)[V], int gl, const IdStage& sm,
                                                  float2 (&acc)[V][(EPV + 1) / 2]) {
   constexpr int UE = (U < G) ? U : G;   // edges per inner step (a batch holds G ids)
+  constexpr bool LANE_BRANCH = HASW && EPV == 8;   // weighted bf16: lanes beyond F skip their load (see accumulate_range)
+  bool act[V];
+#pragma unroll
+  for (int v = 0; v < V; ++v) act[v] = LANE_BRANCH ? active[v] : true;
   const uint32_t row_bytes = (uint32_t)(p.ldx * (int64_t)sizeof(T));
-  const uint64_t pol_hot = make_policy(p.pol_hot), pol_cold = make_policy(p.pol_cold);
+  uint64_t pol_hot = 0, pol_cold = 0;
+  if constexpr (HINTED) {
+    pol_hot = make_policy(p.pol_hot);
+    pol_cold = make_policy(p.pol_cold);
+  }
   const int32_t* __restrict__ col = p.w.col + k0;
   const float* __restrict__ val = HASW ? p.val + k0 : nullptr;
   const int len = (k1 > k0) ? (int)(k1 - k0) : 0;          // <= chunk / long sub-range, fits int
@@ -285,7 +301,7 @@ __device__ __forceinline__ void accumulate_range(const SpmmParams& p, int64_t k0
 #pragma unroll
           for (int u = 0; u < UE; ++u)
 #pragma unroll
-            for (int v = 0; v < V; ++v) gather_vec<T, EPV>(cur[u][v], xb[v], c[u], row_bytes, pol_hot, pol_cold, active[v]);
+            for (int v = 0; v < V; ++v) gather_vec<T, EPV, HINTED>(cur[u][v], xb[v], c[u], row_bytes, pol_hot, pol_cold, act[v]);
         }
 #pragma unroll 1
         for (int j = 0; j < G; j += UE) {
@@ -296,7 +312,7 @@ __device__ __forceinline__ void accumulate_range(const SpmmParams& p, int64_t k0
 #pragma unroll
           for (int u = 0; u < UE; ++u)
 #pragma unroll
-            for (int v = 0; v < V; ++v) gather_vec<T, EPV>(nxt[u][v], xb[v], c[u], row_bytes, pol_hot, pol_cold, active[v]);
+            for (int v = 0; v < V; ++v) gather_vec<T, EPV, HINTED>(nxt[u][v], xb[v], c[u], row_bytes, pol_hot, pol_cold, act[v]);
           float w[UE];
           if constexpr (HASW) lds_wts<UE>(gwt_ + j, w);
 #pragma unroll
@@ -318,7 +334,7 @@ __device__ __forceinline__ void accumulate_range(const SpmmParams& p, int64_t k0
 #pragma unroll
           for (int u = 0; u < UE; ++u)
 #pragma unroll
-            for (int v = 0; v < V; ++v) gather_vec<T, EPV>(raw[u][v], xb[v], c[u], row_bytes, pol_hot, pol_cold, active[v]);
+            for (int v = 0; v < V; ++v) gather_vec<T, EPV, HINTED>(raw[u][v], xb[v], c[u], row_bytes, pol_hot, pol_cold, act[v]);
           float w[UE];
           if constexpr (HASW) lds_wts<UE>(gwt_ + j, w);
 #pragma unroll
@@ -338,8 +354,8 @@ __device__ __forceinline__ void accumulate_range(const SpmmParams& p, int64_t k0
 #pragma unroll
         for (int u = 0; u < UE; ++u) {
 #pragma unroll
-          for (int v = 0; v < V; ++v)
-            gather_vec<T, EPV>(raw[u][v], xb[v], c[u], row_bytes, pol_hot, pol_cold, active[v] && (j + u < nb));
+          for (int v = 0; v < V; ++v)   // an edge past the group's row loads nothing (zeros) and is not added
+            gather_vec<T, EPV, HINTED>(raw[u][v], xb[v], c[u], row_bytes, pol_hot, pol_cold, act[v] && (j + u < nb));
         }
         float w[UE];
         if constexpr (HASW) lds_wts<UE>(gwt_ + j, w);
@@ -353,6 +369,19 @@ __device__ __forceinline__ void accumulate_range(const SpmmParams& p, int64_t k0
       }
     }
   }
+}
+
+// hinted is kernel-uniform: one branch per launch, both edge loops inlined into the same kernel.  Weighted bf16 sums
+// keep the previous loop (the hinted form, which also serves untagged graphs, with a per-lane branch): two loops in one
+// kernel cost them 12 registers, and at 5 CTAs/SM (20-byte spill) or at 4 CTAs/SM the weighted bf16 hop of the
+// papers100M-shaped block ran 7 % / 5 % slower (profiles/r04_spmm_untagged_gather.txt, section 6).
+template <typename T, int EPV, int G, int V, int U, bool HASW, bool PIPE>
+__device__ __forceinline__ void accumulate_range(const SpmmParams& p, int64_t k0, int64_t k1, const char* const (&xb)[V],
+                                                 const bool (&active)[V], int gl, const IdStage& sm,
+                                                 float2 (&acc)[V][(EPV + 1) / 2]) {
+  if (HASW && EPV == 8) accumulate_edges<T, EPV, G, V, U, HASW, PIPE, true>(p, k0, k1, xb, active, gl, sm, acc);
+  else if (p.hinted) accumulate_edges<T, EPV, G, V, U, HASW, PIPE, true>(p, k0, k1, xb, active, gl, sm, acc);
+  else accumulate_edges<T, EPV, G, V, U, HASW, PIPE, false>(p, k0, k1, xb, active, gl, sm, acc);
 }
 
 // epilogue for EPV consecutive features [f, f+EPV) of row `row`
@@ -404,7 +433,8 @@ constexpr int SPMM_THREADS = 256;
 // of 2.95 ms per hop); capping the variants whose in-flight gather data needs <= 32 registers at 64
 // costs no spills and restores 4 CTAs/SM.  Variants with more data in flight get proportionally more; the leanest
 // (one vector, 4 edges) fit 5 CTAs/SM in 48 registers without spills (6 CTAs / 40 registers spill 16 bytes and gain
-// nothing more: 2.77 vs 2.74 ms on the products-shaped hop).
+// nothing more: 2.77 vs 2.74 ms on the products-shaped hop).  With unpredicated gathers (round 4) one vector and 8
+// edges needs 62 registers: 4 CTAs/SM, no spills (capped at 48 for 5 CTAs/SM it spills 224 bytes).
 template <int EPV, int V, int U, bool PIPE>
 constexpr int spmm_minb() {
   constexpr int raw = ((EPV > 1) ? 4 : 1) * V * U * (PIPE ? 2 : 1);   // registers holding gathered vectors
@@ -412,14 +442,16 @@ constexpr int spmm_minb() {
   return need <= 24 ? 5 : (need <= 40 ? 4 : (need <= 56 ? 3 : (need <= 72 ? 2 : 1)));
 }
 
-// per-lane vector bases: lane l of the group owns vectors l, l+G, ... of the feature tile
+// per-lane vector bases: lane l of the group owns vectors l, l+G, ... of the feature tile.  A vector beyond F
+// (active[v] = false) is gathered from the row's last vector and its sum never stored.
 template <typename T, int EPV, int G, int V>
 __device__ __forceinline__ void lane_bases(const SpmmParams& p, int f0, const char* (&xb)[V], bool (&active)[V]) {
+  const int last = (p.F - 1) / EPV * EPV;
 #pragma unroll
   for (int v = 0; v < V; ++v) {
     const int f = f0 + v * G * EPV;
     active[v] = f < p.F;
-    xb[v] = reinterpret_cast<const char*>(p.X) + (size_t)(active[v] ? f : 0) * sizeof(T);   // inactive: never dereferenced
+    xb[v] = reinterpret_cast<const char*>(p.X) + (size_t)(active[v] ? f : last) * sizeof(T);
   }
 }
 
